@@ -6,6 +6,7 @@ baseline (the oracle port of the reference's fp32 step, oracle/two_towers_oracle
 
     python bench.py [--gpus N --steps K --warmup W]            # N>1: launched by torch.distributed.run
     python bench.py --impl reference [--steps K --warmup W]    # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                     # + the last timed step's results as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1], "heavy GPU run shape"): per-GPU batch 2048 triplets, projection dim 512,
 margin 0.3, query length 32 / document length 256 tokens (SURVEY.md §8d shape U: full-length rows, ids
@@ -222,6 +223,27 @@ def workload_config(world):
     }
 
 
+# FusedTrainer's parameter order (TwoTowersModel.projection_parameters): Wq1, bq1, Wq2, bq2, Wd1, bd1, Wd2, bd2
+PROJECTION_NAMES = [f"{t}.projection.{i}.{k}" for t in ("query_tower", "document_tower") for i in (0, 2)
+                    for k in ("weight", "bias")]
+
+
+def dump_outputs(out_dir: str, trainer):
+    """What the last timed step hands its caller, one float32 DIR/<name>.npy each: the loss, the gradients of the 8
+    projection tensors (grad.<name>, this rank's) and the parameters after the Adam update (<name>); 7.4 MB at
+    configs[1].  The inputs depend on the arguments only (seeded model and token batches), so two builds run with the
+    same arguments can be compared file by file."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": trainer.loss_view}
+    for name, p, g in zip(PROJECTION_NAMES, trainer.p_views, trainer.g_views):
+        arrays[name] = p
+        arrays["grad." + name] = g
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------------
 # B200 arm
 # --------------------------------------------------------------------------------------------------
@@ -314,6 +336,8 @@ def run_b200(args):
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
     loss_after = float(trainer.loss_view[0].item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer)
     value = B_PER_GPU * world * K / (ms_total * 1e-3)
 
     # ---- leg 2: end to end through the public API, host buffers --------------------------------------
@@ -1071,7 +1095,13 @@ def main():
     ap.add_argument("--scan-docs", type=int, default=8_800_000)
     ap.add_argument("--scan-queries", type=int, default=100_000)
     ap.add_argument("--scan-passes", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, gradients and parameters of the last timed training step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the B200 arm's timed steps")
     if args.warmup < 3:
         args.warmup = 3
     quiet_stdout()

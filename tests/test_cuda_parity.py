@@ -1022,3 +1022,36 @@ def test_in_batch_negative_index_out_of_range_raises_the_error_flag(tt):
     torch.cuda.synchronize()
     assert int(tr.step_obj.err.item()) != 0
     tr.close()
+
+
+# ---------------------------------------------------------------------------------------------------
+# bench.py --dump-outputs
+# ---------------------------------------------------------------------------------------------------
+def test_bench_dumps_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: loss, the 8 projection gradients and the updated parameters of the last timed step as
+    float32 .npy files, the loss equal to the one the JSON line reports, within the 64 MB budget."""
+    import json
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu",
+                          "--no-scan", "--no-config2", "--no-backbone", "--no-chain-variant", "--no-epoch",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=root)
+    assert out.returncode == 0, out.stderr[-3000:]
+    lines = [l for l in out.stdout.splitlines() if l.strip()]
+    assert len(lines) == 1
+    d = json.loads(lines[0])
+    assert d["steps"] == 2
+    names = [f"{t}.projection.{i}.{k}" for t in ("query_tower", "document_tower") for i in (0, 2)
+             for k in ("weight", "bias")]
+    want = {"loss.npy"} | {n + ".npy" for n in names} | {"grad." + n + ".npy" for n in names}
+    assert set(os.listdir(tmp_path)) == want
+    assert sum(os.path.getsize(tmp_path / f) for f in want) <= 64 << 20
+    arrays = {f[:-4]: np.load(tmp_path / f) for f in want}
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in arrays.values())
+    assert arrays["loss"].shape == (1,) and float(arrays["loss"][0]) == d["loss_after"]
+    P, H = d["config"]["projection_dim"], 384
+    assert arrays["query_tower.projection.0.weight"].shape == (P, H)
+    assert arrays["document_tower.projection.2.weight"].shape == (P, P)
+    assert all(np.abs(arrays["grad." + n]).max() > 0 for n in names)
