@@ -87,11 +87,13 @@ __global__ void __launch_bounds__(1024) colsum_kernel(const float* __restrict__ 
 }
 
 // two-stage column sums for up to two matrices per launch (query | document rows): slices of rows are summed
-// by separate CTAs into scratch[job][slice][N], then added in ascending slice order (deterministic)
+// by separate CTAs into scratch[job][slice][N], then added in ascending slice order (deterministic).  The sums
+// accumulate in double: the bias gradient of the document tower adds positive and negative rows whose dY nearly cancel
+// column by column (condition number ~5e4 at B = 8256), where fp32 running sums over ~65 rows per thread were 2e-3 off.
 __global__ void __launch_bounds__(256) colsum_partial_kernel(const float* __restrict__ X0, int M0,
                                                              const float* __restrict__ X1, int M1, int N, long long ld,
                                                              int S, float* __restrict__ scratch) {
-  __shared__ float s[8][33];
+  __shared__ double s[8][33];
   pdl_wait();
   pdl_launch();
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -101,16 +103,16 @@ __global__ void __launch_bounds__(256) colsum_partial_kernel(const float* __rest
   const int per = (M + S - 1) / S;
   const int r0 = slice * per, r1 = min(M, r0 + per);
   const int n = blockIdx.x * 32 + tx;
-  float sum = 0.f;
+  double sum = 0.0;
   if (n < N)
-    for (int m = r0 + ty; m < r1; m += 8) sum += X[(size_t)m * ld + n];
+    for (int m = r0 + ty; m < r1; m += 8) sum += (double)X[(size_t)m * ld + n];
   s[ty][tx] = sum;
   __syncthreads();
   if (ty == 0 && n < N) {
-    float t = 0.f;
+    double t = 0.0;
 #pragma unroll
     for (int i = 0; i < 8; ++i) t += s[i][tx];
-    scratch[((size_t)job * S + slice) * N + n] = t;
+    scratch[((size_t)job * S + slice) * N + n] = (float)t;
   }
 }
 
@@ -122,10 +124,10 @@ __global__ void __launch_bounds__(256) colsum_final_kernel(const float* __restri
   const int n = blockIdx.x * 256 + threadIdx.x;
   const int job = blockIdx.y;
   if (n >= N) return;
-  float t = 0.f;
-  for (int i = 0; i < S; ++i) t += scratch[((size_t)job * S + i) * N + n];
+  double t = 0.0;
+  for (int i = 0; i < S; ++i) t += (double)scratch[((size_t)job * S + i) * N + n];
   float* out = job ? out1 : out0;
-  out[n] = accumulate ? (out[n] + t) : t;
+  out[n] = accumulate ? (float)((double)out[n] + t) : (float)t;
 }
 
 }  // namespace
