@@ -377,6 +377,7 @@ extern "C" int tt_adam_step_dev(float* param, const float* grad, float* exp_avg,
 // corpus scan
 // ------------------------------------------------------------------------------------------------
 extern "C" size_t tt_scan_ws_bytes(int Q, int64_t N, int P, int k, int precision) {
+  if (N <= 0) return 0;  // an empty shard only writes padding (and has no document splits to plan)
   if (precision == TT_PREC_FP32) return scan_fp32_ws_bytes(Q, N, k);
   return scan_sm100_ws_bytes(Q, N, P, k);
 }
@@ -389,11 +390,7 @@ extern "C" int tt_scan_topk(const float* Qn, const float* Dn, const void* Qb, co
   cudaStream_t st = as_stream(stream);
   if (Q == 0) return 0;
   TT_REQUIRE(ws_bytes >= tt_scan_ws_bytes(Q, N, P, k, precision), "tt_scan_topk: workspace too small");
-  if (N == 0) {
-    TT_CUDA(cudaMemsetAsync(top_id, 0xff, (size_t)Q * k * 8, st));
-    TT_CUDA(cudaMemsetAsync(top_score, 0xff, (size_t)Q * k * 4, st));  // NaN pattern; ids are -1
-    return 0;
-  }
+  if (N == 0) return scan_empty(Q, k, top_score, reinterpret_cast<long long*>(top_id), st);
   if (precision == TT_PREC_FP32)
     return scan_topk_fp32(Qn, Dn, Q, N, P, k, id_base, top_score, reinterpret_cast<long long*>(top_id), ws, ws_bytes,
                           st);

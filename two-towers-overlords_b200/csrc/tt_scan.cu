@@ -287,6 +287,38 @@ int scan_splits(int Q, long long N) {
   return (int)want;
 }
 
+// Dynamic shared memory of scan_topk_fp32_kernel: two operand tiles, the score tile and a k-long list per query
+// (25,352 + 768 k bytes).  Past 48 KB (k > 30) the kernel must opt in, once per process; the 227 KB of an SM100 block
+// are what bounds k.
+static int fp32_scan_smem(int k, size_t* smem) {
+  constexpr size_t kMaxSmem = 227 * 1024;
+  *smem = sizeof(float) * (SK * (SQ + 4 + SD + 4) + SQ * (SD + 1)) + (size_t)SQ * k * 4 + 8 + (size_t)SQ * k * 8;
+  TT_REQUIRE(*smem <= kMaxSmem, "tt_scan_topk: k=%d too large for the fp32 scan", k);
+  static bool attr_done = false;
+  if (*smem > 48 * 1024 && !attr_done) {
+    TT_CUDA(cudaFuncSetAttribute(scan_topk_fp32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    attr_done = true;
+  }
+  return 0;
+}
+
+// k > N rows of an empty shard: the (-inf, -1) padding every other path writes
+__global__ void fill_empty_kernel(long long n, float* __restrict__ os, long long* __restrict__ oi) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) {
+    os[i] = -INFINITY;
+    oi[i] = -1;
+  }
+}
+
+int scan_empty(int Q, int k, float* top_score, long long* top_id, cudaStream_t st) {
+  const long long n = (long long)Q * k;
+  if (n <= 0) return 0;
+  fill_empty_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, top_score, top_id);
+  TT_LAUNCH_CHECK();
+  return 0;
+}
+
 int topk_merge(const float* ps, const long long* pi, int G, int Q, int k, float* os, long long* oi, cudaStream_t st) {
   if (Q <= 0) return 0;
   topk_merge_kernel<<<(Q + 7) / 8, 256, 0, st>>>(ps, pi, G, Q, k, os, oi, nullptr, nullptr, 0);
@@ -311,8 +343,8 @@ int scan_topk_fp32_listed(const float* Qn, const float* Dn, int Q, long long N, 
   const long long max_splits = (N + SD - 1) / SD;
   if (S > max_splits) S = (int)max_splits;
   const long long per = ((N + S - 1) / S + SD - 1) / SD * SD;
-  const size_t smem = sizeof(float) * (SK * (SQ + 4 + SD + 4) + SQ * (SD + 1)) + (size_t)SQ * k * 4 + 8 + (size_t)SQ * k * 8;
-  TT_REQUIRE(smem <= 48 * 1024, "tt_scan_topk: k=%d too large for the fp32 scan", k);
+  size_t smem;
+  if (int rc = fp32_scan_smem(k, &smem)) return rc;
   for (int slot0 = 0; slot0 < Q; slot0 += cap) {  // later rounds find nothing to do unless > cap rows are listed
     const int nq = min(cap, Q - slot0);
     dim3 grid(S, (nq + SQ - 1) / SQ);
@@ -333,8 +365,8 @@ int scan_topk_fp32(const float* Qn, const float* Dn, int Q, long long N, int P, 
   long long* pi = ws_take<long long>(p, (size_t)S * Q * k);
   TT_REQUIRE((size_t)(p - reinterpret_cast<char*>(ws)) <= ws_bytes, "tt_scan_topk: workspace too small");
   const long long per = ((N + S - 1) / S + SD - 1) / SD * SD;
-  const size_t smem = sizeof(float) * (SK * (SQ + 4 + SD + 4) + SQ * (SD + 1)) + (size_t)SQ * k * 4 + 8 + (size_t)SQ * k * 8;
-  TT_REQUIRE(smem <= 48 * 1024, "tt_scan_topk: k=%d too large for the fp32 scan", k);
+  size_t smem;
+  if (int rc = fp32_scan_smem(k, &smem)) return rc;
   dim3 grid(S, (Q + SQ - 1) / SQ);
   scan_topk_fp32_kernel<<<grid, 256, smem, st>>>(Qn, Dn, Q, N, P, k, per, id_base, ps, pi, nullptr, nullptr, 0);
   TT_LAUNCH_CHECK();

@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(kRefineThreads)
   //    element after the previous one" in (value desc, slot asc) order, shuffles only, no block barrier — then warp 0
   //    takes the k-th best of the 4k listed entries (the k best overall are among them).
   {
-    float* wl_v = sel_s;  // [4][k] (the selection buffers are not in use yet; k <= 16 by the caller's contract)
+    float* wl_v = sel_s;  // [4][k] (the selection buffers are not in use yet; 4k <= kSelCap as k <= 32)
     int* wl_c = sel_c;
     float lv = INFINITY;
     int lc = -1;
@@ -446,7 +446,7 @@ __global__ void __launch_bounds__(kRefineThreads)
     }
     __syncthreads();
     if (warp == 0) {
-      const int n = 4 * k;  // <= 64: two entries per lane
+      const int n = 4 * k;  // <= 128: up to four entries per lane
       float mv = INFINITY;
       int mc = -1, found = 0;
       for (int r = 0; r < k; ++r) {
