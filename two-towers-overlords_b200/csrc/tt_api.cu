@@ -214,6 +214,8 @@ extern "C" size_t tt_step_ws_bytes(int B, int Lq, int Ld, int H, int P, int voca
 
 // Diagnostics and parity tests: device address of a named internal buffer of a tensor-core step workspace.
 //   "trace"  per-CTA task timeline of the last TT_CHAIN_TRACE=1 step: [160][64] x {task << 2 | kind, globaltimer ns}
+//   "x_hi" / "x_lo" / "x_lo2"            bf16 terms [3B, H] of the pooled rows xhat (rows q | p | n; x_lo2 is written by
+//                                        bf16x3 steps only)
 //   "h_hi" / "h_lo" / "dy_hi" / "dy_lo"  bf16 terms [3B, P] of the hidden activations / of dY (rows q | p | n)
 extern "C" int tt_debug_step_buffer(void* ws, int B, int Lq, int Ld, int H, int P, int vocab, int precision,
                                     int train_table, const char* name, void** ptr) {
@@ -224,6 +226,9 @@ extern "C" int tt_debug_step_buffer(void* ws, int B, int Lq, int Ld, int H, int 
   tt::carve_step(reinterpret_cast<char*>(w.mma_ws), B, H, P, train_table, &m);
   void* out = nullptr;
   if (!strcmp(name, "trace")) out = m.trace;
+  else if (!strcmp(name, "x_hi")) out = m.x_hi;
+  else if (!strcmp(name, "x_lo")) out = m.x_lo;
+  else if (!strcmp(name, "x_lo2")) out = m.x_lo2;
   else if (!strcmp(name, "h_hi")) out = m.h_hi;
   else if (!strcmp(name, "h_lo")) out = m.h_lo;
   else if (!strcmp(name, "dy_hi")) out = m.dy_hi;

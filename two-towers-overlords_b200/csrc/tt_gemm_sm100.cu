@@ -666,7 +666,7 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
   const bool chain = s.chain == 1 || (s.chain == 0 && chain_enabled());
   if (front) {
     PoolParams pp = s.pool;
-    pp.x_hi = w.x_hi; pp.x_lo = w.x_lo; pp.x_lo2 = (np == 3) ? w.x_lo2 : nullptr; pp.xt_hi = nullptr; pp.xt_lo = nullptr;
+    pp.x_hi = w.x_hi; pp.x_lo = w.x_lo; pp.x_lo2 = (np == 3) ? w.x_lo2 : nullptr;
     pp.share_sm = (s.phases == TT_STEP_FRONT) ? 1 : 0;  // gather-only call = the pipelined trainer's look-ahead gather
     if ((rc = pool_fwd_launch(pp, s.table_dtype, H, st))) return rc;
     // (the persistent chain kernel transposes the xhat terms itself)

@@ -184,17 +184,25 @@ __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams
   for (int i = 0; i < kPoolWarps; ++i) cnt += s_fred[i];
   const float denom = fmaxf(cnt, 1e-9f);  // clamp(min=1e-9), model.py:70-72
 
-  float4 m = make_float4(0.f, 0.f, 0.f, 0.f);
+  // thread tid owns the 4-column groups tid + k * kPoolThreads (k < kOwn) below NV * 32: columns [4*grp, 4*grp+4).
+  // kOwn is 1 for H <= 512 and 2 for H = 768.
+  constexpr int kOwn = (NV * 32 + kPoolThreads - 1) / kPoolThreads;
+  float4 m[kOwn];
   float sq = 0.f;
-  const bool owner = tid < NV * 32;  // thread owns columns [4*tid, 4*tid+4)
-  if (owner) {
 #pragma unroll
-    for (int i = 0; i < kPoolWarps; ++i) {
-      const float4 t = *reinterpret_cast<const float4*>(&s_red[i][tid * 4]);
-      m.x += t.x; m.y += t.y; m.z += t.z; m.w += t.w;
+  for (int k = 0; k < kOwn; ++k) {
+    const int grp = tid + k * kPoolThreads;
+    m[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (grp < NV * 32) {
+#pragma unroll
+      for (int i = 0; i < kPoolWarps; ++i) {
+        const float4 t = *reinterpret_cast<const float4*>(&s_red[i][grp * 4]);
+        m[k].x += t.x; m[k].y += t.y; m[k].z += t.z; m[k].w += t.w;
+      }
+      m[k].x = m[k].x / denom; m[k].y = m[k].y / denom; m[k].z = m[k].z / denom; m[k].w = m[k].w / denom;
+      const float s = m[k].x * m[k].x + m[k].y * m[k].y + m[k].z * m[k].z + m[k].w * m[k].w;
+      sq = k == 0 ? s : sq + s;
     }
-    m.x = m.x / denom; m.y = m.y / denom; m.z = m.z / denom; m.w = m.w / denom;
-    sq = m.x * m.x + m.y * m.y + m.z * m.z + m.w * m.w;
   }
   __syncthreads();  // s_fred is reused below
   sq = warp_sum(sq);
@@ -207,33 +215,32 @@ __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams
   const float dn = fmaxf(nrm, 1e-12f);  // F.normalize eps, model.py:56
 
   const int row_out = sg.row0 + b;
-  float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (owner) x = make_float4(m.x / dn, m.y / dn, m.z / dn, m.w / dn);
-  // every output of one pooled row (owner threads: 4 columns each; thread 0: the count and the norm)
+  float4 x[kOwn];
+#pragma unroll
+  for (int k = 0; k < kOwn; ++k) {
+    x[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (tid + k * kPoolThreads < NV * 32) x[k] = make_float4(m[k].x / dn, m[k].y / dn, m[k].z / dn, m[k].w / dn);
+  }
+  // every output of one pooled row (each thread: its column groups; thread 0: the count and the norm)
   auto emit_row = [&](int row) {
-    if (owner) {
-      *reinterpret_cast<float4*>(p.xhat + (size_t)row * H + tid * 4) = x;
-      if (p.x_hi) {  // operands of the tensor-core projection: bf16 hi/lo split, row-major + transposed
-        const float xv[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+    for (int k = 0; k < kOwn; ++k) {
+      const int grp = tid + k * kPoolThreads;
+      if (grp >= NV * 32) continue;
+      *reinterpret_cast<float4*>(p.xhat + (size_t)row * H + grp * 4) = x[k];
+      if (p.x_hi) {  // operands of the tensor-core projection: bf16 hi/lo(/lo2) split, row-major
+        const float xv[4] = {x[k].x, x[k].y, x[k].z, x[k].w};
         __nv_bfloat16 hi[4], lo[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) split_bf16(xv[c], hi[c], lo[c]);
-        *reinterpret_cast<uint2*>(p.x_hi + (size_t)row * H + tid * 4) = *reinterpret_cast<uint2*>(hi);
-        *reinterpret_cast<uint2*>(p.x_lo + (size_t)row * H + tid * 4) = *reinterpret_cast<uint2*>(lo);
+        *reinterpret_cast<uint2*>(p.x_hi + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(hi);
+        *reinterpret_cast<uint2*>(p.x_lo + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(lo);
         if (p.x_lo2) {
           __nv_bfloat16 l2[4];
 #pragma unroll
           for (int c = 0; c < 4; ++c)
             l2[c] = __float2bfloat16_rn((xv[c] - __bfloat162float(hi[c])) - __bfloat162float(lo[c]));
-          *reinterpret_cast<uint2*>(p.x_lo2 + (size_t)row * H + tid * 4) = *reinterpret_cast<uint2*>(l2);
-        }
-        if (p.xt_hi) {
-          const int tcol = row + (row >= p.t_split_row ? p.t_shift : 0);
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            p.xt_hi[(size_t)(tid * 4 + c) * p.ldt + tcol] = hi[c];
-            p.xt_lo[(size_t)(tid * 4 + c) * p.ldt + tcol] = lo[c];
-          }
+          *reinterpret_cast<uint2*>(p.x_lo2 + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(l2);
         }
       }
     }

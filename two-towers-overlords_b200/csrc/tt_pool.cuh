@@ -19,16 +19,10 @@ struct PoolParams {
   float* cnt;   // [rows] nullable
   float* nrm;   // [rows] nullable
   int* err;     // nullable
-  // optional operands for the tensor-core projection (bf16 hi/lo split)
+  // optional operands for the tensor-core projection (bf16 hi/lo split, row-major)
   __nv_bfloat16* x_hi;   // [rows, H]
   __nv_bfloat16* x_lo;
   __nv_bfloat16* x_lo2;  // nullable third term: xhat - hi - lo
-  __nv_bfloat16* xt_hi;  // [H, ldt] transposed
-  __nv_bfloat16* xt_lo;
-  int ldt;
-  // column of row r in the transposed copies: r + (r >= t_split_row ? t_shift : 0) — lets the document rows
-  // start at a 64-aligned column so each tower's K range is its own TMA tensor
-  int t_split_row, t_shift;
   int share_sm;  // 1: this launch runs beside other kernels (pipelined step): cap the resident CTAs per SM
   // optional row aliases: output row alias_dst_row0 + i is a copy of output row alias_src_row0 + alias[i], i < alias_n
   // (in-batch negatives: negative i is the positive document of item alias[i]); nullptr = none
