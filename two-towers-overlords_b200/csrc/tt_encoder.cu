@@ -205,20 +205,37 @@ size_t carve_enc(char* base, size_t T, int H, int I, EncWs* out) {
   return (size_t)(p - base) + 256;
 }
 
+// attention_kernel<32> keeps K and V of one head plus one mask byte per position in dynamic shared memory
+size_t attention_smem(int L) { return (size_t)2 * L * 32 * sizeof(float) + L; }
+
+// Dynamic shared memory attention_kernel<32> may use: the device's opt-in limit less the kernel's static shared
+// memory (257 B per position: L <= 904 on a B200).  Opted into on the first call.
+int attention_smem_limit(size_t* out) {
+  static size_t limit = 0;
+  if (!limit) {
+    int dev = 0, optin = 0;
+    TT_CUDA(cudaGetDevice(&dev));
+    TT_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    cudaFuncAttributes fa{};
+    TT_CUDA(cudaFuncGetAttributes(&fa, attention_kernel<32>));
+    const size_t lim = (size_t)optin - fa.sharedSizeBytes;
+    TT_CUDA(cudaFuncSetAttribute(attention_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lim));
+    limit = lim;
+  }
+  *out = limit;
+  return 0;
+}
+
 template <int NV>
 int encoder_fwd(const tt_encoder_weights* W, const void* ids, int ids_dtype, const void* mask, int mask_dtype, int B,
                 int L, float* hidden_out, const EncWs& w, int* err, cudaStream_t st) {
   const int H = W->hidden, I = W->inter, T = B * L, D = H / W->heads;
   const int tb = (T + 3) / 4;
+  // without layers the last hidden state is the embedding output, as in BertModel
   embed_ln_kernel<NV><<<tb, 128, 0, st>>>(ids, ids_dtype, T, L, W->vocab, W->word_emb, W->pos_emb, W->type_emb, W->emb_ln_g,
-                                        W->emb_ln_b, W->ln_eps, w.h, w.h_hi, w.h_lo, err);
+                                        W->emb_ln_b, W->ln_eps, W->n_layers ? w.h : hidden_out, w.h_hi, w.h_lo, err);
   TT_LAUNCH_CHECK();
-  const size_t att_smem = (size_t)2 * L * D * sizeof(float) + L;
-  static bool attr_done = false;
-  if (!attr_done) {
-    TT_CUDA(cudaFuncSetAttribute(attention_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    attr_done = true;
-  }
+  const size_t att_smem = attention_smem(L);
   int rc;
   for (int l = 0; l < W->n_layers; ++l) {
     const tt_encoder_layer& Y = W->layers[l];
@@ -267,13 +284,24 @@ extern "C" int tt_split_bf16_terms(const float* x, int rows, int cols, void* hi,
 extern "C" int tt_encoder_fwd(const tt_encoder_weights* w, const void* ids, int ids_dtype, const void* mask, int mask_dtype,
                               int B, int L, float* hidden_out, int* err_flag, void* ws, size_t ws_bytes,
                               tt_stream_t stream) {
-  TT_REQUIRE(w && w->layers && ids && mask && hidden_out, "tt_encoder_fwd: null argument");
+  TT_REQUIRE(w && ids && mask && hidden_out, "tt_encoder_fwd: null argument");
+  TT_REQUIRE(w->n_layers >= 0 && (w->n_layers == 0 || w->layers), "tt_encoder_fwd: bad layers (%d layers)", w->n_layers);
   TT_REQUIRE(B >= 0 && L >= 1 && L <= w->max_pos, "tt_encoder_fwd: bad shape B=%d L=%d (max positions %d)", B, L, w->max_pos);
-  TT_REQUIRE(w->hidden % 128 == 0 && w->hidden <= 768 && w->hidden / w->heads == 32 && w->inter % 64 == 0,
-             "tt_encoder_fwd: supports hidden sizes 128..768 in steps of 128 with 32-wide heads (hidden %d, heads %d)",
-             w->hidden, w->heads);
+  TT_REQUIRE(w->heads >= 1 && w->hidden >= 128 && w->hidden % 128 == 0 && w->hidden <= 768 &&
+                 w->hidden / w->heads == 32 && w->inter >= 64 && w->inter % 64 == 0,
+             "tt_encoder_fwd: supports hidden sizes 128..768 in steps of 128 with 32-wide heads and intermediate sizes "
+             "in steps of 64 (hidden %d, heads %d, intermediate %d)",
+             w->hidden, w->heads, w->inter);
   if (B == 0) return 0;
   TT_REQUIRE(ws_bytes >= tt_encoder_ws_bytes(B * L, w->hidden, w->inter), "tt_encoder_fwd: workspace too small");
+  if (w->n_layers > 0) {
+    size_t limit = 0;
+    int rc = attention_smem_limit(&limit);
+    if (rc) return rc;
+    TT_REQUIRE(attention_smem(L) <= limit,
+               "tt_encoder_fwd: sequence length L=%d needs %zu bytes of shared memory in attention, this device allows "
+               "%zu (L <= %zu)", L, attention_smem(L), limit, limit / attention_smem(1));
+  }
   EncWs e;
   carve_enc(reinterpret_cast<char*>(ws), (size_t)B * L, w->hidden, w->inter, &e);
   cudaStream_t st = as_stream(stream);
@@ -281,6 +309,8 @@ extern "C" int tt_encoder_fwd(const tt_encoder_weights* w, const void* ids, int 
     case 1: return encoder_fwd<1>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
     case 2: return encoder_fwd<2>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
     case 3: return encoder_fwd<3>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
+    case 4: return encoder_fwd<4>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
+    case 5: return encoder_fwd<5>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
     case 6: return encoder_fwd<6>(w, ids, ids_dtype, mask, mask_dtype, B, L, hidden_out, e, err_flag, st);
     default: TT_REQUIRE(false, "tt_encoder_fwd: hidden size %d not supported", w->hidden);
   }
