@@ -158,8 +158,9 @@ typedef struct tt_step_args {
   int precision;
   void* ws; size_t ws_bytes;  /* >= tt_step_ws_bytes(...); zero-fill it once before its first use (it holds an
                                  arrival counter that every call leaves at zero again)                        */
-  int phases;        /* 0 = whole step; TT_STEP_FRONT = pooled gather only (reads tokens + tables, not the
-                        projection weights, so it may overlap the previous step's parameter exchange);
+  int phases;        /* 0 = whole step; TT_STEP_FRONT = pooled gather only (reads tokens + tables, or the pooled
+                        banks below, not the projection weights, so it may overlap the previous step's parameter
+                        exchange);
                         TT_STEP_BACK = everything after it, on the same workspace                             */
   /* optional optimiser (training.py:51 `optimizer.step()`; adam_param NULL = gradients only): torch.optim.Adam
    * arithmetic on ONE flat fp32 parameter buffer of adam_n elements.  The 8 projection tensors above must be
@@ -184,6 +185,20 @@ typedef struct tt_step_args {
    * again, for half the document rows read; n_ids / n_mask are not read then.  Frozen tables only.  An index out
    * of range raises err_flag.                                                                                  */
   const int32_t* neg_index;
+  /* optional frozen front end (NULL = pool tokens as before): rows of F.normalize(masked_mean(backbone(text)))
+   * computed once per text.  Output row i     = pooled_q[pooled_index[i]],
+   *                           row B + i       = pooled_d[pooled_index[B + i]],
+   *                           row 2B + i      = pooled_d[pooled_index[2B + i]]   (int32 [3B] on the device).
+   * Rows are fp32 [rows, H], 16-byte aligned.  Tokens and tables are not read (may be NULL).  Needs frozen tables
+   * and neg_index == NULL.  An index outside [0, rows) sets err_flag and reads row 0.  cnt / nrm of the pooled
+   * rows are not known then: only the table gradient reads them, and it is refused.
+   * These five fields were appended while TT_B200_VERSION stayed at 100, so the version does not tell the two
+   * layouts apart.  A caller compiled against a header without them passes a shorter struct, and the library
+   * reads whatever follows it as pooled_*: rebuild such a caller against this header (the ctypes mirror in
+   * _native.py lists them), and zero-initialise the struct as before.                                          */
+  const float* pooled_q; int64_t pooled_q_rows;
+  const float* pooled_d; int64_t pooled_d_rows;
+  const int32_t* pooled_index;
 } tt_step_args;
 #define TT_STEP_FRONT 1
 #define TT_STEP_BACK 2
@@ -311,6 +326,13 @@ int tt_assemble_triplets(const tt_token_bank* qbank, const tt_token_bank* dbank,
                          int B, uint64_t seed, int Lq, int Ld, void* q_ids, void* q_mask, void* p_ids, void* p_mask,
                          void* n_ids, void* n_mask, int ids_dtype, int mask_dtype, int32_t* neg_out, int* err_flag,
                          tt_stream_t stream);
+/* The same batch as bank ROWS instead of tokens (for a step with tt_step_args.pooled_index): rows_out [3B] int32 =
+ * query rows | positive rows | negative rows, i.e. pair_q[order[row0 + i]], pair_d[order[row0 + i]] and
+ * pair_d[order[neg_out[i]]].  The negatives are drawn by the same code as in tt_assemble_triplets, so for equal
+ * arguments they are the same items.  neg_out (nullable) and err_flag as there. */
+int tt_assemble_triplet_rows(const int32_t* pair_q, const int32_t* pair_d, const int32_t* pair_qid,
+                             const int32_t* order, int Bg, int row0, int B, uint64_t seed,
+                             int32_t* rows_out, int32_t* neg_out, int* err_flag, tt_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * Measurement probe (bench.py): L2 -> SM read bandwidth.  Every SM streams `buf` (`bytes` long, cache-resident

@@ -66,6 +66,9 @@ class StepArgs(ctypes.Structure):
         ("adam_lr", c_float), ("adam_beta1", c_float), ("adam_beta2", c_float), ("adam_eps", c_float),
         ("chain", c_int),
         ("neg_index", c_void_p),
+        ("pooled_q", c_void_p), ("pooled_q_rows", c_int64),
+        ("pooled_d", c_void_p), ("pooled_d_rows", c_int64),
+        ("pooled_index", c_void_p),
     ]
 
 
@@ -126,6 +129,8 @@ _SIGNATURES = {
     "tt_assemble_triplets": (c_int, [POINTER(TokenBankDesc), POINTER(TokenBankDesc), c_void_p, c_void_p, c_void_p,
                                      c_void_p, c_int, c_int, c_int, ctypes.c_uint64, c_int, c_int, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "tt_assemble_triplet_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, ctypes.c_uint64,
+                                         c_void_p, c_void_p, c_void_p, c_void_p]),
     "tt_encoder_ws_bytes": (c_size_t, [c_int, c_int, c_int]),
     "tt_encoder_fwd": (c_int, [POINTER(EncoderWeights), c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
                                c_void_p, c_size_t, c_void_p]),

@@ -273,6 +273,15 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
     pp.alias_src_row0 = B;
     pp.alias_dst_row0 = 2 * B;
   }
+  if (a->pooled_index) {  // frozen front end computed once per text: rows are copied, not pooled
+    TT_REQUIRE(!train_table, "tt_triplet_step: pooled_index needs frozen tables (dtable_q / dtable_d must be NULL)");
+    TT_REQUIRE(!a->neg_index, "tt_triplet_step: pooled_index and neg_index are exclusive (name the negatives' rows in "
+               "pooled_index instead)");
+    pp.rows_q = a->pooled_q; pp.rows_q_n = a->pooled_q_rows;
+    pp.rows_d = a->pooled_d; pp.rows_d_n = a->pooled_d_rows;
+    pp.row_index = a->pooled_index;
+    pp.row_B = B;
+  }
 
   float* dxhat = train_table ? w.dxhat : nullptr;
   bool adam_done = false;

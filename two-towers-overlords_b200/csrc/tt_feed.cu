@@ -84,19 +84,53 @@ __global__ void __launch_bounds__(64) assemble_triplets_kernel(const AssemblePar
   }
 }
 
+// one thread per item: the bank rows of its query, its positive and its negative (a step with a pooled front end
+// gathers precomputed pooled rows by these indices instead of pooling tokens)
+__global__ void __launch_bounds__(128) assemble_triplet_rows_kernel(const AssembleParams p, int* __restrict__ rows_out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= p.B) return;
+  const int i = p.row0 + b;
+  const int j = draw_negative(p, i);
+  if (p.neg_out) p.neg_out[b] = j;
+  rows_out[b] = p.pair_q[p.order[i]];
+  rows_out[p.B + b] = p.pair_d[p.order[i]];
+  rows_out[2 * p.B + b] = p.pair_d[p.order[j]];
+}
+
+int check_slice(const char* who, const int32_t* pair_q, const int32_t* pair_d, const int32_t* pair_qid,
+                const int32_t* order, int Bg, int row0, int B) {
+  TT_REQUIRE(pair_q && pair_d && pair_qid && order, "%s: null input", who);
+  TT_REQUIRE(Bg >= 2 && row0 >= 0 && B >= 0 && row0 + B <= Bg, "%s: bad slice [%d,%d) of %d", who, row0, row0 + B, Bg);
+  return 0;
+}
+
 }  // namespace
 }  // namespace tt
 
 using namespace tt;
+
+extern "C" int tt_assemble_triplet_rows(const int32_t* pair_q, const int32_t* pair_d, const int32_t* pair_qid,
+                                        const int32_t* order, int Bg, int row0, int B, uint64_t seed,
+                                        int32_t* rows_out, int32_t* neg_out, int* err_flag, tt_stream_t stream) {
+  if (int rc = check_slice("tt_assemble_triplet_rows", pair_q, pair_d, pair_qid, order, Bg, row0, B)) return rc;
+  TT_REQUIRE(rows_out != nullptr, "tt_assemble_triplet_rows: null rows_out");
+  if (B == 0) return 0;
+  AssembleParams p{};
+  p.pair_q = pair_q; p.pair_d = pair_d; p.pair_qid = pair_qid; p.order = order;
+  p.Bg = Bg; p.row0 = row0; p.B = B; p.seed = seed;
+  p.neg_out = neg_out; p.err = err_flag;
+  assemble_triplet_rows_kernel<<<(B + 127) / 128, 128, 0, as_stream(stream)>>>(p, rows_out);
+  TT_LAUNCH_CHECK();
+  return 0;
+}
 
 extern "C" int tt_assemble_triplets(const tt_token_bank* qbank, const tt_token_bank* dbank, const int32_t* pair_q,
                                     const int32_t* pair_d, const int32_t* pair_qid, const int32_t* order, int Bg,
                                     int row0, int B, uint64_t seed, int Lq, int Ld, void* q_ids, void* q_mask,
                                     void* p_ids, void* p_mask, void* n_ids, void* n_mask, int ids_dtype, int mask_dtype,
                                     int32_t* neg_out, int* err_flag, tt_stream_t stream) {
-  TT_REQUIRE(qbank && dbank && pair_q && pair_d && pair_qid && order, "tt_assemble_triplets: null input");
-  TT_REQUIRE(Bg >= 2 && row0 >= 0 && B >= 0 && row0 + B <= Bg, "tt_assemble_triplets: bad slice [%d,%d) of %d", row0,
-             row0 + B, Bg);
+  TT_REQUIRE(qbank && dbank, "tt_assemble_triplets: null input");
+  if (int rc = check_slice("tt_assemble_triplets", pair_q, pair_d, pair_qid, order, Bg, row0, B)) return rc;
   TT_REQUIRE(Lq >= 1 && Ld >= 1, "tt_assemble_triplets: bad lengths");
   for (int dt : {qbank->dtype, dbank->dtype, ids_dtype})
     TT_REQUIRE(dt == TT_I64 || dt == TT_I32 || dt == TT_U16, "tt_assemble_triplets: unsupported id dtype %d", dt);

@@ -48,6 +48,46 @@ struct RowVec<__nv_bfloat16> {
   }
 };
 
+// Four consecutive columns [col, col + 4) of output row `row`: xhat and, for the tensor-core projection, its bf16
+// hi / lo (/ lo2) terms.  The one place that defines the split, shared by the pooling and the row-gather kernels.
+__device__ __forceinline__ void store_pooled4(const PoolParams& p, int H, size_t row, int col, float4 x) {
+  *reinterpret_cast<float4*>(p.xhat + row * H + col) = x;
+  if (p.x_hi) {  // operands of the tensor-core projection: bf16 hi/lo(/lo2) split, row-major
+    const float xv[4] = {x.x, x.y, x.z, x.w};
+    __nv_bfloat16 hi[4], lo[4];
+#pragma unroll
+    for (int c = 0; c < 4; ++c) split_bf16(xv[c], hi[c], lo[c]);
+    *reinterpret_cast<uint2*>(p.x_hi + row * H + col) = *reinterpret_cast<uint2*>(hi);
+    *reinterpret_cast<uint2*>(p.x_lo + row * H + col) = *reinterpret_cast<uint2*>(lo);
+    if (p.x_lo2) {
+      __nv_bfloat16 l2[4];
+#pragma unroll
+      for (int c = 0; c < 4; ++c) l2[c] = __float2bfloat16_rn((xv[c] - __bfloat162float(hi[c])) - __bfloat162float(lo[c]));
+      *reinterpret_cast<uint2*>(p.x_lo2 + row * H + col) = *reinterpret_cast<uint2*>(l2);
+    }
+  }
+}
+
+// Pooled-row front end: output row r is a copy of a precomputed pooled row (PoolParams::row_index), written with the
+// same terms the pooling epilogue writes.  One warp per row, coalesced 16-byte loads; the whole launch moves
+// 3B * H * 4 bytes (9.4 MB at B = 2048, H = 384).
+constexpr int kRowThreads = 256;
+__global__ void __launch_bounds__(kRowThreads) pooled_rows_kernel(const PoolParams p, int H) {
+  pdl_launch();  // as pool_fwd_kernel: a programmatic dependent may start filling SMs
+  const int lane = threadIdx.x & 31;
+  const int r = blockIdx.x * (kRowThreads / 32) + (threadIdx.x >> 5);
+  if (r >= 3 * p.row_B) return;
+  const bool q = r < p.row_B;
+  const long long n = q ? p.rows_q_n : p.rows_d_n;
+  long long src = __ldg(p.row_index + r);
+  if (src < 0 || src >= n) {
+    if (lane == 0 && p.err) atomicExch(p.err, 1);
+    src = 0;
+  }
+  const float4* in = reinterpret_cast<const float4*>((q ? p.rows_q : p.rows_d) + (size_t)src * H);
+  for (int v = lane; v < H / 4; v += 32) store_pooled4(p, H, (size_t)r, v * 4, __ldg(in + v));
+}
+
 template <typename TE, int NV, int UNROLL, bool PIPE>
 __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams p) {
   constexpr int H = NV * 128;
@@ -227,22 +267,7 @@ __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams
     for (int k = 0; k < kOwn; ++k) {
       const int grp = tid + k * kPoolThreads;
       if (grp >= NV * 32) continue;
-      *reinterpret_cast<float4*>(p.xhat + (size_t)row * H + grp * 4) = x[k];
-      if (p.x_hi) {  // operands of the tensor-core projection: bf16 hi/lo(/lo2) split, row-major
-        const float xv[4] = {x[k].x, x[k].y, x[k].z, x[k].w};
-        __nv_bfloat16 hi[4], lo[4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) split_bf16(xv[c], hi[c], lo[c]);
-        *reinterpret_cast<uint2*>(p.x_hi + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(hi);
-        *reinterpret_cast<uint2*>(p.x_lo + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(lo);
-        if (p.x_lo2) {
-          __nv_bfloat16 l2[4];
-#pragma unroll
-          for (int c = 0; c < 4; ++c)
-            l2[c] = __float2bfloat16_rn((xv[c] - __bfloat162float(hi[c])) - __bfloat162float(lo[c]));
-          *reinterpret_cast<uint2*>(p.x_lo2 + (size_t)row * H + grp * 4) = *reinterpret_cast<uint2*>(l2);
-        }
-      }
+      store_pooled4(p, H, (size_t)row, grp * 4, x[k]);
     }
     if (tid == 0) {
       if (p.cnt) p.cnt[row] = cnt;
@@ -326,6 +351,18 @@ int launch_pool(const PoolParams& p, int total, cudaStream_t st) {
 }  // namespace
 
 int pool_fwd_launch(PoolParams p, int table_dtype, int H, cudaStream_t st) {
+  if (p.row_index) {  // precomputed pooled rows: a copy with the epilogue's split instead of a gather of tokens
+    TT_REQUIRE(p.rows_q && p.rows_d && p.rows_q_n >= 1 && p.rows_d_n >= 1,
+               "tt_triplet_step: pooled_q / pooled_d need at least one row each");
+    TT_REQUIRE(H >= 4 && H % 4 == 0, "tt_triplet_step: pooled rows need H a multiple of 4, got %d", H);
+    TT_REQUIRE(((reinterpret_cast<uintptr_t>(p.rows_q) | reinterpret_cast<uintptr_t>(p.rows_d)) & 15) == 0,
+               "tt_triplet_step: pooled_q / pooled_d must be 16-byte aligned");
+    if (p.row_B == 0) return 0;
+    constexpr int kRowsPerCta = kRowThreads / 32;
+    pooled_rows_kernel<<<(3 * p.row_B + kRowsPerCta - 1) / kRowsPerCta, kRowThreads, 0, st>>>(p, H);
+    TT_LAUNCH_CHECK();
+    return 0;
+  }
   TT_REQUIRE(p.nseg >= 1 && p.nseg <= 4, "tt_pool_fwd: nseg must be in [1,4], got %d", p.nseg);
   TT_REQUIRE(H == 128 || H == 256 || H == 384 || H == 768,
              "tt_pool_fwd: hidden size %d not supported (128, 256, 384, 768)", H);

@@ -28,6 +28,14 @@ struct PoolParams {
   // (in-batch negatives: negative i is the positive document of item alias[i]); nullptr = none
   const int* alias;
   int alias_n, alias_src_row0, alias_dst_row0;
+  // optional precomputed pooled rows (a frozen front end encoded once per text): when row_index != nullptr the launch
+  // copies output row r = s * row_B + i (s = 0 query, 1 positive, 2 negative) from row row_index[r] of rows_q (s = 0)
+  // or rows_d, instead of pooling tokens; seg[], cnt and nrm are not used then
+  const float* rows_q;
+  const float* rows_d;
+  long long rows_q_n, rows_d_n;
+  const int* row_index;  // [3 * row_B]
+  int row_B;
 };
 
 constexpr int kPoolSharePadBytes = 0;  // default cap (bytes of unused dynamic smem per CTA); tuned on B200, see tt_pool.cu

@@ -137,6 +137,100 @@ class TokenBankTokenizer:
 
 
 # --------------------------------------------------------------------------------------------------
+# pooled banks: the frozen front end of a tower, computed once per text
+# --------------------------------------------------------------------------------------------------
+def backbone_identity(tower) -> tuple:
+    """What a pooled row depends on besides the text: the MiniLM weights (`MiniLMBackbone._key()`: device, tensor
+    versions and addresses) or the token table's version and address.  A bank built under one identity is stale
+    under any other."""
+    bb = tower.pretrained_model
+    if hasattr(bb, "_key"):
+        return ("minilm",) + tuple(bb._key())
+    t = bb.table
+    return ("table", str(t.device), t._version, t.data_ptr())
+
+
+def plan_length_batches(lengths: np.ndarray, max_tokens: int) -> list[np.ndarray]:
+    """Indices of `lengths` sorted by length (stable) and cut into consecutive batches whose padded size
+    (count x longest) stays within max_tokens; a text longer than max_tokens forms a batch of its own."""
+    lengths = np.maximum(np.asarray(lengths, dtype=np.int64), 1)
+    order = np.argsort(lengths, kind="stable")
+    batches, start = [], 0
+    n = len(order)
+    while start < n:
+        end = start + 1
+        # sorted ascending: the batch [start, end) is padded to lengths[order[end - 1]]
+        while end < n and (end + 1 - start) * int(lengths[order[end]]) <= max_tokens:
+            end += 1
+        batches.append(order[start:end])
+        start = end
+    return batches
+
+
+class PooledBank:
+    """Pooled rows of every text of one TokenBank for one tower: rows [n_texts, H] fp32 on the device, row r =
+    F.normalize(masked_mean(backbone(text r truncated to L))), and the backbone identity they were computed under.
+    Only valid while the backbone is frozen and unchanged (`check`)."""
+
+    def __init__(self, rows: torch.Tensor, identity: tuple, L: int):
+        self.rows, self.identity, self.L = rows, identity, int(L)
+
+    def __len__(self):
+        return self.rows.shape[0]
+
+    def check(self, tower, what: str = "pooled bank"):
+        if backbone_identity(tower) != self.identity:
+            raise RuntimeError(f"{what} is stale: the tower's backbone changed after the bank was built; rebuild it "
+                               "with PooledBank.build()")
+
+    @staticmethod
+    def encode_rows(tower, bank: TokenBank, L: int, lo: int, hi: int,
+                    max_tokens_per_call: Optional[int] = None) -> torch.Tensor:
+        """Pooled rows [hi - lo, H] of texts lo .. hi-1 of `bank` (truncated to L tokens) by `tower.pooled`, in
+        length-sorted batches of at most max_tokens_per_call tokens, each padded only to its own longest text."""
+        dev = tower.pretrained_model.device
+        if max_tokens_per_call is None:
+            max_tokens_per_call = getattr(tower.pretrained_model, "max_tokens_per_call", 1 << 17)
+        mine = np.arange(lo, hi, dtype=np.int64)
+        out = torch.empty(hi - lo, tower.embedding_dim, dtype=torch.float32, device=dev)
+        lens = np.minimum(bank.lengths(mine), L)
+        with torch.no_grad():
+            for part in plan_length_batches(lens, int(max_tokens_per_call)):
+                tb = bank.batch(mine[part], max_length=L)
+                out[torch.from_numpy(part).to(dev)] = tower.pooled(tb.to(dev))
+        return out
+
+    @classmethod
+    def build(cls, tower, bank: TokenBank, L: int, max_tokens_per_call: Optional[int] = None, world_size: int = 1,
+              rank: int = 0, process_group=None) -> "PooledBank":
+        """Encodes every text of `bank` (encode_rows).  With world_size > 1 rank r encodes its retrieval.shard_bounds
+        slice and one all_gather_into_tensor assembles the bank, so every rank holds the same bits (a collective;
+        process_group None = the default group)."""
+        try:
+            from .retrieval import shard_bounds
+        except ImportError:
+            from retrieval import shard_bounds
+        identity = backbone_identity(tower)
+        dev = tower.pretrained_model.device
+        H = tower.embedding_dim
+        n = len(bank)
+        lo, hi = shard_bounds(n, world_size, rank)
+        local = cls.encode_rows(tower, bank, L, lo, hi, max_tokens_per_call)
+        if world_size == 1:
+            return cls(local, identity, L)
+        import torch.distributed as dist
+
+        sizes = [shard_bounds(n, world_size, r) for r in range(world_size)]
+        m = max(h - l_ for l_, h in sizes)
+        padded = torch.zeros(m, H, dtype=torch.float32, device=dev)
+        padded[: hi - lo] = local
+        everything = torch.empty(world_size * m, H, dtype=torch.float32, device=dev)
+        dist.all_gather_into_tensor(everything, padded, group=process_group)
+        rows = torch.cat([everything[r * m: r * m + (h - l_)] for r, (l_, h) in enumerate(sizes)], dim=0)
+        return cls(rows, identity, L)
+
+
+# --------------------------------------------------------------------------------------------------
 # dataset
 # --------------------------------------------------------------------------------------------------
 class MSMarcoDataset(torch.utils.data.Dataset):
@@ -266,17 +360,21 @@ class TripletDataLoader:
 class TokenTripletLoader:
     """Token-level feeder for the fused step: shuffles pairs, samples in-batch negatives over the GLOBAL
     batch (SURVEY.md §8e), then hands this rank its contiguous slice as pinned, fixed-shape token tensors
-    (ids int32, mask uint8, padded to Lq/Ld so CUDA-graph replays see one shape)."""
+    (ids int32, mask uint8, padded to Lq/Ld so CUDA-graph replays see one shape).
+
+    rows=True yields the same batches as bank rows instead: an int32 [3, B] tensor of query-bank rows, document-bank
+    rows of the positives and document-bank rows of the negatives (for a FusedTrainer over pooled banks)."""
 
     def __init__(self, dataset: MSMarcoDataset, global_batch: int, Lq: int = 32, Ld: int = 256, rank: int = 0,
                  world_size: int = 1, seed: int = 0, drop_last: bool = True, ids_dtype=torch.int32,
-                 mask_dtype=torch.uint8):
+                 mask_dtype=torch.uint8, rows: bool = False):
         assert dataset.query_bank is not None, "TokenTripletLoader needs a token-bank dataset"
         assert global_batch % world_size == 0
         self.ds, self.gb, self.Lq, self.Ld = dataset, global_batch, Lq, Ld
         self.rank, self.world = rank, world_size
         self.rng = np.random.default_rng(seed)  # same seed on every rank -> same global batches
         self.drop_last = drop_last
+        self.rows = bool(rows)
         self.ids_dtype, self.mask_dtype = ids_dtype, mask_dtype
         self.q_idx = np.array([int(d["query"].split(":")[1]) for d in dataset.data], dtype=np.int64)
         self.d_idx = np.array([int(d["positive"].split(":")[1]) for d in dataset.data], dtype=np.int64)
@@ -293,6 +391,10 @@ class TokenTripletLoader:
             g = order[s: s + self.gb]
             neg = g[sample_negative_indices(self.qid[g], self.rng)]
             mine = slice(self.rank * per, (self.rank + 1) * per)
+            if self.rows:
+                rows = np.stack([self.q_idx[g[mine]], self.d_idx[g[mine]], self.d_idx[neg[mine]]]).astype(np.int32)
+                yield torch.from_numpy(rows)
+                continue
             kw = dict(ids_dtype=self.ids_dtype, mask_dtype=self.mask_dtype, pin=True)
             yield (self.ds.query_bank.batch(self.q_idx[g[mine]], self.Lq, self.Lq, **kw),
                    self.ds.doc_bank.batch(self.d_idx[g[mine]], self.Ld, self.Ld, **kw),
@@ -305,10 +407,13 @@ class DeviceTripletFeeder:
     token tensors of a FusedTrainer slot and draws the in-batch negatives (same rule as backend/data.py:124-137) — no
     host work and no H2D traffic per step.  Under data parallelism every rank holds the banks, uses the same epoch
     permutation (same seed) and assembles only its slice of the global batch; the negatives are a pure function of
-    (seed, position in the global batch), so the ranks agree without communicating."""
+    (seed, position in the global batch), so the ranks agree without communicating.
+
+    rows_only=True: the feeder serves only trainers over pooled banks (bank rows, `tt_assemble_triplet_rows`) and does
+    not upload the token banks."""
 
     def __init__(self, dataset: MSMarcoDataset, global_batch: int, Lq: int = 32, Ld: int = 256, device="cuda",
-                 rank: int = 0, world_size: int = 1, seed: int = 0, drop_last: bool = True):
+                 rank: int = 0, world_size: int = 1, seed: int = 0, drop_last: bool = True, rows_only: bool = False):
         assert dataset.query_bank is not None, "DeviceTripletFeeder needs a token-bank dataset"
         assert global_batch % world_size == 0 and global_batch >= 2
         try:
@@ -331,8 +436,10 @@ class DeviceTripletFeeder:
             desc = N.TokenBankDesc(flat.data_ptr(), off.data_ptr(), N.dtype_code(flat), 0)
             return flat, off, desc
 
-        self.q_flat, self.q_off, self.q_desc = upload(dataset.query_bank)
-        self.d_flat, self.d_off, self.d_desc = upload(dataset.doc_bank)
+        self.rows_only = bool(rows_only)
+        if not self.rows_only:
+            self.q_flat, self.q_off, self.q_desc = upload(dataset.query_bank)
+            self.d_flat, self.d_off, self.d_desc = upload(dataset.doc_bank)
         as_dev = lambda a: torch.from_numpy(np.asarray(a, dtype=np.int32)).to(self.device)  # noqa: E731
         self.pair_q = as_dev([int(d["query"].split(":")[1]) for d in dataset.data])
         self.pair_d = as_dev([int(d["positive"].split(":")[1]) for d in dataset.data])
@@ -357,15 +464,27 @@ class DeviceTripletFeeder:
         N = self.N
         assert self.order is not None, "call start_epoch() first"
         assert 0 <= step < len(self)
+        order = self.order[step * self.gb: (step + 1) * self.gb]
+        step_seed = (self.seed * 0x9E3779B1 + self.epoch * 0x85EBCA77 + step) & 0xFFFFFFFFFFFFFFFF
+        row_bufs = getattr(trainer, "row_bufs", None)
+        if row_bufs is not None:
+            # a trainer over pooled banks takes bank rows (same items, same negatives as the token path would give)
+            N.check(N.load().tt_assemble_triplet_rows(
+                N.ptr(self.pair_q), N.ptr(self.pair_d), N.ptr(self.pair_qid), order.data_ptr(), self.gb,
+                self.rank * self.per, self.per, step_seed, N.ptr(row_bufs[slot]), N.ptr(self.neg) if want_neg else None,
+                N.ptr(self.err), N.stream()), "tt_assemble_triplet_rows")
+            trainer._rows_loaded[slot] = True
+            return
+        if self.rows_only:
+            raise RuntimeError("DeviceTripletFeeder(rows_only=True) holds no token banks: it feeds trainers over pooled "
+                               "banks only")
         q_ids, q_mask, p_ids, p_mask, n_ids, n_mask = trainer.tok_slots[slot]
         assert tuple(q_ids.shape) == (self.per, self.Lq) and tuple(p_ids.shape) == (self.per, self.Ld)
-        order = self.order[step * self.gb: (step + 1) * self.gb]
         # a trainer that reuses the positives' pooled rows for the in-batch negatives wants their indices in its slot
         neg_bufs = getattr(trainer, "neg_bufs", None)
         neg_ptr = N.ptr(neg_bufs[slot]) if neg_bufs is not None else (N.ptr(self.neg) if want_neg else None)
         if neg_bufs is not None:
             trainer._neg_loaded[slot] = True
-        step_seed = (self.seed * 0x9E3779B1 + self.epoch * 0x85EBCA77 + step) & 0xFFFFFFFFFFFFFFFF
         N.check(N.load().tt_assemble_triplets(
             ctypes.byref(self.q_desc), ctypes.byref(self.d_desc), N.ptr(self.pair_q), N.ptr(self.pair_d),
             N.ptr(self.pair_qid), order.data_ptr(), self.gb, self.rank * self.per, self.per, step_seed, self.Lq, self.Ld,

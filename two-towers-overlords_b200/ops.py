@@ -215,19 +215,24 @@ class TripletStep:
 
     def bind(self, tokens, tables, params, grads, margin, inv_batch, grad_scale=1.0, table_grads=None):
         """tokens = (q_ids,q_mask,p_ids,p_mask,n_ids,n_mask) CUDA tensors; tables = (table_q, table_d);
-        params / grads = 8 fp32 tensors in the order Wq1,bq1,Wq2,bq2,Wd1,bd1,Wd2,bd2."""
+        params / grads = 8 fp32 tensors in the order Wq1,bq1,Wq2,bq2,Wd1,bd1,Wd2,bd2.
+        tokens and tables are None for a step that reads precomputed pooled rows only (bind_pooled)."""
         B, Lq, Ld, H, P, vocab = self.shape
-        q_ids, q_mask, p_ids, p_mask, n_ids, n_mask = tokens
-        assert tuple(q_ids.shape) == (B, Lq) and tuple(p_ids.shape) == (B, Ld) and tuple(n_ids.shape) == (B, Ld)
-        assert q_ids.dtype == p_ids.dtype == n_ids.dtype and q_mask.dtype == p_mask.dtype == n_mask.dtype
         a = self.args
-        a.q_ids, a.q_mask, a.Lq = N.ptr(q_ids), N.ptr(q_mask), Lq
-        a.p_ids, a.p_mask = N.ptr(p_ids), N.ptr(p_mask)
-        a.n_ids, a.n_mask, a.Ld = N.ptr(n_ids), N.ptr(n_mask), Ld
-        a.ids_dtype, a.mask_dtype, a.B = N.dtype_code(q_ids), N.dtype_code(q_mask), B
-        a.table_q, a.table_d = N.ptr(tables[0]), N.ptr(tables[1])
-        assert tables[0].dtype == tables[1].dtype
-        a.table_dtype, a.vocab, a.H, a.P = N.dtype_code(tables[0]), vocab, H, P
+        a.Lq, a.Ld, a.B = Lq, Ld, B
+        if tokens is not None:
+            q_ids, q_mask, p_ids, p_mask, n_ids, n_mask = tokens
+            assert tuple(q_ids.shape) == (B, Lq) and tuple(p_ids.shape) == (B, Ld) and tuple(n_ids.shape) == (B, Ld)
+            assert q_ids.dtype == p_ids.dtype == n_ids.dtype and q_mask.dtype == p_mask.dtype == n_mask.dtype
+            a.q_ids, a.q_mask = N.ptr(q_ids), N.ptr(q_mask)
+            a.p_ids, a.p_mask = N.ptr(p_ids), N.ptr(p_mask)
+            a.n_ids, a.n_mask = N.ptr(n_ids), N.ptr(n_mask)
+            a.ids_dtype, a.mask_dtype = N.dtype_code(q_ids), N.dtype_code(q_mask)
+        a.table_dtype, a.vocab, a.H, a.P = N.TT_F32, vocab, H, P
+        if tables is not None:
+            a.table_q, a.table_d = N.ptr(tables[0]), N.ptr(tables[1])
+            assert tables[0].dtype == tables[1].dtype
+            a.table_dtype = N.dtype_code(tables[0])
         for name, t in zip(("Wq1", "bq1", "Wq2", "bq2", "Wd1", "bd1", "Wd2", "bd2"), params):
             assert t.dtype == torch.float32
             setattr(a, name, N.ptr(t))
@@ -248,15 +253,17 @@ class TripletStep:
 
     def add_tokens(self, tokens) -> int:
         """Another token-buffer set sharing every other argument (rotating / double-buffered inputs);
-        returns its slot index for run(slot)."""
+        returns its slot index for run(slot).  tokens = None adds a slot of a pooled-row step (set_pooled_index)."""
         B, Lq, Ld = self.shape[:3]
-        q_ids, q_mask, p_ids, p_mask, n_ids, n_mask = tokens
-        assert tuple(q_ids.shape) == (B, Lq) and tuple(p_ids.shape) == (B, Ld) and tuple(n_ids.shape) == (B, Ld)
         a = N.StepArgs.from_buffer_copy(self.args)
-        assert N.dtype_code(q_ids) == a.ids_dtype and N.dtype_code(q_mask) == a.mask_dtype
-        a.q_ids, a.q_mask = N.ptr(q_ids), N.ptr(q_mask)
-        a.p_ids, a.p_mask = N.ptr(p_ids), N.ptr(p_mask)
-        a.n_ids, a.n_mask = N.ptr(n_ids), N.ptr(n_mask)
+        a.pooled_index = None
+        if tokens is not None:
+            q_ids, q_mask, p_ids, p_mask, n_ids, n_mask = tokens
+            assert tuple(q_ids.shape) == (B, Lq) and tuple(p_ids.shape) == (B, Ld) and tuple(n_ids.shape) == (B, Ld)
+            assert N.dtype_code(q_ids) == a.ids_dtype and N.dtype_code(q_mask) == a.mask_dtype
+            a.q_ids, a.q_mask = N.ptr(q_ids), N.ptr(q_mask)
+            a.p_ids, a.p_mask = N.ptr(p_ids), N.ptr(p_mask)
+            a.n_ids, a.n_mask = N.ptr(n_ids), N.ptr(n_mask)
         self.slots.append(a)
         self._keep.append(tokens)
         return len(self.slots) - 1
@@ -304,6 +311,28 @@ class TripletStep:
         assert neg_index.dtype == torch.int32 and neg_index.is_cuda and tuple(neg_index.shape) == (self.shape[0],)
         a.neg_index = N.ptr(neg_index)
         self._keep.append(neg_index)
+
+    def bind_pooled(self, rows_q: torch.Tensor, rows_d: torch.Tensor):
+        """Frozen front end computed once per text (tt_step_args.pooled_*): fp32 [n, H] banks of pooled rows, one per
+        tower.  Every slot then copies its 3B rows out of them by its index buffer (set_pooled_index) instead of
+        pooling tokens; the static addresses keep captured graphs valid."""
+        assert not self.train_table, "pooled rows need frozen tables"
+        H = self.shape[3]
+        for t in (rows_q, rows_d):
+            assert t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 and t.shape[1] == H and t.shape[0] >= 1
+            assert t.is_contiguous(), "pooled rows are read with a row stride of H: pass a contiguous bank"
+        for a in self.slots:
+            a.pooled_q, a.pooled_q_rows = N.ptr(rows_q), rows_q.shape[0]
+            a.pooled_d, a.pooled_d_rows = N.ptr(rows_d), rows_d.shape[0]
+        self._keep.append((rows_q, rows_d))
+
+    def set_pooled_index(self, slot: int, index: torch.Tensor):
+        """Bank rows of `slot` (tt_step_args.pooled_index): int32 [3B] on the device, query rows | positive rows |
+        negative rows."""
+        assert self.args.pooled_q is not None, "set_pooled_index needs bind_pooled() first"
+        assert index.dtype == torch.int32 and index.is_cuda and tuple(index.shape) == (3 * self.shape[0],)
+        self.slots[slot].pooled_index = N.ptr(index)
+        self._keep.append(index)
 
     def set_chain(self, mode: int):
         """tt_step_args.chain: 0 = library default (TT_CHAIN env, else the persistent kernel), 1 = persistent chain

@@ -19,6 +19,7 @@ from __future__ import annotations
 import math
 import os
 import random
+import time
 from typing import Optional, Union
 
 import numpy as np
@@ -27,13 +28,13 @@ from torch import GradScaler, autocast
 
 try:
     from . import comm, ops, retrieval
-    from .data import DeviceTripletFeeder, MSMarcoDataset, TokenTripletLoader, TripletDataLoader
+    from .data import DeviceTripletFeeder, MSMarcoDataset, PooledBank, TokenTripletLoader, TripletDataLoader
     from .model import TokenBatch, TripletLoss, TwoTowersModel
 except ImportError:
     import comm
     import ops
     import retrieval
-    from data import DeviceTripletFeeder, MSMarcoDataset, TokenTripletLoader, TripletDataLoader
+    from data import DeviceTripletFeeder, MSMarcoDataset, PooledBank, TokenTripletLoader, TripletDataLoader
     from model import TokenBatch, TripletLoss, TwoTowersModel
 
 try:  # wandb is optional at import time; only touched when logging is requested
@@ -131,7 +132,7 @@ class FusedTrainer:
                  precision: Optional[str] = None, world_size: int = 1, rank: int = 0, use_graph: bool = True,
                  betas=(0.9, 0.999), eps: float = 1e-8, process_group=None, ids_dtype=torch.int32,
                  mask_dtype=torch.uint8, token_slots: int = 1, exchange: Optional[str] = None,
-                 exchange_ctas: int = 0, in_batch_negatives: bool = False):
+                 exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None):
         qt, dt = model.query_tower, model.document_tower
         self.model = model
         self.device = qt.pretrained_model.device
@@ -144,7 +145,30 @@ class FusedTrainer:
         self.margin, self.lr, self.betas, self.eps = float(margin), float(lr), betas, float(eps)
         self.world, self.rank, self.pg = world_size, rank, process_group
         self.precision = precision or qt.precision
-        self.train_table = bool(qt.pretrained_model.table.requires_grad)
+        # pooled = (bank_q, bank_d), data.PooledBank: the frozen front end (backbone -> masked mean -> normalise) was
+        # computed once per text, so a step copies its 3B pooled rows out of the banks by index instead of pooling
+        # tokens.  This is how the MiniLM backbone trains: it has no token table to gather from.
+        self.pooled = tuple(pooled) if pooled is not None else None
+        if self.pooled is None and not hasattr(qt.pretrained_model, "table"):
+            raise ValueError("FusedTrainer: this backbone has no token table to gather from (MiniLM); encode the "
+                             "training texts once with data.PooledBank.build(tower, bank, L) for each tower and pass "
+                             "pooled=(bank_q, bank_d)")
+        if self.pooled is not None:
+            if any(p.requires_grad for t in (qt, dt) for p in t.pretrained_model.parameters()):
+                raise ValueError("FusedTrainer(pooled=...) needs a frozen backbone: pooled rows of a trainable table "
+                                 "would go stale at the first step")
+            if in_batch_negatives:
+                raise ValueError("FusedTrainer(pooled=...): the negatives are named by their own bank rows; "
+                                 "in_batch_negatives does not apply")
+            self.pooled[0].check(qt, "the query tower's pooled bank")
+            self.pooled[1].check(dt, "the document tower's pooled bank")
+            if (self.pooled[0].L, self.pooled[1].L) != (Lq, Ld):
+                raise ValueError(f"FusedTrainer(pooled=...): the banks truncate texts to {self.pooled[0].L} / "
+                                 f"{self.pooled[1].L} tokens, the trainer to Lq = {Lq} / Ld = {Ld}; build them with the "
+                                 "trainer's lengths")
+            self.train_table = False
+        else:
+            self.train_table = bool(qt.pretrained_model.table.requires_grad)
         params = model.projection_parameters()
         sizes = [p.numel() for p in params]
         self.n_param = sum(sizes)
@@ -202,9 +226,17 @@ class FusedTrainer:
 
         # token_slots > 1: rotating input buffers (prefetch step i+1 while step i computes; each slot has
         # its own captured graph because a graph replays fixed addresses)
-        sets = [new_set() for _ in range(max(1, token_slots))]
-        self.tok_bufs = [b for b, _ in sets]
-        self.tok_slots = [v for _, v in sets]
+        n_slots = max(1, token_slots)
+        self.row_bufs = None
+        if self.pooled is None:
+            sets = [new_set() for _ in range(n_slots)]
+            self.tok_bufs = [b for b, _ in sets]
+            self.tok_slots = [v for _, v in sets]
+        else:  # no token buffers: a slot is the int32 [3B] bank rows of its batch (q | p | n), see load_rows()
+            self.tok_bufs = []
+            self.tok_slots = [None] * n_slots
+            self.row_bufs = [torch.zeros(3 * batch_size, dtype=torch.int32, device=dev) for _ in range(n_slots)]
+            self._rows_loaded = [False] * n_slots  # step() refuses a slot whose rows were never given
         self.tok = self.tok_slots[0]
         self.table_grads = None
         if self.train_table:
@@ -230,10 +262,15 @@ class FusedTrainer:
             so = ops.TripletStep(batch_size, Lq, Ld, self.H, self.P, self.vocab, self.precision, dev,
                                  train_table=self.train_table)
             so.loss = self.flat_g[self.n_param:]  # this rank's loss term lands in the flat gradient's last slot
-            so.bind(self.tok, (qt.pretrained_model.table.data, dt.pretrained_model.table.data), self.p_views,
-                    self.g_views, self.margin, 1.0 / (batch_size * world_size), 1.0, self.table_grads)
+            tables = None if self.pooled else (qt.pretrained_model.table.data, dt.pretrained_model.table.data)
+            so.bind(self.tok, tables, self.p_views, self.g_views, self.margin, 1.0 / (batch_size * world_size), 1.0,
+                    self.table_grads)
             for toks in self.tok_slots[1:]:
                 so.add_tokens(toks)
+            if self.pooled:
+                so.bind_pooled(self.pooled[0].rows, self.pooled[1].rows)
+                for slot, buf in enumerate(self.row_bufs):
+                    so.set_pooled_index(slot, buf)
             so.set_chain(self.chain_mode)
             if self.exchange == "none" and self.world == 1:
                 # single GPU: torch.optim.Adam rides inside the step call (the tail of the persistent chain kernel
@@ -316,6 +353,27 @@ class FusedTrainer:
         for dst, src in zip(self.tok_slots[slot], (q.input_ids, q.attention_mask, p.input_ids, p.attention_mask,
                                                    n.input_ids, n.attention_mask)):
             dst.copy_(src, non_blocking=True)
+
+    def load_rows(self, rows: torch.Tensor, slot: int = 0):
+        """Bank rows of the batch in `slot` for a trainer over pooled banks: int [3, B] or [3B] (query rows | positive
+        rows | negative rows; host or device), async on the current stream."""
+        if self.row_bufs is None:
+            raise RuntimeError("FusedTrainer.load_rows needs a trainer built with pooled=(bank_q, bank_d)")
+        self.row_bufs[slot].copy_(rows.reshape(-1).to(torch.int32), non_blocking=True)
+        self._rows_loaded[slot] = True
+
+    def check_banks(self):
+        """Raises if a pooled bank no longer matches its tower's backbone (weights changed after the build): a stale
+        bank must never train silently.  Called by prepare() and at the start of every epoch."""
+        if self.pooled is not None:
+            self.pooled[0].check(self.model.query_tower, "the query tower's pooled bank")
+            self.pooled[1].check(self.model.document_tower, "the document tower's pooled bank")
+
+    def _load(self, batch, slot: int):
+        if self.pooled is not None:
+            self.load_rows(batch, slot)
+        else:
+            self.load_tokens(*batch, slot=slot)
 
     def load_neg_index(self, neg_index: torch.Tensor, slot: int = 0):
         """Indices of the in-batch negatives of the batch in `slot` (int [B]; host or device), async on the current stream."""
@@ -435,6 +493,7 @@ class FusedTrainer:
     def prepare(self, n_slots: Optional[int] = None):
         """Captures the steady-state graphs of a round-robin schedule over the first `n_slots` token slots
         (step(s, (s + 1) % n_slots)), so no capture happens inside a timed region."""
+        self.check_banks()
         n = n_slots or len(self.tok_slots)
         if not self.use_graph:
             return
@@ -458,6 +517,9 @@ class FusedTrainer:
         if self.neg_bufs is not None and not self._neg_loaded[slot]:
             raise RuntimeError(f"FusedTrainer(in_batch_negatives=True): no negative indices were loaded for slot {slot} "
                                "(load_neg_index / DeviceTripletFeeder.assemble)")
+        if self.row_bufs is not None and not self._rows_loaded[slot]:
+            raise RuntimeError(f"FusedTrainer(pooled=...): no bank rows were loaded for slot {slot} "
+                               "(load_rows / DeviceTripletFeeder.assemble)")
         if self.train_table:
             next_slot = None  # a trainable table changes between steps: its gather cannot run ahead of the update
         lib = ops.N.load()
@@ -496,6 +558,7 @@ class FusedTrainer:
         steps = len(feeder)
         if steps == 0:
             raise ZeroDivisionError("FusedTrainer.train_epoch_device: not enough pairs for one batch")
+        self.check_banks()
         feeder.start_epoch()
         total = torch.zeros((), dtype=torch.float64, device=self.device)
         n_slots = len(self.tok_slots)
@@ -538,7 +601,25 @@ class FusedTrainer:
                 "steps_done": self.steps_done, "lr": self.lr, "betas": tuple(self.betas), "eps": self.eps}
 
     def load_state_dict(self, sd: dict):
-        self.model.load_state_dict(sd["model"])  # in-place copies: the parameters keep aliasing the flat buffer
+        model_sd = sd["model"]
+        if self.pooled is not None:
+            # The pooled banks were computed from the frozen backbone and are keyed to its tensors' versions: copying the
+            # backbone in place, even with equal values, would make them stale.  A checkpoint of this training run holds
+            # the same backbone, so equal tensors are left untouched; a different backbone would need new banks.
+            cur = self.model.state_dict()
+            frozen = [k for k in model_sd if k.split(".", 2)[1:2] == ["pretrained_model"]]
+            differ = [k for k in frozen if k not in cur or not torch.equal(cur[k].cpu(), model_sd[k].cpu())]
+            if differ:
+                raise RuntimeError(f"FusedTrainer(pooled=...): the checkpoint's backbone differs from the model's "
+                                   f"({len(differ)} tensors, e.g. {differ[0]}); the pooled banks would be stale. Load it "
+                                   "into the model first, rebuild the banks with PooledBank.build() and a new trainer")
+            model_sd = {k: v for k, v in model_sd.items() if k not in set(frozen)}
+            missing, unexpected = self.model.load_state_dict(model_sd, strict=False)
+            if unexpected or set(missing) - set(frozen):
+                raise RuntimeError(f"FusedTrainer.load_state_dict: missing keys {sorted(set(missing) - set(frozen))}, "
+                                   f"unexpected keys {sorted(unexpected)}")
+        else:
+            self.model.load_state_dict(model_sd)  # in-place copies: the parameters keep aliasing the flat buffer
         self.exp_avg.copy_(sd["exp_avg"])
         self.exp_avg_sq.copy_(sd["exp_avg_sq"])
         if self.xchg is not None:
@@ -583,6 +664,7 @@ class FusedTrainer:
     def train_epoch(self, loader: TokenTripletLoader, log_every: int = 0) -> float:
         """One pass over the loader.  With >= 2 token slots the next batch is staged one step ahead so that its
         pooled gather overlaps the current step."""
+        self.check_banks()
         total = torch.zeros((), dtype=torch.float64, device=self.device)
         nb = 0
         n_slots = len(self.tok_slots)
@@ -591,13 +673,13 @@ class FusedTrainer:
         if cur is None:
             raise ZeroDivisionError("FusedTrainer.train_epoch: empty loader")
         slot = 0
-        self.load_tokens(*cur, slot=slot)
+        self._load(cur, slot)
         while cur is not None:
             nxt = next(it, None)
             nslot = None
             if nxt is not None and n_slots >= 2 and len(nxt[0]) == self.B:
                 nslot = (slot + 1) % n_slots
-                self.load_tokens(*nxt, slot=nslot)
+                self._load(nxt, nslot)
             loss = self.step(slot, nslot)
             total += loss.double()
             nb += 1
@@ -606,7 +688,7 @@ class FusedTrainer:
                     print(f"Batch {nb}, Loss: {loss.item():.4f}")
                 self.check()
             if nxt is not None and nslot is None:
-                self.load_tokens(*nxt, slot=slot)
+                self._load(nxt, slot)
             else:
                 slot = nslot if nslot is not None else slot
             cur = nxt
@@ -904,10 +986,20 @@ def run_training(
     run_comprehensive_test: bool = True,
     fused: Optional[bool] = None,
     table_dtype: torch.dtype = torch.float32,
+    backbone: Optional[str] = None,
 ) -> TwoTowersModel:
     """Main training function (training.py:383-529).  `fused` (additive) selects the FusedTrainer; by
     default it is used whenever the dataset is token-bank backed and no gradient accumulation / wandb
-    gradient hooks require the reference-shaped loop."""
+    gradient hooks require the reference-shaped loop.
+
+    `backbone` (additive): "table" (the token-table backbone) or "minilm" (the reference's frozen MiniLM encoder);
+    None reads the TT_BACKBONE environment variable, default "table", so an unmodified main.py can choose.  On the
+    fused path a MiniLM model encodes every text of the training split once into pooled banks (data.PooledBank) and
+    trains the projections on rows gathered from them; otherwise it runs the reference-shaped loop."""
+    if backbone is None:
+        backbone = os.environ.get("TT_BACKBONE", "table")
+    if backbone not in ("table", "minilm"):
+        raise ValueError(f"backbone must be 'table' or 'minilm', got {backbone!r}")
     # one process per GPU under torchrun / torch.distributed.run (SURVEY.md §8e): `batch_size` is the GLOBAL batch,
     # every rank trains on its contiguous slice and evaluates its shard of the documents
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -948,7 +1040,10 @@ def run_training(
         if not wandb.run:
             wandb.init(project=project_name, config=config)
 
-    model = TwoTowersModel(projection_dim=projection_dim, table_dtype=table_dtype).to(device)
+    if backbone == "minilm":
+        model = TwoTowersModel(projection_dim=projection_dim, backbone="minilm").to(device)
+    else:
+        model = TwoTowersModel(projection_dim=projection_dim, table_dtype=table_dtype).to(device)
     if world > 1:  # random-init tables and projections are drawn per process: rank 0's become everybody's
         for t in list(model.parameters()) + list(model.buffers()):
             dist.broadcast(t.data, src=0)
@@ -997,19 +1092,31 @@ def run_training(
         if world > 1:  # the epoch permutation and the in-batch negatives are functions of this seed: share rank 0's
             dist.broadcast_object_list(seed_box, src=0)
         host_feeder = os.environ.get("TT_HOST_FEEDER") == "1" or len(train_ds) < 2 * batch_size
-        # the device feeder draws the in-batch negatives itself and hands their indices to the trainer, which then pools
-        # every positive document once (TT_NEG_REUSE=0: gather the negatives' tokens like any document)
-        reuse = (not host_feeder and world == 1 and os.environ.get("TT_NEG_REUSE", "1") != "0"
-                 and not model.query_tower.pretrained_model.table.requires_grad)
-        trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, token_slots=2, world_size=world,
-                               rank=rank, in_batch_negatives=reuse)
+        if backbone == "minilm":
+            # the frozen encoder runs once per training text, not three times per triplet and step
+            t0 = time.perf_counter()
+            Lq, Ld = 32, 256  # FusedTrainer's token lengths
+            banks = (PooledBank.build(model.query_tower, train_ds.query_bank, Lq, world_size=world, rank=rank),
+                     PooledBank.build(model.document_tower, train_ds.doc_bank, Ld, world_size=world, rank=rank))
+            torch.cuda.synchronize()
+            say(f"Encoded {len(banks[0]) + len(banks[1])} training texts ({len(banks[0])} queries, "
+                f"{len(banks[1])} passages) with the frozen MiniLM backbone in {time.perf_counter() - t0:.1f}s")
+            trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, Lq, Ld, token_slots=2,
+                                   world_size=world, rank=rank, pooled=banks)
+        else:
+            # the device feeder draws the in-batch negatives itself and hands their indices to the trainer, which then
+            # pools every positive document once (TT_NEG_REUSE=0: gather the negatives' tokens like any document)
+            reuse = (not host_feeder and world == 1 and os.environ.get("TT_NEG_REUSE", "1") != "0"
+                     and not model.query_tower.pretrained_model.table.requires_grad)
+            trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, token_slots=2, world_size=world,
+                                   rank=rank, in_batch_negatives=reuse)
         if host_feeder:
             # host-assembled batches (negatives drawn over the global batch, this rank's slice)
             token_dl = TokenTripletLoader(train_ds, batch_size, trainer.Lq, trainer.Ld, rank=rank, world_size=world,
-                                          seed=seed_box[0])
+                                          seed=seed_box[0], rows=trainer.pooled is not None)
         else:  # token bank resident in HBM, batches (and in-batch negatives) assembled by one kernel per step
             feeder = DeviceTripletFeeder(train_ds, batch_size, trainer.Lq, trainer.Ld, device, rank=rank,
-                                         world_size=world, seed=seed_box[0])
+                                         world_size=world, seed=seed_box[0], rows_only=trainer.pooled is not None)
         trainer.prepare(2)
 
     say(f"Starting training for {num_epochs} epochs...")
