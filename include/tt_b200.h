@@ -335,6 +335,48 @@ int tt_assemble_triplet_rows(const int32_t* pair_q, const int32_t* pair_d, const
                              int32_t* rows_out, int32_t* neg_out, int* err_flag, tt_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Hard negatives mined with the corpus scan (DPR / ANCE style): the passages the current towers rank highest for a
+ * query that are not its positives.
+ *
+ * tt_mine_negatives: top_id [Q,k] i64 = tt_scan_topk / tt_topk_merge lists of query-bank rows (score desc, id asc,
+ * -1 padding); excl_offsets [Q+1] i64 / excl_ids i32 = CSR exclusion list of every query, sorted ascending within
+ * each query.  Each list is walked in rank order, every id of the query's exclusion list is dropped, the first `skip`
+ * survivors are dropped, and the next up to `depth` survivors are written in rank order to table_out [Q,depth] i32;
+ * count_out [Q] i32 = how many were written, the rest of the row is -1.  Needs 1 <= depth, 0 <= skip,
+ * skip + depth <= k <= 32.
+ *
+ * tt_assemble_triplets_mined / tt_assemble_triplet_rows_mined: tt_assemble_triplets / tt_assemble_triplet_rows whose
+ * item i may take its negative from the table instead.  With qrow = pair_q[order[i]], x ^ y bitwise xor, u >> s a
+ * logical shift, all arithmetic on uint64 mod 2^64 and splitmix64 as in the in-batch draw:
+ *   h0 = splitmix64(seed ^ 0x6A09E667F3BCC909 ^ (i * 0x9E6C63D0676A9A99)),  h1 = splitmix64(h0),  h2 = splitmix64(h1)
+ *   hard = count[qrow] > 0  and  float(h1 >> 40) < ratio * 2^24           (fp32 compare, both sides exact)
+ *   hard item:  negative = document row table[qrow][(h2 >> 32) mod count[qrow]],  neg_out[i - row0] = -1
+ *   otherwise:  the in-batch draw of tt_assemble_triplets, unchanged (neg_out = its item j)
+ * so ratio = 0, or all counts 0, gives the batches of the entry points without _mined bit for bit, and every rank of
+ * a data-parallel job draws the same negatives.  A qrow outside [0, n_rows), a count above depth or a table entry
+ * outside [0, n_docs) sets err_flag to 3 and the item falls back to its in-batch draw.
+ * ---------------------------------------------------------------------------------------- */
+typedef struct tt_mined_negatives {
+  const int32_t* table;   /* [n_rows, depth] document-bank rows, device */
+  const int32_t* count;   /* [n_rows] valid entries per row, device     */
+  int depth;
+  int n_rows;             /* query-bank rows                            */
+  int n_docs;             /* document-bank rows                         */
+  float ratio;            /* probability of a hard negative, [0, 1]     */
+} tt_mined_negatives;
+int tt_mine_negatives(const int64_t* top_id, int Q, int k, const int64_t* excl_offsets, const int32_t* excl_ids,
+                      int skip, int depth, int32_t* table_out, int32_t* count_out, tt_stream_t stream);
+int tt_assemble_triplets_mined(const tt_token_bank* qbank, const tt_token_bank* dbank, const int32_t* pair_q,
+                               const int32_t* pair_d, const int32_t* pair_qid, const int32_t* order, int Bg, int row0,
+                               int B, uint64_t seed, int Lq, int Ld, void* q_ids, void* q_mask, void* p_ids,
+                               void* p_mask, void* n_ids, void* n_mask, int ids_dtype, int mask_dtype, int32_t* neg_out,
+                               int* err_flag, const tt_mined_negatives* mined, tt_stream_t stream);
+int tt_assemble_triplet_rows_mined(const int32_t* pair_q, const int32_t* pair_d, const int32_t* pair_qid,
+                                   const int32_t* order, int Bg, int row0, int B, uint64_t seed, int32_t* rows_out,
+                                   int32_t* neg_out, int* err_flag, const tt_mined_negatives* mined,
+                                   tt_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Measurement probe (bench.py): L2 -> SM read bandwidth.  Every SM streams `buf` (`bytes` long, cache-resident
  * when it fits the 126 MB L2) `iters` times with coalesced 16-byte loads at full occupancy; the caller times the
  * launch with CUDA events: GB/s = bytes * iters / seconds.  This is the ceiling of the pooled gather, whose token

@@ -40,6 +40,11 @@ class TokenBankDesc(ctypes.Structure):
     _fields_ = [("flat", c_void_p), ("offsets", c_void_p), ("dtype", c_int), ("_pad", c_int)]
 
 
+class MinedNegatives(ctypes.Structure):
+    _fields_ = [("table", c_void_p), ("count", c_void_p), ("depth", c_int), ("n_rows", c_int), ("n_docs", c_int),
+                ("ratio", c_float)]
+
+
 class StepArgs(ctypes.Structure):
     _fields_ = [
         ("q_ids", c_void_p), ("q_mask", c_void_p), ("Lq", c_int),
@@ -131,6 +136,15 @@ _SIGNATURES = {
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "tt_assemble_triplet_rows": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, ctypes.c_uint64,
                                          c_void_p, c_void_p, c_void_p, c_void_p]),
+    "tt_mine_negatives": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p,
+                                  c_void_p]),
+    "tt_assemble_triplets_mined": (c_int, [POINTER(TokenBankDesc), POINTER(TokenBankDesc), c_void_p, c_void_p,
+                                           c_void_p, c_void_p, c_int, c_int, c_int, ctypes.c_uint64, c_int, c_int,
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                           c_void_p, c_void_p, POINTER(MinedNegatives), c_void_p]),
+    "tt_assemble_triplet_rows_mined": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                               ctypes.c_uint64, c_void_p, c_void_p, c_void_p, POINTER(MinedNegatives),
+                                               c_void_p]),
     "tt_encoder_ws_bytes": (c_size_t, [c_int, c_int, c_int]),
     "tt_encoder_fwd": (c_int, [POINTER(EncoderWeights), c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p,
                                c_void_p, c_size_t, c_void_p]),

@@ -12,6 +12,8 @@ Datasets and triplet batching — drop-in for the reference's backend/data.py su
                           `tower.tokenizer` and returns the HF call's dict (model.py:43-45).
   * TokenTripletLoader    yields device-resident (q,p,n) TokenBatches for the fused step; with
                           world_size > 1 each rank receives its contiguous slice of the global batch.
+  * HardNegativeMiner     per-query tables of hard negatives mined with the corpus scan from the current towers,
+                          drawn by DeviceTripletFeeder beside the in-batch negatives.
 """
 from __future__ import annotations
 
@@ -25,8 +27,10 @@ import numpy as np
 import torch
 
 try:
+    from . import ops
     from .model import TokenBatch, VOCAB_SIZE
 except ImportError:
+    import ops
     from model import TokenBatch, VOCAB_SIZE
 
 MsMarcoDatasetItem = dict[str, Union[str, int]]
@@ -401,6 +405,158 @@ class TokenTripletLoader:
                    self.ds.doc_bank.batch(self.d_idx[neg[mine]], self.Ld, self.Ld, **kw))
 
 
+def exclusion_csr(pair_q: np.ndarray, pair_d: np.ndarray, pair_qid: np.ndarray, n_rows: int):
+    """Positives of every query-bank row as CSR (offsets int64 [n_rows + 1], ids int32 sorted and unique per row).
+    Row r excludes every pair_d[i] whose pair_qid[i] is the query id of some pair naming row r: the in-batch draw's
+    rule ("a different query_id") applied to mined passages."""
+    pair_q, pair_d = np.asarray(pair_q, dtype=np.int64), np.asarray(pair_d, dtype=np.int64)
+    _, qid = np.unique(np.asarray(pair_qid), return_inverse=True)  # query ids renumbered 0 .. n_qid-1
+    qid = qid.reshape(-1).astype(np.int64)
+    n_qid, n_d = int(qid.max(initial=-1)) + 1, max(int(pair_d.max(initial=-1)) + 1, 1)
+    # the pairs grouped by query id: group g is by_qid[starts[g] : starts[g + 1]]
+    by_qid = np.argsort(qid, kind="stable")
+    starts = np.searchsorted(qid[by_qid], np.arange(n_qid + 1))
+    # every distinct (row, query id), expanded to every passage of that query id
+    rq = np.unique(pair_q * max(n_qid, 1) + qid)
+    rows, groups = rq // max(n_qid, 1), rq % max(n_qid, 1)
+    per = starts[groups + 1] - starts[groups]
+    within = np.arange(int(per.sum())) - np.repeat(np.cumsum(per) - per, per)
+    passages = pair_d[by_qid[np.repeat(starts[groups], per) + within]]
+    keys = np.unique(np.repeat(rows, per) * n_d + passages)  # sorted by row, then passage
+    counts = np.bincount(keys // n_d, minlength=n_rows)[:n_rows]
+    return np.concatenate([[0], np.cumsum(counts)]).astype(np.int64), (keys % n_d).astype(np.int32)
+
+
+class HardNegativeMiner:
+    """Hard negatives for DeviceTripletFeeder, mined with the exact corpus scan from the current towers (DPR / ANCE):
+    for every query-bank row, the passages the towers rank highest that are not its positives.
+
+    refresh(model) projects every pooled row of both banks with the current weights, ranks all passages for all
+    queries with the tensor-core scan (this rank's document shard, then the merge every data-parallel rank ends
+    identical on), drops each query's positives and the first `skip` survivors and keeps the next `depth` in rank
+    order (tt_mine_negatives).  The table lives in static device buffers; a feeder with `hard_negatives = miner` then
+    gives each item a mined negative with probability `ratio` (tt_assemble_*_mined).  The table is a function of the
+    weights, so a checkpoint needs no extra state.  Needs frozen backbones: the banks hold their pooled rows."""
+
+    def __init__(self, dataset: MSMarcoDataset, bank_q: "PooledBank", bank_d: "PooledBank", depth: int = 8,
+                 skip: int = 0, ratio: float = 0.5, k_scan: int = 32, world_size: int = 1, rank: int = 0,
+                 process_group=None):
+        self.depth, self.skip, self.ratio, self.k_scan = self.check_config(depth, skip, ratio, k_scan)
+        if dataset.query_bank is None:
+            raise ValueError("HardNegativeMiner needs a token-bank dataset")
+        if (len(bank_q), len(bank_d)) != (len(dataset.query_bank), len(dataset.doc_bank)):
+            raise ValueError(f"HardNegativeMiner: the pooled banks hold {len(bank_q)} / {len(bank_d)} rows, the "
+                             f"dataset's token banks {len(dataset.query_bank)} / {len(dataset.doc_bank)}; build them "
+                             "from the same dataset")
+        self.bank_q, self.bank_d = bank_q, bank_d
+        self.world, self.rank, self.pg = int(world_size), int(rank), process_group
+        pq = np.array([int(d["query"].split(":")[1]) for d in dataset.data], dtype=np.int64)
+        pd = np.array([int(d["positive"].split(":")[1]) for d in dataset.data], dtype=np.int64)
+        qid = np.array([int(d["query_id"]) for d in dataset.data], dtype=np.int64)
+        self.n_rows, self.n_docs = len(bank_q), len(bank_d)
+        off, ids = exclusion_csr(pq, pd, qid, self.n_rows)
+        dev = bank_q.rows.device
+        self.excl_offsets = torch.from_numpy(off).to(dev)
+        self.excl_ids = torch.from_numpy(ids).to(dev)
+        self.table = torch.full((self.n_rows, self.depth), -1, dtype=torch.int32, device=dev)
+        self.count = torch.zeros(self.n_rows, dtype=torch.int32, device=dev)
+        self.refreshed = False
+
+    @staticmethod
+    def check_config(depth, skip, ratio, k_scan):
+        depth, skip, k_scan, ratio = int(depth), int(skip), int(k_scan), float(ratio)
+        if not 1 <= k_scan <= 32:
+            raise ValueError(f"HardNegativeMiner: k_scan = {k_scan}; the corpus scan keeps at most 32 per query")
+        if depth < 1 or skip < 0 or skip + depth > k_scan:
+            raise ValueError(f"HardNegativeMiner: need depth >= 1, skip >= 0 and skip + depth <= k_scan (depth {depth}, "
+                             f"skip {skip}, k_scan {k_scan})")
+        if not 0.0 <= ratio <= 1.0:
+            raise ValueError(f"HardNegativeMiner: ratio = {ratio} is a probability, outside [0, 1]")
+        return depth, skip, ratio, k_scan
+
+    def _check_towers(self, model):
+        qt, dt = model.query_tower, model.document_tower
+        if any(p.requires_grad for t in (qt, dt) for p in t.pretrained_model.parameters()):
+            raise ValueError("HardNegativeMiner needs frozen backbones: the pooled banks of a trainable table go stale "
+                             "at the first step")
+        self.bank_q.check(qt, "the query tower's pooled bank")
+        self.bank_d.check(dt, "the document tower's pooled bank")
+
+    @staticmethod
+    def _project(tower, rows: torch.Tensor, chunk: int = 1 << 16) -> torch.Tensor:
+        p0, p2 = tower.projection[0], tower.projection[2]
+        out = torch.empty(rows.shape[0], p0.out_features, dtype=torch.float32, device=rows.device)
+        with torch.no_grad():
+            for s in range(0, rows.shape[0], chunk):
+                out[s: s + chunk] = ops.mlp(rows[s: s + chunk], p0.weight, p0.bias, p2.weight, p2.bias, tower.precision)
+        return out
+
+    def local_lists(self, model, events=None):
+        """Top-k_scan (scores, global ids) of every query over this rank's document shard (id_base = lo)."""
+        try:
+            from .retrieval import shard_bounds
+        except ImportError:
+            from retrieval import shard_bounds
+        self._check_towers(model)
+        ev = events if events is not None else {}
+        mark = lambda name: ev.setdefault(name, torch.cuda.Event(enable_timing=True)).record()  # noqa: E731
+        lo, hi = shard_bounds(self.n_docs, self.world, self.rank)
+        mark("start")
+        yq = self._project(model.query_tower, self.bank_q.rows)
+        yd = self._project(model.document_tower, self.bank_d.rows[lo:hi])
+        mark("project")
+        Qn, Qb = ops.l2_normalize_rows(yq, want_bf16=True)
+        Dn, Db = ops.l2_normalize_rows(yd, want_bf16=True)
+        del yq, yd
+        mark("normalize")
+        if hi > lo:
+            top = ops.scan_topk(Qn, Dn, k=self.k_scan, id_base=lo, precision="bf16", Qb=Qb, Db=Db)
+        else:  # an empty shard (more ranks than passages)
+            top = (torch.full((self.n_rows, self.k_scan), -math.inf, device=Qn.device),
+                   torch.full((self.n_rows, self.k_scan), -1, dtype=torch.int64, device=Qn.device))
+        mark("scan")
+        return top
+
+    def filter(self, top_id: torch.Tensor):
+        """Merged lists [n_rows, k_scan] -> the table and counts (tt_mine_negatives), in place."""
+        ops.mine_negatives(top_id, self.excl_offsets, self.excl_ids, self.skip, self.depth, self.table, self.count)
+        self.refreshed = True
+
+    def refresh(self, model) -> dict:
+        """Re-mines the table from the model's current weights (current stream; ends in a host sync).  Returns the
+        seconds of each phase (device events) and the table's mean count and number of empty rows."""
+        try:
+            from .retrieval import gather_and_merge
+        except ImportError:
+            from retrieval import gather_and_merge
+        ev = {}
+        top_s, top_i = self.local_lists(model, ev)
+        top_s, top_i = gather_and_merge(top_s, top_i, self.world, self.pg)
+        ev.setdefault("merge", torch.cuda.Event(enable_timing=True)).record()
+        self.filter(top_i)
+        ev.setdefault("filter", torch.cuda.Event(enable_timing=True)).record()
+        del top_s, top_i
+        ev["filter"].synchronize()
+        names = ["start", "project", "normalize", "scan", "merge", "filter"]
+        stats = {f"{b}_s": ev[a].elapsed_time(ev[b]) / 1e3 for a, b in zip(names, names[1:])}
+        stats["total_s"] = ev["start"].elapsed_time(ev["filter"]) / 1e3
+        cnt = self.count.double()
+        stats["mean_count"] = float(cnt.mean()) if self.n_rows else 0.0
+        stats["empty_queries"] = int((self.count == 0).sum())
+        return stats
+
+    def descriptor(self):
+        """tt_mined_negatives of the current table (ctypes), or None before the first refresh."""
+        if not self.refreshed:
+            return None
+        try:
+            from . import _native as N
+        except ImportError:
+            import _native as N
+        return N.MinedNegatives(self.table.data_ptr(), self.count.data_ptr(), self.depth, self.n_rows, self.n_docs,
+                                self.ratio)
+
+
 class DeviceTripletFeeder:
     """Batch assembly on the device (SURVEY.md §8f rank 1): the tokenised dataset lives in HBM as two ragged token
     banks; every step ONE kernel (`tt_assemble_triplets`) turns a slice of the epoch permutation into the six padded
@@ -450,6 +606,9 @@ class DeviceTripletFeeder:
         self.neg = torch.zeros(self.per, dtype=torch.int32, device=self.device)
         self.order = None
         self.epoch = 0
+        self.n_rows, self.n_docs = len(dataset.query_bank), len(dataset.doc_bank)
+        # a HardNegativeMiner: once its table is refreshed, items draw mined negatives (tt_assemble_*_mined)
+        self.hard_negatives: Optional[HardNegativeMiner] = None
 
     def __len__(self):
         return self.n // self.gb
@@ -466,13 +625,18 @@ class DeviceTripletFeeder:
         assert 0 <= step < len(self)
         order = self.order[step * self.gb: (step + 1) * self.gb]
         step_seed = (self.seed * 0x9E3779B1 + self.epoch * 0x85EBCA77 + step) & 0xFFFFFFFFFFFFFFFF
+        mined = self._mined_descriptor(trainer)
         row_bufs = getattr(trainer, "row_bufs", None)
         if row_bufs is not None:
             # a trainer over pooled banks takes bank rows (same items, same negatives as the token path would give)
-            N.check(N.load().tt_assemble_triplet_rows(
-                N.ptr(self.pair_q), N.ptr(self.pair_d), N.ptr(self.pair_qid), order.data_ptr(), self.gb,
-                self.rank * self.per, self.per, step_seed, N.ptr(row_bufs[slot]), N.ptr(self.neg) if want_neg else None,
-                N.ptr(self.err), N.stream()), "tt_assemble_triplet_rows")
+            args = (N.ptr(self.pair_q), N.ptr(self.pair_d), N.ptr(self.pair_qid), order.data_ptr(), self.gb,
+                    self.rank * self.per, self.per, step_seed, N.ptr(row_bufs[slot]),
+                    N.ptr(self.neg) if want_neg else None, N.ptr(self.err))
+            if mined is None:
+                N.check(N.load().tt_assemble_triplet_rows(*args, N.stream()), "tt_assemble_triplet_rows")
+            else:
+                N.check(N.load().tt_assemble_triplet_rows_mined(*args, ctypes.byref(mined), N.stream()),
+                        "tt_assemble_triplet_rows_mined")
             trainer._rows_loaded[slot] = True
             return
         if self.rows_only:
@@ -485,14 +649,34 @@ class DeviceTripletFeeder:
         neg_ptr = N.ptr(neg_bufs[slot]) if neg_bufs is not None else (N.ptr(self.neg) if want_neg else None)
         if neg_bufs is not None:
             trainer._neg_loaded[slot] = True
-        N.check(N.load().tt_assemble_triplets(
-            ctypes.byref(self.q_desc), ctypes.byref(self.d_desc), N.ptr(self.pair_q), N.ptr(self.pair_d),
-            N.ptr(self.pair_qid), order.data_ptr(), self.gb, self.rank * self.per, self.per, step_seed, self.Lq, self.Ld,
-            N.ptr(q_ids), N.ptr(q_mask), N.ptr(p_ids), N.ptr(p_mask), N.ptr(n_ids), N.ptr(n_mask), N.dtype_code(q_ids),
-            N.dtype_code(q_mask), neg_ptr, N.ptr(self.err), N.stream()),
-            "tt_assemble_triplets")
+        args = (ctypes.byref(self.q_desc), ctypes.byref(self.d_desc), N.ptr(self.pair_q), N.ptr(self.pair_d),
+                N.ptr(self.pair_qid), order.data_ptr(), self.gb, self.rank * self.per, self.per, step_seed, self.Lq,
+                self.Ld, N.ptr(q_ids), N.ptr(q_mask), N.ptr(p_ids), N.ptr(p_mask), N.ptr(n_ids), N.ptr(n_mask),
+                N.dtype_code(q_ids), N.dtype_code(q_mask), neg_ptr, N.ptr(self.err))
+        if mined is None:
+            N.check(N.load().tt_assemble_triplets(*args, N.stream()), "tt_assemble_triplets")
+        else:
+            N.check(N.load().tt_assemble_triplets_mined(*args, ctypes.byref(mined), N.stream()),
+                    "tt_assemble_triplets_mined")
+
+    def _mined_descriptor(self, trainer):
+        """tt_mined_negatives of the attached miner once it has a table, else None (in-batch negatives only)."""
+        miner = self.hard_negatives
+        if miner is None:
+            return None
+        if getattr(trainer, "neg_bufs", None) is not None:
+            raise ValueError("a trainer built with in_batch_negatives=True cannot take mined negatives: a mined negative "
+                             "is not a positive of the batch")
+        if (miner.n_rows, miner.n_docs) != (self.n_rows, self.n_docs):
+            raise ValueError(f"the miner's table covers {miner.n_rows} queries / {miner.n_docs} passages, the feeder's "
+                             f"dataset {self.n_rows} / {self.n_docs}")
+        return miner.descriptor()
 
     def check(self):
-        """Host sync: raises if some item had no eligible in-batch negative (the reference would loop forever)."""
-        if int(self.err.item()) != 0:
+        """Host sync: raises if some item had no eligible in-batch negative (the reference would loop forever), or a
+        mined negative was out of range."""
+        err = int(self.err.item())
+        if err == 3:
+            raise ValueError("a mined negative or its query row was outside the banks")
+        if err != 0:
             raise ValueError("batch has an item with no in-batch negative (all query_ids equal)")

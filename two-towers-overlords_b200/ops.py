@@ -462,6 +462,23 @@ def topk_merge(parts_s, parts_i):
     return top_s, top_i
 
 
+def mine_negatives(top_id, excl_offsets, excl_ids, skip: int, depth: int, table=None, count=None):
+    """tt_mine_negatives: scan lists top_id [Q,k] i64 minus each query's exclusion list (CSR, offsets i64 [Q+1], ids
+    i32 sorted per query), `skip` survivors dropped, the next `depth` kept in rank order -> (table [Q,depth] i32,
+    count [Q] i32).  table / count: optional preallocated outputs."""
+    N.ensure_sm100()
+    Q, k = top_id.shape
+    dev = top_id.device
+    table = torch.empty(Q, depth, dtype=torch.int32, device=dev) if table is None else table
+    count = torch.empty(Q, dtype=torch.int32, device=dev) if count is None else count
+    assert table.dtype == count.dtype == torch.int32 and tuple(table.shape) == (Q, depth) and tuple(count.shape) == (Q,)
+    excl_ids = excl_ids if excl_ids.numel() > 0 else torch.zeros(1, dtype=torch.int32, device=dev)
+    N.check(N.load().tt_mine_negatives(N.ptr(top_id.contiguous()), Q, k, N.ptr(excl_offsets.contiguous()),
+                                       N.ptr(excl_ids.contiguous()), int(skip), int(depth), N.ptr(table), N.ptr(count),
+                                       N.stream()), "tt_mine_negatives")
+    return table, count
+
+
 def ndcg_at_k(top_id, rel_offsets, rel_ids, kk=None):
     N.ensure_sm100()
     Q, k = top_id.shape

@@ -28,13 +28,15 @@ from torch import GradScaler, autocast
 
 try:
     from . import comm, ops, retrieval
-    from .data import DeviceTripletFeeder, MSMarcoDataset, PooledBank, TokenTripletLoader, TripletDataLoader
+    from .data import (DeviceTripletFeeder, HardNegativeMiner, MSMarcoDataset, PooledBank, TokenTripletLoader,
+                       TripletDataLoader)
     from .model import TokenBatch, TripletLoss, TwoTowersModel
 except ImportError:
     import comm
     import ops
     import retrieval
-    from data import DeviceTripletFeeder, MSMarcoDataset, PooledBank, TokenTripletLoader, TripletDataLoader
+    from data import (DeviceTripletFeeder, HardNegativeMiner, MSMarcoDataset, PooledBank, TokenTripletLoader,
+                      TripletDataLoader)
     from model import TokenBatch, TripletLoss, TwoTowersModel
 
 try:  # wandb is optional at import time; only touched when logging is requested
@@ -970,6 +972,37 @@ def evaluate_model(
 # --------------------------------------------------------------------------------------------------
 # run driver (training.py:383-529)
 # --------------------------------------------------------------------------------------------------
+def hard_negative_config(hard_negatives: Union[None, int, dict]) -> Optional[dict]:
+    """run_training(hard_negatives=...) -> None (off) or {"miner": HardNegativeMiner kwargs, "warmup_epochs": n}.
+    None reads TT_HARD_NEGATIVES (unset / 0 = off, an integer d = depth d)."""
+    if hard_negatives is None:
+        env = os.environ.get("TT_HARD_NEGATIVES", "0").strip() or "0"
+        try:
+            hard_negatives = int(env)
+        except ValueError:
+            raise ValueError(f"TT_HARD_NEGATIVES must be an integer depth (0 = off), got {env!r}") from None
+    if isinstance(hard_negatives, bool) or not isinstance(hard_negatives, (int, dict)):
+        raise ValueError(f"hard_negatives must be None, an integer depth or a dict, got {hard_negatives!r}")
+    if isinstance(hard_negatives, int):
+        if hard_negatives < 0:
+            raise ValueError(f"hard_negatives depth must be >= 0, got {hard_negatives}")
+        hard_negatives = {"depth": hard_negatives} if hard_negatives else None
+    if hard_negatives is None:
+        return None
+    kw = dict(hard_negatives)
+    warmup = int(kw.pop("warmup_epochs", 1))
+    if warmup < 0:
+        raise ValueError(f"warmup_epochs must be >= 0, got {warmup}")
+    allowed = {"depth", "skip", "ratio", "k_scan"}
+    if set(kw) - allowed:
+        raise ValueError(f"hard_negatives: unknown keys {sorted(set(kw) - allowed)} (allowed: {sorted(allowed)} and "
+                         "warmup_epochs)")
+    d = dict(depth=8, skip=0, ratio=0.5, k_scan=32)
+    d.update(kw)
+    HardNegativeMiner.check_config(**d)
+    return {"miner": kw, "warmup_epochs": warmup}
+
+
 def run_training(
     num_epochs: int = 3,
     batch_size: int = 1024,
@@ -987,6 +1020,7 @@ def run_training(
     fused: Optional[bool] = None,
     table_dtype: torch.dtype = torch.float32,
     backbone: Optional[str] = None,
+    hard_negatives: Union[None, int, dict] = None,
 ) -> TwoTowersModel:
     """Main training function (training.py:383-529).  `fused` (additive) selects the FusedTrainer; by
     default it is used whenever the dataset is token-bank backed and no gradient accumulation / wandb
@@ -995,7 +1029,13 @@ def run_training(
     `backbone` (additive): "table" (the token-table backbone) or "minilm" (the reference's frozen MiniLM encoder);
     None reads the TT_BACKBONE environment variable, default "table", so an unmodified main.py can choose.  On the
     fused path a MiniLM model encodes every text of the training split once into pooled banks (data.PooledBank) and
-    trains the projections on rows gathered from them; otherwise it runs the reference-shaped loop."""
+    trains the projections on rows gathered from them; otherwise it runs the reference-shaped loop.
+
+    `hard_negatives` (additive): mined negatives on the fused path with the device feeder (data.HardNegativeMiner).
+    None reads TT_HARD_NEGATIVES (unset or 0 = off, the default; an integer d = on with depth d); an int d is the same;
+    a dict holds the miner's arguments plus "warmup_epochs" (default 1).  After warmup_epochs epochs of in-batch
+    negatives the table is re-mined from the current towers at the start of every epoch."""
+    hn = hard_negative_config(hard_negatives)
     if backbone is None:
         backbone = os.environ.get("TT_BACKBONE", "table")
     if backbone not in ("table", "minilm"):
@@ -1073,6 +1113,11 @@ def run_training(
         fused = bank_backed and (world > 1 or (accumulation_steps == 1 and not use_wandb))
     if world > 1 and not fused:
         raise ValueError("data-parallel training needs the fused step (a token-bank dataset and fused != False)")
+    host_feeder = os.environ.get("TT_HOST_FEEDER") == "1" or len(train_ds) < 2 * batch_size
+    if hn is not None and (not fused or host_feeder):
+        raise ValueError("hard negatives need the fused step with the device feeder (DeviceTripletFeeder); the "
+                         "reference-shaped loops and TokenTripletLoader draw in-batch negatives only (unset "
+                         "TT_HOST_FEEDER, use at least two batches of pairs)")
     if world > 1 and accumulation_steps != 1:
         say(f"  note: accumulation_steps={accumulation_steps} is ignored under data parallelism; the global batch "
             f"of {batch_size} triplets is one optimiser step")
@@ -1086,12 +1131,11 @@ def run_training(
     say(f"  Fused B200 step: {fused}")
 
     scaler = GradScaler(device.type) if use_mixed_precision else None
-    trainer = token_dl = feeder = None
+    trainer = token_dl = feeder = miner = None
     if fused:
         seed_box = [random.randrange(2 ** 31)]
         if world > 1:  # the epoch permutation and the in-batch negatives are functions of this seed: share rank 0's
             dist.broadcast_object_list(seed_box, src=0)
-        host_feeder = os.environ.get("TT_HOST_FEEDER") == "1" or len(train_ds) < 2 * batch_size
         if backbone == "minilm":
             # the frozen encoder runs once per training text, not three times per triplet and step
             t0 = time.perf_counter()
@@ -1108,8 +1152,16 @@ def run_training(
             # pools every positive document once (TT_NEG_REUSE=0: gather the negatives' tokens like any document)
             reuse = (not host_feeder and world == 1 and os.environ.get("TT_NEG_REUSE", "1") != "0"
                      and not model.query_tower.pretrained_model.table.requires_grad)
+            if hn is not None:
+                reuse = False
+                say("  Hard negatives: neg-index reuse is off (a mined negative is not a positive of the batch)")
             trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, token_slots=2, world_size=world,
                                    rank=rank, in_batch_negatives=reuse)
+            if hn is not None:  # the frozen table's pooled rows, for mining only (the step still pools tokens)
+                banks = (PooledBank.build(model.query_tower, train_ds.query_bank, trainer.Lq, world_size=world,
+                                          rank=rank),
+                         PooledBank.build(model.document_tower, train_ds.doc_bank, trainer.Ld, world_size=world,
+                                          rank=rank))
         if host_feeder:
             # host-assembled batches (negatives drawn over the global batch, this rank's slice)
             token_dl = TokenTripletLoader(train_ds, batch_size, trainer.Lq, trainer.Ld, rank=rank, world_size=world,
@@ -1117,11 +1169,20 @@ def run_training(
         else:  # token bank resident in HBM, batches (and in-batch negatives) assembled by one kernel per step
             feeder = DeviceTripletFeeder(train_ds, batch_size, trainer.Lq, trainer.Ld, device, rank=rank,
                                          world_size=world, seed=seed_box[0], rows_only=trainer.pooled is not None)
+            if hn is not None:
+                miner = HardNegativeMiner(train_ds, *banks, world_size=world, rank=rank, **hn["miner"])
+                feeder.hard_negatives = miner
         trainer.prepare(2)
 
     say(f"Starting training for {num_epochs} epochs...")
     for epoch in range(num_epochs):
         say(f"\nEpoch {epoch + 1}/{num_epochs}")
+        if miner is not None and epoch >= hn["warmup_epochs"]:
+            st = miner.refresh(model)
+            say(f"Hard negatives refreshed in {st['total_s'] * 1e3:.1f} ms (project {st['project_s'] * 1e3:.1f}, "
+                f"normalize {st['normalize_s'] * 1e3:.1f}, scan {st['scan_s'] * 1e3:.1f}, merge "
+                f"{st['merge_s'] * 1e3:.1f}, filter {st['filter_s'] * 1e3:.1f}): mean {st['mean_count']:.2f} of "
+                f"{miner.depth} per query, {st['empty_queries']} queries without one")
         if trainer is not None and feeder is not None:
             avg_loss = trainer.train_epoch_device(feeder, log_every=10)
         elif trainer is not None:
