@@ -27,13 +27,6 @@ int check_cuda(cudaError_t e, const char* what, const char* file, int line) {
 
 static unsigned long long g_launches = 0;
 void note_launch() { __atomic_fetch_add(&g_launches, 1ull, __ATOMIC_RELAXED); }
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("TT_PDL");
-    return e ? atoi(e) != 0 : false;  // measured on B200: 0.261 ms/step with the attribute, 0.244 without -> off
-  }();
-  return on;
-}
 
 int sm_count() {
   static int cached = 0;
@@ -63,8 +56,6 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 }
 
 __global__ void adam_advance_kernel(double* state, double beta1, double beta2) {
-  pdl_wait();
-  pdl_launch();
   const double t = state[0];
   state[0] = t + 1.0;
   state[1] = (t == 0.0 ? 1.0 : state[1]) * beta1;
@@ -74,8 +65,6 @@ __global__ void adam_advance_kernel(double* state, double beta1, double beta2) {
 __global__ void adam_dev_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                 float* __restrict__ v, size_t n, float lr, float beta1, float beta2, float eps,
                                 const double* __restrict__ state, float grad_scale) {
-  pdl_wait();
-  pdl_launch();
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float step_size = (float)((double)lr / (1.0 - state[1]));
@@ -328,8 +317,8 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
     s.ws = w.mma_ws; s.ws_bytes = w.mma_ws_bytes;
     s.phases = a->phases;
     TT_REQUIRE(a->chain >= 0 && a->chain <= 2, "tt_triplet_step: bad chain selector %d", a->chain);
-    s.chain = a->chain;
-    if (a->adam_param && (a->chain == 1 || (a->chain == 0 && chain_enabled()))) {  // the optimiser rides in the chain kernel's tail
+    s.chain = a->chain == 1 || (a->chain == 0 && chain_enabled());
+    if (a->adam_param && s.chain) {  // the optimiser rides in the chain kernel's tail
       s.adam = FusedAdam{a->adam_state, a->adam_param, a->adam_grad, a->adam_exp_avg, a->adam_exp_avg_sq, a->adam_n,
                          a->adam_lr, a->adam_beta1, a->adam_beta2, a->adam_eps};
       adam_done = true;
@@ -378,12 +367,12 @@ extern "C" int tt_adam_step_dev(float* param, const float* grad, float* exp_avg,
                                 tt_stream_t stream) {
   TT_REQUIRE(state != nullptr, "tt_adam_step_dev: null state");
   cudaStream_t st = as_stream(stream);
-  TT_CUDA(launch_pdl(adam_advance_kernel, dim3(1), dim3(1), 0, st, state, (double)beta1, (double)beta2));
-  note_launch();
+  adam_advance_kernel<<<1, 1, 0, st>>>(state, beta1, beta2);
+  TT_LAUNCH_CHECK();
   if (n == 0) return 0;
-  TT_CUDA(launch_pdl(adam_dev_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, st, param, (const float*)grad,
-                     exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, (const double*)state, grad_scale));
-  note_launch();
+  adam_dev_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2,
+                                                                eps, state, grad_scale);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 

@@ -82,13 +82,12 @@ struct SplitJobC {  // fp32 [R, C] dense -> bf16 terms hi/lo[/lo2] [R, C]
 
 struct alignas(64) ChainParams {
   TowerMaps tm[2];
-  int B, H, P, RTB, NC, NCH, NCF, ldt, dcol;  // NCF: 64-column tiles of the fused layer-2 / loss phase
+  int B, H, P, RTB, NC, NCH, NCF;  // NCF: 64-column tiles of the fused layer-2 / loss phase
   int pairs, terms, pairs1, terms1;
   int kcb, nch[2], kbt[2];
   int off[T_COUNT + 1];
   int stages, n_sj, n_split_f4, n_split_f4_w1;
   int nS;        // tasks of the S, T and G phases: one per CTA
-  int krot;      // rotate the k-block order per CTA (tuning hook TT_CHAIN_KROT)
   int use_pdl;   // launched as a programmatic dependent of the pooled gather: wait for it before touching x
   SplitJobC sj[6];
   float margin, inv_batch, grad_scale;
@@ -954,10 +953,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         fence_proxy_async();  // other CTAs' generic-proxy writes (acquired above) before this thread's TMA reads
         for (int k = 0; k < ns; ++k) {
           const Sub sb = get_sub(p, tk, k);
-          // CTAs working on the same operand (every row tile reads the same weight tiles) start at different k-blocks,
-          // so that they do not all pull the same L2 lines at the same moment; the order is fixed per task
-          int kb = sb.kb0 + (p.krot ? (int)(blockIdx.x % (unsigned)sb.nkb) : 0);
-          for (int kbi = 0; kbi < sb.nkb; ++kbi, kb = (kb + 1 == sb.kb0 + sb.nkb) ? sb.kb0 : kb + 1) {
+          for (int kb = sb.kb0; kb < sb.kb0 + sb.nkb; ++kb) {
             for (int j = 0; j < sb.terms; ++j) {
               mbar_wait(&empty[s], ph ^ 1u);
               mbar_arrive_expect_tx(&full[s], kABytes + (uint32_t)sb.bn * BK * 2);
@@ -1078,15 +1074,9 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
   if (warp == 1) tmem_dealloc(tmem_base, kAcc * BN);
 }
 
-int chain_stages() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TT_CHAIN_STAGES");
-    v = e ? atoi(e) : 0;
-    if (v < 3 || v > kMaxStages) v = 5;  // (6 x 32 KB + 29 KB of epilogue staging still fit the 227 KB; 5 measured best)
-  }
-  return v;
-}
+// operand ring depth (6 x 32 KB + 29 KB of epilogue staging still fit the 227 KB; 5 measured best)
+constexpr int kChainStages = 5;
+static_assert(kChainStages <= kMaxStages, "the barrier block holds kMaxStages slots");
 
 int chain_debug_out() {  // TT_CHAIN_FP32_OUT=1: also write h, y, dY and dz1 in fp32 (diagnostics; read per call)
   const char* e = getenv("TT_CHAIN_FP32_OUT");
@@ -1120,7 +1110,7 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   carve_step(reinterpret_cast<char*>(s.ws), B, H, P, s.dxhat != nullptr, &w);
   static bool attr_done = false;
   if (!attr_done) {
-    TT_CUDA(cudaFuncSetAttribute(chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem(chain_stages())));
+    TT_CUDA(cudaFuncSetAttribute(chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem(kChainStages)));
     attr_done = true;
   }
   static thread_local ChainParams p;  // ~8 KB: kept off the stack; copied into the launch before this returns
@@ -1154,18 +1144,12 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   }
   p.B = B; p.H = H; p.P = P;
   p.RTB = (B + BM - 1) / BM; p.NC = (P + BN - 1) / BN; p.NCH = (H + BN - 1) / BN; p.NCF = P / 64;
-  p.ldt = w.ldt; p.dcol = w.dcol;  // (unused by the kernel now; kept in the parameter block for the trace tools)
   p.pairs = x3 ? 3 : 1; p.terms = x3 ? 2 : 1;
-  {
-    const char* e = getenv("TT_FWD1_PRODUCTS");  // tuning hook shared with the per-kernel chain
-    const int six = !(e && atoi(e) == 3);
-    p.pairs1 = x3 ? (six ? 6 : 3) : 1;
-    p.terms1 = x3 ? (six ? 3 : 2) : 1;
-  }
+  p.pairs1 = x3 ? 6 : 1; p.terms1 = x3 ? 3 : 1;  // layer 1 (its ReLU sign gates the backward): 6-product split
   for (int t = 0; t < 2; ++t) p.kbt[t] = (rows[t] + BK - 1) / BK;
   p.kcb = 8;
   {
-    const char* e = getenv("TT_CHAIN_KCB");  // tuning hook: k-blocks (64 batch rows each) per weight-gradient chunk
+    const char* e = getenv("TT_CHAIN_KCB");  // test hook: k-blocks (64 batch rows each) per weight-gradient chunk
     if (e && atoi(e) >= 4) p.kcb = atoi(e) / 4 * 4;
   }
   while ((p.kbt[0] + p.kcb - 1) / p.kcb + (p.kbt[1] + p.kcb - 1) / p.kcb > 48) p.kcb += 8;
@@ -1188,7 +1172,7 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   for (int k = 0; k < T_COUNT; ++k) p.off[k + 1] = p.off[k] + count[k];
   p.total_signals = (unsigned)(count[T_F2L] + count[T_DZ] + count[T_DW2] + count[T_DW1]);
   p.dw2_signals = (unsigned)count[T_DW2];
-  p.stages = chain_stages();
+  p.stages = kChainStages;
   // weights of both towers -> bf16 terms (+ transposes for the backward contractions); the first-layer weights come
   // first in the flat pass: layer 1 starts as soon as THEY are split (counter 0), the rest signals counter 2
   int f4 = 0;
@@ -1218,10 +1202,6 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   p.ctr = w.counters;
   p.n_counters = w.n_counters;
   p.nS = grid;
-  {
-    const char* e = getenv("TT_CHAIN_KROT");
-    p.krot = e ? atoi(e) : 0;  // off: no speed-up measured, and ascending k keeps the rounding correlated with the fp32 oracle
-  }
   if (s.adam.param) {
     const FusedAdam& a = s.adam;
     TT_REQUIRE(a.state && a.grad && a.exp_avg && a.exp_avg_sq, "tt_triplet_step: fused Adam needs state, grad and both moments");

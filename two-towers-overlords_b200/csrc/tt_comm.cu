@@ -94,8 +94,6 @@ __device__ __forceinline__ bool wait_flag(const unsigned* flag, unsigned epoch, 
 }
 
 __global__ void __launch_bounds__(kDpThreads) dp_rs_adam_ag_kernel(const __grid_constant__ DpParams p) {
-  pdl_wait();
-  pdl_launch();
   // Sticky error: once a peer has timed out (ctl[3] != 0) the protocol state (tickets, epoch, the peers' flags) is
   // no longer consistent, so every later launch is a no-op until the host has seen the error (DpExchange.check()
   // raises) — no update is ever applied on half-exchanged gradients.  The value is stable for the whole kernel only
@@ -342,8 +340,8 @@ extern "C" int tt_dp_reduce_adam(void* const* segments, int world, int rank, siz
   const int cap = max_ctas > 0 ? (max_ctas < sm_count() ? max_ctas : sm_count()) : sm_count();
   if (ctas > cap) ctas = cap;
   if (ctas < 1) ctas = 1;
-  TT_CUDA(launch_pdl(dp_rs_adam_ag_kernel, dim3((unsigned)ctas), dim3(kDpThreads), 0, as_stream(stream), p));
-  note_launch();
+  dp_rs_adam_ag_kernel<<<(unsigned)ctas, kDpThreads, 0, as_stream(stream)>>>(p);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 

@@ -37,28 +37,6 @@ void note_launch();
 
 static inline cudaStream_t as_stream(tt_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 
-// Programmatic dependent launch for the kernels of the training-step chain: the next kernel of the stream is
-// scheduled while the previous one drains, runs its prologue (barrier init, TMEM allocation, index math) and then
-// blocks in pdl_wait() until the previous grid has completed and its writes are visible.  EVERY kernel launched
-// through launch_pdl() calls pdl_wait() before its first global access (also when it does not read the previous
-// kernel's output: completion order must stay transitive along the chain) and pdl_launch() right after it.
-bool pdl_enabled();  // TT_PDL=1 turns the attribute on; default off (early-launched dependents slowed the step down)
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                     Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, args...);
-}
-
 template <typename T>
 static inline T* ws_take(char*& p, size_t n_elems) {
   uintptr_t a = (reinterpret_cast<uintptr_t>(p) + 255) & ~uintptr_t(255);
@@ -71,6 +49,10 @@ static inline size_t ws_round(size_t bytes) { return (bytes + 255) & ~size_t(255
 int sm_count();
 
 // ---- device helpers -------------------------------------------------------------------------
+// Programmatic dependent launch, used between the pooled gather and the persistent chain kernel of a whole-step call:
+// pdl_launch() lets the next kernel of the stream start filling SMs, which then blocks in pdl_wait() until this grid
+// has completed and its writes are visible.  pdl_wait() returns at once in a kernel launched without the attribute,
+// and pdl_launch() does nothing when the next kernel is launched without it.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ float warp_sum(float v) {

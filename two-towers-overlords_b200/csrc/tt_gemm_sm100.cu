@@ -11,8 +11,6 @@
 //     (tcgen05.ld 32 lanes x 16 columns per warp quarter), STAGES-deep mbarrier ring between producer and issuer;
 //   * up to two problem groups per launch (query tower | document tower) and split-K over blockIdx.z for the
 //     weight-gradient contractions (K = batch rows), reduced afterwards in a fixed order (deterministic).
-#include <stdlib.h>
-
 #include "tt_ptx.cuh"
 #include "tt_simt.cuh"
 #include "tt_sm100.cuh"
@@ -94,8 +92,6 @@ __global__ void __launch_bounds__(kGemmThreads, 2) gemm_tn_kernel(const __grid_c
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();    // everything above overlapped the tail of the previous kernel; operands are read from here on
-  pdl_launch();
 
   // Producer and issuer loops run on one lane chosen by elect.sync: in a `lane == 0` region every UTMALDG / UTCHMMA /
   // UTCBAR is wrapped in an ELECT + BRA.U.ANY loop (~80 clk each); under an elect.sync predicate they issue directly.
@@ -227,8 +223,6 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
                                                             size_t n0, const float* __restrict__ partial1,
                                                             float* __restrict__ out1, size_t n1, int splits,
                                                             int accumulate) {
-  pdl_wait();
-  pdl_launch();
   const float* partial = blockIdx.y ? partial1 : partial0;
   float* out = blockIdx.y ? out1 : out0;
   const size_t n = blockIdx.y ? n1 : n0;
@@ -257,8 +251,6 @@ struct SplitJobs {
 
 __global__ void __launch_bounds__(256) split_transpose_kernel(const SplitJobs jobs) {
   __shared__ bf16 s_hi[32][33], s_lo[32][33];
-  pdl_wait();
-  pdl_launch();
   const SplitJob& J = jobs.j[blockIdx.z];
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
   const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
@@ -298,8 +290,6 @@ __global__ void __launch_bounds__(256) transpose_pair_kernel(const bf16* __restr
                                                              bf16* __restrict__ tlo, int ldt, int tcol0, int split_row,
                                                              int shift) {
   __shared__ bf16 s[2][32][33];
-  pdl_wait();
-  pdl_launch();
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
 #pragma unroll
@@ -373,18 +363,8 @@ int ensure_gemm_attr() {
   return 0;
 }
 
-// ring depth: 3 slots (98 KB) keep two CTAs per SM, so one CTA's epilogue overlaps the other's main loop;
-// TT_GEMM_STAGES overrides (tuning hook)
-int gemm_stages(int n_pairs) {
-  static int env = -1;
-  if (env < 0) {
-    const char* e = getenv("TT_GEMM_STAGES");
-    env = e ? atoi(e) : 0;
-  }
-  if (env >= 3 && env <= kMaxStages) return env;
-  (void)n_pairs;
-  return 3;
-}
+// ring depth: 3 slots (98 KB) keep two CTAs per SM, so one CTA's epilogue overlaps the other's main loop
+constexpr int kGemmStages = 3;
 
 // Launches 1 or 2 problem groups.  partial != nullptr: every group is a split-K contraction whose raw partial sums
 // go to `partial` ([group][split][M*N], groups packed back to back) and are then reduced into d.C (+= if accumulate).
@@ -428,10 +408,10 @@ int launch_gemm(const GemmDesc* d, int ngroups, int n_pairs, int splits, float* 
       off += (size_t)splits * d[i].M * d[i].N;
     }
   }
-  p.stages = gemm_stages(n_pairs);
+  p.stages = kGemmStages;
   dim3 grid(tiles_n, tiles_m, ngroups * splits);
-  TT_CUDA(launch_pdl(gemm_tn_kernel, grid, dim3(kGemmThreads), gemm_smem(p.stages), st, p));
-  note_launch();
+  gemm_tn_kernel<<<grid, kGemmThreads, gemm_smem(p.stages), st>>>(p);
+  TT_LAUNCH_CHECK();
   if (use_partial) {
     size_t n[2] = {0, 0};
     for (int i = 0; i < ngroups; ++i) {
@@ -439,10 +419,10 @@ int launch_gemm(const GemmDesc* d, int ngroups, int n_pairs, int splits, float* 
       TT_REQUIRE(d[i].ldc == 0 || d[i].ldc == d[i].N, "gemm: split-K output must be dense");
     }
     const size_t nmax = n[0] > n[1] ? n[0] : n[1];
-    TT_CUDA(launch_pdl(splitk_reduce_kernel, dim3((unsigned)((nmax / 4 + 255) / 256), ngroups), dim3(256), 0, st,
-                       (const float*)p.g[0].partial, d[0].C, n[0], (const float*)(ngroups > 1 ? p.g[1].partial : nullptr),
-                       ngroups > 1 ? d[1].C : (float*)nullptr, n[1], splits, accumulate));
-    note_launch();
+    splitk_reduce_kernel<<<dim3((unsigned)((nmax / 4 + 255) / 256), ngroups), 256, 0, st>>>(
+        p.g[0].partial, d[0].C, n[0], ngroups > 1 ? p.g[1].partial : nullptr, ngroups > 1 ? d[1].C : nullptr, n[1],
+        splits, accumulate);
+    TT_LAUNCH_CHECK();
   } else {
     TT_REQUIRE(!accumulate, "gemm: accumulate needs the split-K path");  // checked before the launch in practice
   }
@@ -451,12 +431,6 @@ int launch_gemm(const GemmDesc* d, int ngroups, int n_pairs, int splits, float* 
 
 int choose_splits(int tiles, int K) {
   const int kb = (K + BK - 1) / BK;
-  static int env = -1;
-  if (env < 0) {
-    const char* e = getenv("TT_GEMM_SPLITS");  // tuning hook
-    env = e ? atoi(e) : 0;
-  }
-  if (env >= 2) return min(env, max(kb, 2));
   int s = (2 * sm_count() + tiles - 1) / tiles;
   s = min(s, kb);
   s = min(s, 32);
@@ -471,8 +445,8 @@ int split_jobs(const SplitJob* jobs, int n, cudaStream_t st) {
     rmax = max(rmax, jobs[i].R);
     cmax = max(cmax, jobs[i].C);
   }
-  TT_CUDA(launch_pdl(split_transpose_kernel, dim3((cmax + 31) / 32, (rmax + 31) / 32, n), dim3(256), 0, st, J));
-  note_launch();
+  split_transpose_kernel<<<dim3((cmax + 31) / 32, (rmax + 31) / 32, n), 256, 0, st>>>(J);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 
@@ -485,8 +459,8 @@ int split_transpose(const float* X, int R, int C, long long ld, bf16* hi, bf16* 
 int transpose_pair(const bf16* hi, const bf16* lo, int R, int C, bf16* thi, bf16* tlo, int ldt, int tcol0,
                    int split_row, int shift, cudaStream_t st) {
   dim3 grid((C + 31) / 32, (R + 31) / 32);
-  TT_CUDA(launch_pdl(transpose_pair_kernel, grid, dim3(256), 0, st, hi, lo, R, C, thi, tlo, ldt, tcol0, split_row, shift));
-  note_launch();
+  transpose_pair_kernel<<<grid, 256, 0, st>>>(hi, lo, R, C, thi, tlo, ldt, tcol0, split_row, shift);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 
@@ -628,23 +602,6 @@ static int get_forks(Forks** out) {
   *out = &f;
   return 0;
 }
-static int fwd1_products() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TT_FWD1_PRODUCTS");  // tuning hook: 3 = hi*hi + hi*lo + lo*hi only
-    v = (e && atoi(e) == 3) ? 3 : 6;
-  }
-  return v;
-}
-static bool pdl_chain_enabled() {
-  const char* e = getenv("TT_CHAIN_PDL");  // tuning hook: 0 = plain stream order between the gather and the chain kernel
-  return e ? atoi(e) != 0 : true;
-}
-static int step_concurrency() {
-  const char* e = getenv("TT_STEP_FORK");  // tuning hook: 0 = one serial chain
-  return e ? atoi(e) : 1;
-}
-
 int step_sm100(const StepSm100& s, cudaStream_t st) {
   const int B = s.B, H = s.H, P = s.P, np = s.n_split;
   TT_REQUIRE(s.ws && s.ws_bytes >= step_sm100_ws_bytes(B, H, P, s.dxhat != nullptr), "tt_triplet_step: tensor-core workspace too small");
@@ -663,17 +620,16 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
 
   // 1. pooled gather: fp32 xhat + its bf16 split (row-major); the transposed copy comes from a tiled transpose
   const bool front = s.phases == 0 || (s.phases & TT_STEP_FRONT), back = s.phases == 0 || (s.phases & TT_STEP_BACK);
-  const bool chain = s.chain == 1 || (s.chain == 0 && chain_enabled());
   if (front) {
     PoolParams pp = s.pool;
     pp.x_hi = w.x_hi; pp.x_lo = w.x_lo; pp.x_lo2 = (np == 3) ? w.x_lo2 : nullptr;
     pp.share_sm = (s.phases == TT_STEP_FRONT) ? 1 : 0;  // gather-only call = the pipelined trainer's look-ahead gather
     if ((rc = pool_fwd_launch(pp, s.table_dtype, H, st))) return rc;
     // (the persistent chain kernel transposes the xhat terms itself)
-    if (!chain && (rc = transpose_pair(w.x_hi, w.x_lo, 3 * B, H, w.xt_hi, w.xt_lo, w.ldt, 0, B, w.dcol - B, st))) return rc;
+    if (!s.chain && (rc = transpose_pair(w.x_hi, w.x_lo, 3 * B, H, w.xt_hi, w.xt_lo, w.ldt, 0, B, w.dcol - B, st))) return rc;
   }
   if (!back) return 0;
-  if (chain) return chain_sm100(s, /*after_gather=*/front && pdl_chain_enabled(), st);
+  if (s.chain) return chain_sm100(s, /*after_gather=*/front, st);
   // 2. weights of both towers -> bf16 terms (+ transposes for the backward contractions), one launch
   {
     SplitJob jobs[4];
@@ -696,7 +652,7 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
     g[t].Ct_hi = w.ht_hi + tcol[t]; g[t].Ct_lo = w.ht_lo + tcol[t]; g[t].ldt = w.ldt;
   }
   // (6-product split for this layer only: its ReLU sign gates the backward, see mlp_fwd_sm100)
-  if ((rc = launch_gemm(g, 2, np == 3 ? fwd1_products() : 1, 1, nullptr, 0, st))) return rc;
+  if ((rc = launch_gemm(g, 2, np == 3 ? 6 : 1, 1, nullptr, 0, st))) return rc;
   // 4. y = h W2^T + b2
   for (int t = 0; t < 2; ++t) {
     g[t] = GemmDesc{};
@@ -718,13 +674,10 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
   // From here the chain forks: {dY^T -> dW2}, {db2, db1} and {dz1 -> dW1} only share inputs.
   Forks* fk = nullptr;
   if ((rc = get_forks(&fk))) return rc;
-  const bool fork = step_concurrency() != 0;
-  cudaStream_t sA = fork ? fk->aux[0] : st, sB = fork ? fk->aux[1] : st;
-  if (fork) {
-    TT_CUDA(cudaEventRecord(fk->ev[0], st));
-    TT_CUDA(cudaStreamWaitEvent(sA, fk->ev[0], 0));
-    TT_CUDA(cudaStreamWaitEvent(sB, fk->ev[0], 0));
-  }
+  cudaStream_t sA = fk->aux[0], sB = fk->aux[1];
+  TT_CUDA(cudaEventRecord(fk->ev[0], st));
+  TT_CUDA(cudaStreamWaitEvent(sA, fk->ev[0], 0));
+  TT_CUDA(cudaStreamWaitEvent(sB, fk->ev[0], 0));
   // 6a. (branch A) dY^T, then dW2 = dY^T h   (split-K over the batch rows)
   if ((rc = transpose_pair(w.dy_hi, w.dy_lo, 3 * B, P, w.dyt_hi, w.dyt_lo, w.ldt, 0, B, w.dcol - B, sA))) return rc;
   for (int t = 0; t < 2; ++t) {
@@ -734,7 +687,7 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
     g[t].M = P; g[t].N = P; g[t].K = rows[t]; g[t].C = dW2[t];
   }
   const int tiles2 = 2 * ((P + BM - 1) / BM) * ((P + BN - 1) / BN);
-  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles2, B), fork ? w.partial2 : w.partial, 0, sA))) return rc;
+  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles2, B), w.partial2, 0, sA))) return rc;
   // 6b. (branch B) db2
   if ((rc = colsum2(s.dy, rows[0], db2[0], s.dy + (size_t)row0[1] * P, rows[1], db2[1], P, P, 0, w.colsum2, sB))) return rc;
   // 7. (main) dz1 = (dY W2) * (h > 0)
@@ -750,10 +703,9 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
     g[t].Ct_hi = w.dzt_hi + tcol[t]; g[t].Ct_lo = w.dzt_lo + tcol[t]; g[t].ldt = w.ldt;
   }
   if ((rc = launch_gemm(g, 2, np, 1, nullptr, 0, st))) return rc;
-  if (fork) {  // branch B continues with db1 once dz1 exists
-    TT_CUDA(cudaEventRecord(fk->ev[1], st));
-    TT_CUDA(cudaStreamWaitEvent(sB, fk->ev[1], 0));
-  }
+  // branch B continues with db1 once dz1 exists
+  TT_CUDA(cudaEventRecord(fk->ev[1], st));
+  TT_CUDA(cudaStreamWaitEvent(sB, fk->ev[1], 0));
   if ((rc = colsum2(w.dz1, rows[0], db1[0], w.dz1 + (size_t)row0[1] * P, rows[1], db1[1], P, P, 0, w.colsum, sB)))
     return rc;
   // 8. (main) dW1 = dz1^T x
@@ -765,12 +717,11 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
   }
   const int tiles1 = 2 * ((P + BM - 1) / BM) * ((H + BN - 1) / BN);
   if ((rc = launch_gemm(g, 2, np, choose_splits(tiles1, B), w.partial, 0, st))) return rc;
-  if (fork) {  // join
-    TT_CUDA(cudaEventRecord(fk->ev[2], sA));
-    TT_CUDA(cudaEventRecord(fk->ev[3], sB));
-    TT_CUDA(cudaStreamWaitEvent(st, fk->ev[2], 0));
-    TT_CUDA(cudaStreamWaitEvent(st, fk->ev[3], 0));
-  }
+  // join
+  TT_CUDA(cudaEventRecord(fk->ev[2], sA));
+  TT_CUDA(cudaEventRecord(fk->ev[3], sB));
+  TT_CUDA(cudaStreamWaitEvent(st, fk->ev[2], 0));
+  TT_CUDA(cudaStreamWaitEvent(st, fk->ev[3], 0));
   // 9. dxhat = dz1 W1 (only when the token tables train)
   if (s.dxhat) {
     for (int t = 0; t < 2; ++t) {

@@ -106,8 +106,6 @@ __global__ void __launch_bounds__(128)
                          float* __restrict__ dn, LossSplitOut sp, float* __restrict__ scratch) {
   __shared__ float s_h[4];
   __shared__ int s_last;
-  pdl_wait();
-  pdl_launch();
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int i = blockIdx.x * 4 + w;
   float hinge = 0.f;
@@ -190,9 +188,9 @@ int triplet_loss_fused(const float* q, const float* p, const float* n, int B, in
   TT_REQUIRE(B >= 1, "triplet loss: empty batch");
   LossSplitOut sp{};
   if (split) sp = *split;
-  TT_CUDA(launch_pdl(triplet_fused_kernel, dim3((B + 3) / 4), dim3(128), 0, st, q, p, n, B, P, margin, inv_batch,
-                     grad_scale, stats, loss, dq, dp, dn, sp, scratch));
-  note_launch();
+  triplet_fused_kernel<<<(B + 3) / 4, 128, 0, st>>>(q, p, n, B, P, margin, inv_batch, grad_scale, stats, loss, dq, dp,
+                                                    dn, sp, scratch);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 

@@ -94,8 +94,6 @@ __global__ void __launch_bounds__(256) colsum_partial_kernel(const float* __rest
                                                              const float* __restrict__ X1, int M1, int N, long long ld,
                                                              int S, float* __restrict__ scratch) {
   __shared__ double s[8][33];
-  pdl_wait();
-  pdl_launch();
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int job = blockIdx.z, slice = blockIdx.y;
   const float* X = job ? X1 : X0;
@@ -119,8 +117,6 @@ __global__ void __launch_bounds__(256) colsum_partial_kernel(const float* __rest
 __global__ void __launch_bounds__(256) colsum_final_kernel(const float* __restrict__ scratch, int S, int N,
                                                            float* __restrict__ out0, float* __restrict__ out1,
                                                            int accumulate) {
-  pdl_wait();
-  pdl_launch();
   const int n = blockIdx.x * 256 + threadIdx.x;
   const int job = blockIdx.y;
   if (n >= N) return;
@@ -137,11 +133,11 @@ int colsum2(const float* X0, int M0, float* out0, const float* X1, int M1, float
   if (N <= 0) return 0;
   const int njobs = X1 ? 2 : 1;
   dim3 grid((N + 31) / 32, kColsumSlices, njobs);
-  TT_CUDA(launch_pdl(colsum_partial_kernel, grid, dim3(256), 0, st, X0, M0, X1, M1, N, ld, (int)kColsumSlices, scratch));
-  note_launch();
-  TT_CUDA(launch_pdl(colsum_final_kernel, dim3((N + 255) / 256, njobs), dim3(256), 0, st, (const float*)scratch,
-                     (int)kColsumSlices, N, out0, out1, accumulate));
-  note_launch();
+  colsum_partial_kernel<<<grid, 256, 0, st>>>(X0, M0, X1, M1, N, ld, (int)kColsumSlices, scratch);
+  TT_LAUNCH_CHECK();
+  colsum_final_kernel<<<dim3((N + 255) / 256, njobs), 256, 0, st>>>(scratch, (int)kColsumSlices, N, out0, out1,
+                                                                     accumulate);
+  TT_LAUNCH_CHECK();
   return 0;
 }
 

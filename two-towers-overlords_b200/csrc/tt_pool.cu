@@ -5,8 +5,6 @@
 // A warp reads one row per step as fully coalesced 16 B (fp32) / 8 B (bf16) per-lane vectors,
 // UNROLL rows in flight per warp, 4 warps per sequence, fp32 accumulation in registers, cross-warp
 // reduction staged in shared memory, warp-shuffle reduction for the norm.
-#include <stdlib.h>
-
 #include "tt_pool.cuh"
 
 namespace tt {
@@ -88,7 +86,7 @@ __global__ void __launch_bounds__(kRowThreads) pooled_rows_kernel(const PoolPara
   for (int v = lane; v < H / 4; v += 32) store_pooled4(p, H, (size_t)r, v * 4, __ldg(in + v));
 }
 
-template <typename TE, int NV, int UNROLL, bool PIPE>
+template <typename TE, int NV, int UNROLL>
 __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams p) {
   constexpr int H = NV * 128;
   __shared__ unsigned s_row[kMaxL];
@@ -161,55 +159,28 @@ __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams
   for (int i = 0; i < NV * 4; ++i) acc[i] = 0.f;
 
   using RV = RowVec<TE>;
-  // Software-pipelined in registers: the UNROLL*NV row loads of batch i+1 are issued before the FMAs of
-  // batch i, so a warp always has one whole batch in flight and the FMAs only ever wait on loads issued a
-  // full iteration earlier.  A padding entry re-reads row s_row[0] with weight 0 instead of predicating
-  // the load, which keeps each batch one unconditional run of loads.
-  typename RV::V v[UNROLL][NV];
-  float wt[UNROLL];
-  auto issue = [&](int e0, typename RV::V (&dst)[UNROLL][NV], float (&w)[UNROLL]) {
+  // One batch of UNROLL rows in flight per warp; latency is hidden by the other resident warps.  A padding entry
+  // re-reads row s_row[0] with weight 0 instead of predicating the load, which keeps each batch one unconditional run
+  // of loads.
+  for (int e0 = warp; e0 < n_valid; e0 += kPoolWarps * UNROLL) {
+    typename RV::V v[UNROLL][NV];
+    float wt[UNROLL];
     const TE* rows[UNROLL];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const int e = e0 + u * kPoolWarps;
       const bool ok = e < n_valid;
-      w[u] = ok ? s_w[e] : 0.f;
+      wt[u] = ok ? s_w[e] : 0.f;
       rows[u] = table + (size_t)s_row[ok ? e : 0] * H;
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u)
 #pragma unroll
-      for (int j = 0; j < NV; ++j) dst[u][j] = RV::load(rows[u], j * 32 + lane);
-  };
-  if (PIPE) {
-    if (warp < n_valid) issue(warp, v, wt);
-    for (int e0 = warp; e0 < n_valid; e0 += kPoolWarps * UNROLL) {
-      typename RV::V vn[UNROLL][NV];
-      float wn[UNROLL];
-      const int e1 = e0 + kPoolWarps * UNROLL;
-      const bool more = e1 < n_valid;
-      if (more) issue(e1, vn, wn);
+      for (int j = 0; j < NV; ++j) v[u][j] = RV::load(rows[u], j * 32 + lane);
 #pragma unroll
-      for (int u = 0; u < UNROLL; ++u)
+    for (int u = 0; u < UNROLL; ++u)
 #pragma unroll
-        for (int j = 0; j < NV; ++j) RV::fma(wt[u], v[u][j], acc + j * 4);
-      if (more) {
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-          wt[u] = wn[u];
-#pragma unroll
-          for (int j = 0; j < NV; ++j) v[u][j] = vn[u][j];
-        }
-      }
-    }
-  } else {  // one batch of UNROLL rows in flight per warp; latency is hidden by the other resident warps
-    for (int e0 = warp; e0 < n_valid; e0 += kPoolWarps * UNROLL) {
-      issue(e0, v, wt);
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-        for (int j = 0; j < NV; ++j) RV::fma(wt[u], v[u][j], acc + j * 4);
-    }
+      for (int j = 0; j < NV; ++j) RV::fma(wt[u], v[u][j], acc + j * 4);
   }
 
   // ---- 3. cross-warp reduction staged in shared memory --------------------------------------
@@ -304,46 +275,16 @@ __global__ void __launch_bounds__(kPoolThreads) pool_fwd_kernel(const PoolParams
   }
 }
 
-// Rows in flight per warp.  TT_POOL_VARIANT (tuning hook): 0 = register-pipelined x4, 1 = x4 (36 warps per SM),
-// 2 = x8, 3 = pipelined x2.  Default: x8 for fp32 tables when the gather has the SMs to itself (whole-step calls:
-// 100.5 vs 103 us per launch, 0.2373 vs 0.2407 ms per configs[1] step), x4 when it shares them with other kernels
-// (more, lighter warps interleave better) and for bf16 tables.
-int pool_variant(bool share_sm, bool fp32_table) {
-  static int env = -2;
-  if (env == -2) {
-    const char* e = getenv("TT_POOL_VARIANT");
-    env = e ? atoi(e) : -1;
-  }
-  if (env >= 0) return env;
-  return (!share_sm && fp32_table) ? 2 : 1;
-}
-
-// Unused dynamic shared memory that caps how many gather CTAs an SM holds.  When the gather of step i+1 runs beside the
-// tensor-core chain of step i (p.share_sm), an SM full of gather CTAs (36 warps, ~62 K registers) leaves no room for
-// a GEMM CTA until a whole wave of gathers has retired: the chain — the critical path — then stalls ~60 us per step
-// (torch.profiler timeline).  Fewer resident gather CTAs cost the gather some latency hiding, which does not matter
-// because it runs in the chain's shadow.
-size_t pool_pad_smem(bool share_sm) {
-  static int pad = -1;
-  if (pad < 0) {
-    const char* e = getenv("TT_POOL_PAD_SMEM");  // tuning hook (bytes, <= 40960)
-    pad = e ? atoi(e) : kPoolSharePadBytes;
-    if (pad < 0) pad = 0;
-    if (pad > 40960) pad = 40960;
-  }
-  return share_sm ? (size_t)pad : 0;
-}
-
+// Rows in flight per warp: 8 for bf16 tables.  For fp32 tables 8 when the gather has the SMs to itself (whole-step
+// calls: 100.5 vs 103 us per launch, 0.2373 vs 0.2407 ms per configs[1] step), 4 when it shares them with other kernels
+// (p.share_sm: more, lighter warps interleave better).
 template <typename TE, int NV>
 int launch_pool(const PoolParams& p, int total, cudaStream_t st) {
-  constexpr int UNROLL = sizeof(TE) == 4 ? 4 : 8;
-  const size_t pad = pool_pad_smem(p.share_sm != 0);
-  switch (pool_variant(p.share_sm != 0, sizeof(TE) == 4)) {
-    case 1: pool_fwd_kernel<TE, NV, UNROLL, false><<<total, kPoolThreads, pad, st>>>(p); break;
-    case 2: pool_fwd_kernel<TE, NV, UNROLL * 2, false><<<total, kPoolThreads, pad, st>>>(p); break;
-    case 3: pool_fwd_kernel<TE, NV, UNROLL / 2, true><<<total, kPoolThreads, pad, st>>>(p); break;
-    default: pool_fwd_kernel<TE, NV, UNROLL, true><<<total, kPoolThreads, pad, st>>>(p); break;
-  }
+  constexpr int kSharedUnroll = sizeof(TE) == 4 ? 4 : 8;
+  if (p.share_sm)
+    pool_fwd_kernel<TE, NV, kSharedUnroll><<<total, kPoolThreads, 0, st>>>(p);
+  else
+    pool_fwd_kernel<TE, NV, 8><<<total, kPoolThreads, 0, st>>>(p);
   TT_LAUNCH_CHECK();
   return 0;
 }

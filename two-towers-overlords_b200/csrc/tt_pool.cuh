@@ -23,7 +23,7 @@ struct PoolParams {
   __nv_bfloat16* x_hi;   // [rows, H]
   __nv_bfloat16* x_lo;
   __nv_bfloat16* x_lo2;  // nullable third term: xhat - hi - lo
-  int share_sm;  // 1: this launch runs beside other kernels (pipelined step): cap the resident CTAs per SM
+  int share_sm;  // 1: this launch runs beside other kernels (pipelined step): fewer rows in flight per warp
   // optional row aliases: output row alias_dst_row0 + i is a copy of output row alias_src_row0 + alias[i], i < alias_n
   // (in-batch negatives: negative i is the positive document of item alias[i]); nullptr = none
   const int* alias;
@@ -37,8 +37,6 @@ struct PoolParams {
   const int* row_index;  // [3 * row_B]
   int row_B;
 };
-
-constexpr int kPoolSharePadBytes = 0;  // default cap (bytes of unused dynamic smem per CTA); tuned on B200, see tt_pool.cu
 
 int pool_fwd_launch(PoolParams p, int table_dtype, int H, cudaStream_t st);
 

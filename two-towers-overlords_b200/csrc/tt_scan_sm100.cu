@@ -39,6 +39,7 @@ constexpr size_t kSmemLimit = 227 * 1024;
 // |bf16(q).bf16(d) - q.d| <= |q - q~||d| + |q~||d - d~| <= 2^-9 + 2^-9 (1 + 2^-9) for rows of norm <= 1, plus the
 // tensor-core accumulation error (< 1e-6): a rigorous, deliberately loose bound
 constexpr float kScanEps = 4e-3f;
+constexpr int kScanStagger = 4;  // document tiles between the starting points of neighbouring CTAs
 
 struct alignas(64) ScanParams {
   CUtensorMap d_map;
@@ -613,7 +614,6 @@ __global__ void __launch_bounds__(1024) compact_flags_kernel(const int* __restri
 }
 
 int scan_pair_enabled(int Q, long long N);
-int scan_stagger();
 float scan_eps();
 
 struct ScanPlan {
@@ -681,11 +681,6 @@ int scan_pair_enabled(int Q, long long N) {
   return (N >= 3000000 && Q >= 4096) ? 1 : 0;
 }
 
-int scan_stagger() {
-  const char* e = getenv("TT_SCAN_STAGGER");  // tuning hook: tiles between the starting points of neighbouring CTAs
-  return e ? atoi(e) : 4;
-}
-
 float scan_eps() {
   const char* e = getenv("TT_SCAN_EPS");  // test hook: a huge value forces every query through the exact re-scan
   return e ? (float)atof(e) : kScanEps;
@@ -748,7 +743,7 @@ int scan_topk_sm100(const float* Qn, const float* Dn, const void* Qb, const void
   int rc;
   if ((rc = make_map_bf16_kmajor(&sp.d_map, Db, (uint64_t)N, P, P, pl.pair ? TD / 2 : TD))) return rc;
   sp.Qb = reinterpret_cast<const bf16*>(Qb);
-  sp.stagger = scan_stagger();
+  sp.stagger = kScanStagger;
   sp.Q = Q; sp.P = P; sp.KB = pl.KB; sp.KC = pl.KC; sp.stages = pl.stages;
   sp.N = N; sp.docs_per_split = pl.docs_per_split;
   sp.cand_s = w.cand_s; sp.cand_i = w.cand_i; sp.bound = w.bound;

@@ -34,12 +34,12 @@ struct StepSm100 {
   size_t ws_bytes;
   int phases;                 // 0 / TT_STEP_FRONT | TT_STEP_BACK
   FusedAdam adam;
-  int chain;                  // 1 = persistent chain kernel, 2 = per-kernel chain, 0 = default (chain_enabled())
+  bool chain;                 // persistent chain kernel (else one kernel per contraction)
 };
 size_t step_sm100_ws_bytes(int B, int H, int P, int train_table);
 int step_sm100(const StepSm100& s, cudaStream_t st);
 // persistent chain kernel (tt_chain_sm100.cu): everything of the step after the pooled gather in ONE launch
-bool chain_enabled();  // TT_CHAIN=0 selects the per-kernel chain
+bool chain_enabled();  // TT_CHAIN=0 selects the per-kernel chain for tt_step_args.chain == 0
 int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st);
 
 // generic tensor-core contraction on bf16 (hi, lo) terms: C = act(A B^T + bias); act: 0 none, 1 ReLU, 2 GELU (erf)

@@ -429,8 +429,7 @@ class FusedTrainer:
 
     def _whole_step(self) -> bool:
         """Single GPU with the persistent chain kernel: a step is gather -> chain in one stream, no look-ahead."""
-        return (self.xchg is None and self.world == 1 and self.step_objs[0].chain_active()
-                and os.environ.get("TT_STEP_ORDER", "whole") == "whole")
+        return self.xchg is None and self.world == 1 and self.step_objs[0].chain_active()
 
     def wait(self):
         """Kept for API symmetry: every step() leaves parameters and `loss_view` final in stream order."""
