@@ -134,7 +134,7 @@ int tt_triplet_loss_bwd(const float* q, const float* p, const float* n, const fl
 /* ------------------------------------------------------------------------------------------
  * One whole triplet training step, forward + backward (training.py:37-50 without the optimiser):
  * pool(q), pool(p), pool(n) -> both tower MLPs -> loss -> gradients of the 8 projection tensors
- * (and of the tables when dtable_q/dtable_d are non-NULL).  Gradients are OVERWRITTEN.
+ * (and of the tables when dtable_q/dtable_d are non-NULL).  Gradients are OVERWRITTEN (see grad_accumulate).
  * ---------------------------------------------------------------------------------------- */
 typedef struct tt_step_args {
   /* tokens */
@@ -199,6 +199,15 @@ typedef struct tt_step_args {
   const float* pooled_q; int64_t pooled_q_rows;
   const float* pooled_d; int64_t pooled_d_rows;
   const int32_t* pooled_index;
+  /* gradient accumulation (the reference's `loss / accumulation_steps; backward()` over the micro-batches of a
+   * window, backend/training.py:66-133): 0 = the gradient outputs are OVERWRITTEN as described above; 1 = every
+   * gradient output (the 8 projection gradients, and dtable_q / dtable_d when given) becomes fl(old + new) in fp32,
+   * where new is exactly what the same call writes with 0 — autograd's `.grad += new`.  The loss is still overwritten
+   * with this call's loss.  With adam_param set the optimiser consumes the accumulated gradient, so a window of a
+   * micro-batches is a - 1 calls with grad_accumulate = 1 and no optimiser, then one with both (the first call of a
+   * window that carries nothing uses 0; set grad_scale = 1/a for the reference's scaling).  Appended, like the
+   * pooled_* fields, while TT_B200_VERSION stayed at 100: rebuild callers against this header.                    */
+  int grad_accumulate;
 } tt_step_args;
 #define TT_STEP_FRONT 1
 #define TT_STEP_BACK 2

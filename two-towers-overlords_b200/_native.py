@@ -74,6 +74,7 @@ class StepArgs(ctypes.Structure):
         ("pooled_q", c_void_p), ("pooled_q_rows", c_int64),
         ("pooled_d", c_void_p), ("pooled_d_rows", c_int64),
         ("pooled_index", c_void_p),
+        ("grad_accumulate", c_int),
     ]
 
 

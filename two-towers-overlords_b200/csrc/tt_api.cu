@@ -235,6 +235,9 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
   TT_REQUIRE(B >= 1, "tt_triplet_step: empty batch");
   const int train_table = (a->dtable_q != nullptr || a->dtable_d != nullptr) ? 1 : 0;
   TT_REQUIRE(!train_table || (a->dtable_q && a->dtable_d), "tt_triplet_step: give both table gradients or neither");
+  TT_REQUIRE(a->grad_accumulate == 0 || a->grad_accumulate == 1, "tt_triplet_step: grad_accumulate must be 0 or 1, got %d",
+             a->grad_accumulate);
+  const int acc = a->grad_accumulate;
   const size_t need = tt_step_ws_bytes(B, a->Lq, a->Ld, H, P, a->vocab, a->precision, train_table);
   TT_REQUIRE(a->ws && a->ws_bytes >= need, "tt_triplet_step: workspace too small (%zu < %zu)", a->ws_bytes, need);
   cudaStream_t st = as_stream(stream);
@@ -293,11 +296,11 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
                                w.dy + (size_t)B * P, w.dy + (size_t)2 * B * P, nullptr, st)))
       return rc;
     // 5. tower backward (document tower: positives and negatives in one M = 2B pass)
-    if ((rc = mlp_bwd_fp32(w.dy, w.xhat, w.h, a->Wq1, a->Wq2, B, H, P, a->dWq1, a->dbq1, a->dWq2, a->dbq2, dxhat, 0,
+    if ((rc = mlp_bwd_fp32(w.dy, w.xhat, w.h, a->Wq1, a->Wq2, B, H, P, a->dWq1, a->dbq1, a->dWq2, a->dbq2, dxhat, acc,
                            w.dz1, st)))
       return rc;
     if ((rc = mlp_bwd_fp32(w.dy + (size_t)B * P, w.xhat + (size_t)B * H, w.h + (size_t)B * P, a->Wd1, a->Wd2, 2 * B, H,
-                           P, a->dWd1, a->dbd1, a->dWd2, a->dbd2, dxhat ? dxhat + (size_t)B * H : nullptr, 0,
+                           P, a->dWd1, a->dbd1, a->dWd2, a->dbd2, dxhat ? dxhat + (size_t)B * H : nullptr, acc,
                            w.dz1 + (size_t)B * P, st)))
       return rc;
   } else {
@@ -314,6 +317,7 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
     s.h = w.h; s.y = w.y; s.stats = w.stats; s.dy = w.dy;
     s.dxhat = dxhat;
     s.n_split = (a->precision == TT_PREC_BF16X3) ? 3 : 1;
+    s.grad_accumulate = acc;
     s.ws = w.mma_ws; s.ws_bytes = w.mma_ws_bytes;
     s.phases = a->phases;
     TT_REQUIRE(a->chain >= 0 && a->chain <= 2, "tt_triplet_step: bad chain selector %d", a->chain);
@@ -337,11 +341,11 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
   if (train_table) {
     if ((rc = pool_bwd_prep(w.dxhat, w.xhat, w.cnt, w.nrm, 3 * B, H, w.g, st))) return rc;
     PoolBwdSeg sq{a->q_ids, a->q_mask, B, a->Lq, 0};
-    if ((rc = pool_bwd_scatter(&sq, 1, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_q, 0, w.pool_ws,
+    if ((rc = pool_bwd_scatter(&sq, 1, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_q, acc, w.pool_ws,
                                w.pool_ws_bytes, st)))
       return rc;
     PoolBwdSeg sd[2] = {{a->p_ids, a->p_mask, B, a->Ld, B}, {a->n_ids, a->n_mask, B, a->Ld, 2 * B}};
-    if ((rc = pool_bwd_scatter(sd, 2, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_d, 0, w.pool_ws,
+    if ((rc = pool_bwd_scatter(sd, 2, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_d, acc, w.pool_ws,
                                w.pool_ws_bytes, st)))
       return rc;
   }

@@ -103,6 +103,7 @@ struct alignas(64) ChainParams {
   double* adam_state;  // {t, beta1^t, beta2^t, -}: advanced once per launch (by the first task), read by the tail
   float *adam_p, *adam_g, *adam_m, *adam_v;
   float lr, beta1, beta2, eps;
+  int grad_accumulate;  // 1: a gradient element becomes fl(old + its fixed-order sum), and Adam consumes that
   unsigned total_signals, dw2_signals;
   unsigned long long* trace;  // nullable (TT_CHAIN_TRACE=1)
 };
@@ -772,9 +773,11 @@ __device__ __forceinline__ float adam1(const ChainParams& p, const AdamCoef& k, 
   const float denom = sqrtf(v) / k.bc2_sqrt + p.eps;
   return w - k.step_size * (m / denom);
 }
-// gradient element(s) at dst (a slice of the flat gradient buffer) -> memory, and the Adam update of the parameter,
+// gradient element(s) at dst (a slice of the flat gradient buffer; added to what dst holds when accumulating) -> memory,
+// and the Adam update of the parameter,
 // exp_avg and exp_avg_sq elements at the same offset of their flat buffers
 __device__ __forceinline__ void emit4(const ChainParams& p, const AdamCoef& k, float4* dst, float4 g) {
+  if (p.grad_accumulate) g = add4(*dst, g);
   *dst = g;
   if (!p.adam_p) return;
   const size_t off = reinterpret_cast<float*>(dst) - p.adam_g;
@@ -789,6 +792,7 @@ __device__ __forceinline__ void emit4(const ChainParams& p, const AdamCoef& k, f
   *reinterpret_cast<float4*>(p.adam_p + off) = w;
 }
 __device__ __forceinline__ void emit1(const ChainParams& p, const AdamCoef& k, float* dst, float g) {
+  if (p.grad_accumulate) g = *dst + g;
   *dst = g;
   if (!p.adam_p) return;
   const size_t off = dst - p.adam_g;
@@ -1202,6 +1206,7 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   p.ctr = w.counters;
   p.n_counters = w.n_counters;
   p.nS = grid;
+  p.grad_accumulate = s.grad_accumulate;
   if (s.adam.param) {
     const FusedAdam& a = s.adam;
     TT_REQUIRE(a.state && a.grad && a.exp_avg && a.exp_avg_sq, "tt_triplet_step: fused Adam needs state, grad and both moments");

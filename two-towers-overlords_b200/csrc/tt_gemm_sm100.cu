@@ -219,6 +219,7 @@ __global__ void __launch_bounds__(kGemmThreads, 2) gemm_tn_kernel(const __grid_c
 }
 
 // out[i] = (accumulate ? out[i] : 0) + sum_z partial[z][i], z ascending: fixed order, no atomics.  blockIdx.y = group.
+// accumulate == kAccumAfterSum: out[i] = fl(out[i] + sum_z partial[z][i]), the sum taken in the same order as for 0.
 __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restrict__ partial0, float* __restrict__ out0,
                                                             size_t n0, const float* __restrict__ partial1,
                                                             float* __restrict__ out1, size_t n1, int splits,
@@ -228,10 +229,15 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
   const size_t n = blockIdx.y ? n1 : n0;
   const size_t i = ((size_t)blockIdx.x * 256 + threadIdx.x) * 4;
   if (i >= n) return;
-  float4 acc = accumulate ? *reinterpret_cast<const float4*>(out + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+  const bool old_first = accumulate && accumulate != kAccumAfterSum;
+  float4 acc = old_first ? *reinterpret_cast<const float4*>(out + i) : make_float4(0.f, 0.f, 0.f, 0.f);
   for (int z = 0; z < splits; ++z) {
     const float4 t = *reinterpret_cast<const float4*>(partial + (size_t)z * n + i);
     acc.x += t.x; acc.y += t.y; acc.z += t.z; acc.w += t.w;
+  }
+  if (accumulate == kAccumAfterSum) {
+    const float4 old = *reinterpret_cast<const float4*>(out + i);
+    acc.x = old.x + acc.x; acc.y = old.y + acc.y; acc.z = old.z + acc.z; acc.w = old.w + acc.w;
   }
   *reinterpret_cast<float4*>(out + i) = acc;
 }
@@ -687,9 +693,11 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
     g[t].M = P; g[t].N = P; g[t].K = rows[t]; g[t].C = dW2[t];
   }
   const int tiles2 = 2 * ((P + BM - 1) / BM) * ((P + BN - 1) / BN);
-  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles2, B), w.partial2, 0, sA))) return rc;
+  // (s.grad_accumulate: every gradient output is fl(old + the sum a call without it writes))
+  const int acc = s.grad_accumulate ? kAccumAfterSum : 0;
+  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles2, B), w.partial2, acc, sA))) return rc;
   // 6b. (branch B) db2
-  if ((rc = colsum2(s.dy, rows[0], db2[0], s.dy + (size_t)row0[1] * P, rows[1], db2[1], P, P, 0, w.colsum2, sB))) return rc;
+  if ((rc = colsum2(s.dy, rows[0], db2[0], s.dy + (size_t)row0[1] * P, rows[1], db2[1], P, P, acc, w.colsum2, sB))) return rc;
   // 7. (main) dz1 = (dY W2) * (h > 0)
   for (int t = 0; t < 2; ++t) {
     g[t] = GemmDesc{};
@@ -706,7 +714,7 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
   // branch B continues with db1 once dz1 exists
   TT_CUDA(cudaEventRecord(fk->ev[1], st));
   TT_CUDA(cudaStreamWaitEvent(sB, fk->ev[1], 0));
-  if ((rc = colsum2(w.dz1, rows[0], db1[0], w.dz1 + (size_t)row0[1] * P, rows[1], db1[1], P, P, 0, w.colsum, sB)))
+  if ((rc = colsum2(w.dz1, rows[0], db1[0], w.dz1 + (size_t)row0[1] * P, rows[1], db1[1], P, P, acc, w.colsum, sB)))
     return rc;
   // 8. (main) dW1 = dz1^T x
   for (int t = 0; t < 2; ++t) {
@@ -716,7 +724,7 @@ int step_sm100(const StepSm100& s, cudaStream_t st) {
     g[t].M = P; g[t].N = H; g[t].K = rows[t]; g[t].C = dW1[t];
   }
   const int tiles1 = 2 * ((P + BM - 1) / BM) * ((H + BN - 1) / BN);
-  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles1, B), w.partial, 0, st))) return rc;
+  if ((rc = launch_gemm(g, 2, np, choose_splits(tiles1, B), w.partial, acc, st))) return rc;
   // join
   TT_CUDA(cudaEventRecord(fk->ev[2], sA));
   TT_CUDA(cudaEventRecord(fk->ev[3], sB));

@@ -123,7 +123,8 @@ __global__ void __launch_bounds__(256) colsum_final_kernel(const float* __restri
   double t = 0.0;
   for (int i = 0; i < S; ++i) t += (double)scratch[((size_t)job * S + i) * N + n];
   float* out = job ? out1 : out0;
-  out[n] = accumulate ? (float)((double)out[n] + t) : (float)t;
+  if (accumulate == kAccumAfterSum) out[n] = out[n] + (float)t;
+  else out[n] = accumulate ? (float)((double)out[n] + t) : (float)t;
 }
 
 }  // namespace

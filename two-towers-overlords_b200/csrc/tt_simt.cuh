@@ -23,6 +23,11 @@ int sgemm(const SgemmArgs& a, cudaStream_t st);
 // out[n] (+)= sum_m X[m*ld + n], fixed summation order
 int colsum(const float* X, int M, int N, long long ld, float* out, int accumulate, cudaStream_t st);
 
+// `accumulate` of colsum2 and of the split-K reduction (launch_gemm): 0 = out is overwritten; kAccumOldFirst = the
+// running sum starts from out (tt_encode_bwd); kAccumAfterSum = out = fl(out + sum) in fp32, the sum being exactly what
+// 0 writes (tt_step_args.grad_accumulate, autograd's `.grad += new`)
+constexpr int kAccumOldFirst = 1, kAccumAfterSum = 2;
+
 // same sums for one or two matrices (X1 nullable) in two launches; scratch: 2 * kColsumSlices * N floats
 constexpr int kColsumSlices = 32;
 int colsum2(const float* X0, int M0, float* out0, const float* X1, int M1, float* out1, int N, long long ld,

@@ -35,6 +35,7 @@ struct StepSm100 {
   int phases;                 // 0 / TT_STEP_FRONT | TT_STEP_BACK
   FusedAdam adam;
   bool chain;                 // persistent chain kernel (else one kernel per contraction)
+  int grad_accumulate;        // 1: every gradient output becomes fl(old + new) (tt_step_args.grad_accumulate)
 };
 size_t step_sm100_ws_bytes(int B, int H, int P, int train_table);
 int step_sm100(const StepSm100& s, cudaStream_t st);

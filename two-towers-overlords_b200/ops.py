@@ -370,11 +370,13 @@ class TripletStep:
                       float(lr), float(betas[0]), float(betas[1]), float(eps))
         self._keep.append((state, param, grad, exp_avg, exp_avg_sq))
 
-    def run(self, slot: int = 0, phases: int = 0, optimise: bool = False):
+    def run(self, slot: int = 0, phases: int = 0, optimise: bool = False, accumulate: bool = False):
         """phases: 0 = whole step, 1 = pooled gather only (TT_STEP_FRONT), 2 = the rest (TT_STEP_BACK).
-        optimise: also apply the optimiser bound with bind_adam() (gradients only otherwise)."""
+        optimise: also apply the optimiser bound with bind_adam() (gradients only otherwise).
+        accumulate: add this micro-batch's gradients to the gradient buffers (tt_step_args.grad_accumulate)."""
         a = self.slots[slot]
         a.phases = int(phases)
+        a.grad_accumulate = int(bool(accumulate))
         if optimise and phases != 1:
             assert self._adam is not None, "run(optimise=True) needs bind_adam() first"
             (a.adam_state, a.adam_param, a.adam_grad, a.adam_exp_avg, a.adam_exp_avg_sq, a.adam_n, a.adam_lr,
@@ -384,6 +386,7 @@ class TripletStep:
         N.check(self.lib.tt_triplet_step(ctypes.byref(a), N.stream()), "tt_triplet_step")
         a.phases = 0
         a.adam_param = None
+        a.grad_accumulate = 0
         return self.loss
 
 

@@ -119,6 +119,39 @@ def train_epoch_optimized(model, dataloader, criterion, optimizer, device, scale
 # --------------------------------------------------------------------------------------------------
 # fused B200 trainer
 # --------------------------------------------------------------------------------------------------
+class AccumulationWindow:
+    """Optimiser cadence of the reference's gradient accumulation (backend/training.py:66-133) over micro-steps: the
+    optimiser runs after micro-batch `batch_idx` whenever (batch_idx + 1) % a == 0, batch_idx restarts at 0 every epoch,
+    and a trailing partial window carries its gradient into the next epoch's first window.  Host only."""
+
+    def __init__(self, accumulation_steps: int):
+        if (isinstance(accumulation_steps, bool) or int(accumulation_steps) != accumulation_steps
+                or accumulation_steps < 1):
+            raise ValueError(f"accumulation_steps must be an integer >= 1, got {accumulation_steps!r}")
+        self.a = int(accumulation_steps)
+        self.batch_idx = 0  # micro-batch position in the epoch
+        self.pending = 0    # micro-batches summed in the gradient buffers since the last optimiser step
+
+    def start_epoch(self):
+        self.batch_idx = 0
+
+    def mode(self) -> tuple:
+        """(accumulate, close) of the next micro-step: add to the gradient buffers (they carry an unstepped gradient)
+        instead of overwriting them; run the optimiser after it."""
+        return (self.pending > 0, (self.batch_idx + 1) % self.a == 0)
+
+    def advance(self):
+        close = self.mode()[1]
+        self.batch_idx += 1
+        self.pending = 0 if close else self.pending + 1
+
+    def modes(self) -> list:
+        """Every mode the schedule can reach: a = 1 overwrites and steps every time; a > 1 opens a window by
+        overwriting, continues it by adding, closes it by adding and stepping — and a first window that continues a
+        carried partial one starts by adding."""
+        return [(False, True)] if self.a == 1 else [(False, False), (True, False), (True, True)]
+
+
 class FusedTrainer:
     """Whole training step (training.py:37-51) as: tokens into a static slot (one packed H2D copy or the device
     feeder) -> tt_triplet_step -> tt_adam_step_dev (one GPU) / tt_dp_reduce_adam (data parallel, peer memory) /
@@ -128,14 +161,23 @@ class FusedTrainer:
     the rest of `slot` (it reads tokens and the frozen tables only, so this is still exact synchronous SGD).
     The 8 projection tensors are re-pointed at views of one flat fp32 buffer, so the model's
     `state_dict()` / `parameters()` always see the trained values; gradients live in a second flat buffer
-    whose last element carries the loss (one exchange covers both)."""
+    whose last element carries the loss (one exchange covers both).
+
+    `accumulation_steps = a` reproduces the reference's gradient accumulation (backend/training.py:66-133): every
+    micro-batch (one step() call) adds the gradient of loss / a into the flat gradient, and the optimiser (and, data
+    parallel, the one exchange) runs after micro-batch `batch_idx` of the epoch whenever (batch_idx + 1) % a == 0.
+    `batch_idx` restarts at 0 with every epoch (train_epoch / train_epoch_device / start_epoch()); a trailing partial
+    window is not stepped and its gradient carries into the next epoch's first window, as in the reference.  a = 1 is
+    the plain trainer."""
 
     def __init__(self, model: TwoTowersModel, margin: float, lr: float, batch_size: int, Lq: int = 32, Ld: int = 256,
                  precision: Optional[str] = None, world_size: int = 1, rank: int = 0, use_graph: bool = True,
                  betas=(0.9, 0.999), eps: float = 1e-8, process_group=None, ids_dtype=torch.int32,
                  mask_dtype=torch.uint8, token_slots: int = 1, exchange: Optional[str] = None,
-                 exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None):
+                 exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None, accumulation_steps: int = 1):
         qt, dt = model.query_tower, model.document_tower
+        self.window = AccumulationWindow(accumulation_steps)
+        self.accum = self.window.a
         self.model = model
         self.device = qt.pretrained_model.device
         if self.device.type != "cuda":
@@ -265,8 +307,9 @@ class FusedTrainer:
                                  train_table=self.train_table)
             so.loss = self.flat_g[self.n_param:]  # this rank's loss term lands in the flat gradient's last slot
             tables = None if self.pooled else (qt.pretrained_model.table.data, dt.pretrained_model.table.data)
-            so.bind(self.tok, tables, self.p_views, self.g_views, self.margin, 1.0 / (batch_size * world_size), 1.0,
-                    self.table_grads)
+            # upstream gradient 1/a: the reference backpropagates loss / accumulation_steps
+            so.bind(self.tok, tables, self.p_views, self.g_views, self.margin, 1.0 / (batch_size * world_size),
+                    1.0 / self.accum, self.table_grads)
             for toks in self.tok_slots[1:]:
                 so.add_tokens(toks)
             if self.pooled:
@@ -309,6 +352,11 @@ class FusedTrainer:
         self._warm = False
         self.steps_done = 0
         self.kernel_launches_per_step = None
+        # data parallel with accumulation: the exchange (which publishes the global loss) runs on closing micro-steps
+        # only, so the epoch's loss is this rank's share of every micro-batch's global loss, summed over the ranks once
+        # per epoch
+        self._loss_share = (torch.zeros((), dtype=torch.float64, device=dev)
+                            if self.world > 1 and self.accum > 1 else None)
 
     # -- data-parallel hygiene ---------------------------------------------------------------------
     def _dist_ready(self) -> bool:
@@ -382,24 +430,28 @@ class FusedTrainer:
         self.neg_bufs[slot].copy_(neg_index.to(torch.int32), non_blocking=True)
         self._neg_loaded[slot] = True
 
-    def _fwd_bwd(self, slot: int = 0, phases: int = 0, parity: int = 0, optimise: bool = False):
-        self.step_objs[parity].run(slot, phases, optimise=optimise)
+    def _fwd_bwd(self, slot: int = 0, phases: int = 0, parity: int = 0, optimise: bool = False,
+                 accumulate: bool = False):
+        self.step_objs[parity].run(slot, phases, optimise=optimise, accumulate=accumulate)
 
     def _exchange(self):
         """The fused reduce-scatter / Adam / all-gather kernel (tt_dp_reduce_adam) on the current stream."""
         self.xchg.reduce_adam(self.flat_g, self.exp_avg, self.exp_avg_sq, self.lr, self.betas, self.eps,
                               self.exchange_ctas)
 
-    def _pipelined(self, slot: int, next_slot: Optional[int], parity: int):
+    def _pipelined(self, slot: int, next_slot: Optional[int], parity: int, mode=(False, True)):
         """One training step on the current stream, in the schedule __init__ chose: whole step (gather -> persistent
         chain kernel), per-kernel chain beside the look-ahead gather of `next_slot`, or — data parallel — persistent
-        chain, then the exchange beside the look-ahead gather."""
+        chain, then the exchange beside the look-ahead gather.  mode = (accumulate, close): add the gradients to the
+        buffers instead of overwriting them; run the optimiser / the exchange (a closing micro-step)."""
         cur = torch.cuda.current_stream()
-        fused_opt = self.xchg is None and self.world == 1
+        acc, close = mode
+        fused_opt = self.xchg is None and self.world == 1 and close
+        exchange = self.xchg is not None and close
         if self._whole_step():
             # ONE call = pooled gather -> persistent chain kernel (+ Adam in its tail): two launches, the second a
             # programmatic dependent of the first
-            self._fwd_bwd(slot, 0, parity, optimise=fused_opt)
+            self._fwd_bwd(slot, 0, parity, optimise=fused_opt, accumulate=acc)
             return
         chain_mode = self.step_objs[0].chain_active()
         if not chain_mode:
@@ -408,8 +460,8 @@ class FusedTrainer:
                 self.side.wait_stream(cur)
                 with torch.cuda.stream(self.side):
                     self._fwd_bwd(next_slot, 1, parity ^ 1)
-            self._fwd_bwd(slot, 2, parity, optimise=fused_opt)
-            if self.xchg is not None:
+            self._fwd_bwd(slot, 2, parity, optimise=fused_opt, accumulate=acc)
+            if exchange:
                 self._exchange()
             if next_slot is not None:
                 cur.wait_stream(self.side)
@@ -417,12 +469,12 @@ class FusedTrainer:
         # Persistent chain kernel + data parallelism: the chain wants one CTA on EVERY SM (its CTAs wait for each other),
         # so nothing runs beside it; the look-ahead gather runs beside the exchange kernel instead, which spends most
         # of its time waiting for the peers' gradient flags on one small CTA per SM.
-        self._fwd_bwd(slot, 2, parity, optimise=fused_opt)
+        self._fwd_bwd(slot, 2, parity, optimise=fused_opt, accumulate=acc)
         if next_slot is not None:
             self.side.wait_stream(cur)
             with torch.cuda.stream(self.side):
                 self._fwd_bwd(next_slot, 1, parity ^ 1)
-        if self.xchg is not None:
+        if exchange:
             self._exchange()
         if next_slot is not None:
             cur.wait_stream(self.side)
@@ -461,25 +513,32 @@ class FusedTrainer:
         # (table training uses a plain SGD-free path: the caller owns the table optimiser)
 
     def _warm_up(self):
-        # one eager forward/backward on a side stream (first-use kernel attributes), gradients only: harmless
+        # one eager forward/backward on a side stream (first-use kernel attributes), gradients only: harmless, except
+        # that it overwrites the gradient buffers, so an open window (a resumed checkpoint) is put back afterwards
+        keep = None
+        if self.window.pending:
+            keep = [t.clone() for t in (self.flat_g,) + tuple(self.table_grads or ())]
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
             self._fwd_bwd(0, 0, 0)
             self._fwd_bwd(0, 0, 1)
         torch.cuda.current_stream().wait_stream(s)
+        if keep is not None:
+            for t, k in zip((self.flat_g,) + tuple(self.table_grads or ()), keep):
+                t.copy_(k)
         torch.cuda.synchronize()
         self._warm = True
 
-    def _graph(self, slot: int, next_slot: Optional[int], parity: int):
-        key = (slot, next_slot, parity)
+    def _graph(self, slot: int, next_slot: Optional[int], parity: int, mode=(False, True)):
+        key = (slot, next_slot, parity, mode)
         g = self.graphs.get(key)
         if g is None:
             lib = ops.N.load()
             n0 = lib.tt_launch_count()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, stream=self.cap_stream):
-                self._pipelined(slot, next_slot, parity)
+                self._pipelined(slot, next_slot, parity, mode)
             self.graphs[key] = g
             self.graph_captures += 1
             self.kernel_launches_per_step = lib.tt_launch_count() - n0
@@ -491,6 +550,20 @@ class FusedTrainer:
                 self.kernel_launches_per_step += 2  # adam_advance + adam
         return g
 
+    def start_epoch(self):
+        """The reference's batch_idx restarts at 0 every epoch; a trailing partial window stays in the gradient
+        buffers and is continued by the next epoch's first window.  train_epoch / train_epoch_device call this."""
+        self.window.start_epoch()
+        if self._loss_share is not None:
+            self._loss_share.zero_()
+
+    def _epoch_average(self, total: torch.Tensor, n: int) -> float:
+        if self._loss_share is not None:
+            total = self._loss_share.clone()
+            if self._dist_ready():
+                torch.distributed.all_reduce(total, group=self.pg)
+        return float(total.item()) / n
+
     def prepare(self, n_slots: Optional[int] = None):
         """Captures the steady-state graphs of a round-robin schedule over the first `n_slots` token slots
         (step(s, (s + 1) % n_slots)), so no capture happens inside a timed region."""
@@ -500,19 +573,23 @@ class FusedTrainer:
             return
         if not self._warm:
             self._warm_up()
-        for s_ in range(n):
-            if self._whole_step():
-                self._graph(s_, None, self._parity)  # whole-step graphs: no look-ahead, one workspace
-                continue
-            nxt = (s_ + 1) % n
-            for parity in ((s_ & 1,) if n % 2 == 0 else (0, 1)):
-                self._graph(s_, nxt, parity)
+        for mode in self.window.modes():
+            for s_ in range(n):
+                if self._whole_step():
+                    self._graph(s_, None, self._parity, mode)  # whole-step graphs: no look-ahead, one workspace
+                    continue
+                nxt = (s_ + 1) % n
+                for parity in ((s_ & 1,) if n % 2 == 0 else (0, 1)):
+                    self._graph(s_, nxt, parity, mode)
         self.sync_ranks()  # capture time differs per rank: line the ranks up before the first exchanged step
 
     def step(self, slot: int = 0, next_slot: Optional[int] = None) -> torch.Tensor:
-        """One optimiser step on the tokens in the static buffers of `slot`; returns the (global) loss as a device
-        scalar — no host sync.  `next_slot`: slot holding the tokens of the FOLLOWING step (already resident);
-        its pooled gather then runs beside this step and the following step(next_slot, ...) skips it."""
+        """One micro-step on the tokens in the static buffers of `slot` (an optimiser step when it closes a window of
+        accumulation_steps micro-batches; always, with a = 1); returns the loss as a device scalar — no host sync: the
+        micro-batch's global loss, except on a data-parallel micro-step that does not close its window, which runs no
+        exchange and returns this rank's share of the global loss (its hinge sum over the global batch size; the shares
+        of all ranks add up to the global loss).  `next_slot`: slot holding the tokens of the FOLLOWING step (already
+        resident); its pooled gather then runs beside this step and the following step(next_slot, ...) skips it."""
         if not self._warm:
             self._warm_up()
         if self.neg_bufs is not None and not self._neg_loaded[slot]:
@@ -534,13 +611,17 @@ class FusedTrainer:
             self._parity = slot & 1
             self._fwd_bwd(slot, 1, self._parity)
         parity = self._parity
+        mode = self.window.mode()
         if self.use_graph:
-            self._graph(slot, next_slot, parity).replay()
+            self._graph(slot, next_slot, parity, mode).replay()
         else:
             n0 = lib.tt_launch_count()
-            self._pipelined(slot, next_slot, parity)
+            self._pipelined(slot, next_slot, parity, mode)
             self.kernel_launches_per_step = lib.tt_launch_count() - n0
-        if self.world > 1 and self.xchg is None:
+        if self._loss_share is not None:  # before the all-reduce below sums the loss slot over the ranks
+            self._loss_share += self.flat_g[self.n_param].double()
+        close = mode[1]
+        if self.world > 1 and self.xchg is None and close:
             torch.distributed.all_reduce(self.flat_g, group=self.pg)
             if self.use_graph:
                 self.graph_opt.replay()
@@ -551,6 +632,9 @@ class FusedTrainer:
         if next_slot is not None:
             self._parity ^= 1
         self.steps_done += 1
+        self.window.advance()
+        if not close:  # no exchange published a loss: this rank's term (the whole loss on one GPU)
+            return self.flat_g[self.n_param]
         return self.loss_view[0]
 
     def train_epoch_device(self, feeder, log_every: int = 0) -> float:
@@ -561,6 +645,7 @@ class FusedTrainer:
             raise ZeroDivisionError("FusedTrainer.train_epoch_device: not enough pairs for one batch")
         self.check_banks()
         feeder.start_epoch()
+        self.start_epoch()
         total = torch.zeros((), dtype=torch.float64, device=self.device)
         n_slots = len(self.tok_slots)
         feeder.assemble(self, 0, 0)
@@ -579,7 +664,7 @@ class FusedTrainer:
                     print(f"Batch {i + 1}, Loss: {loss.item():.4f}")
                 self.check()
         feeder.check()
-        avg = float(total.item()) / steps
+        avg = self._epoch_average(total, steps)
         self.check()
         return avg
 
@@ -591,17 +676,41 @@ class FusedTrainer:
 
     def state_dict(self) -> dict:
         """Model weights (reference key names) + Adam moments and step count.  Collective in peer mode with
-        world_size > 1 (the moments are sharded over the ranks there)."""
+        world_size > 1 (the moments are sharded over the ranks there).  Inside an open accumulation window it also holds
+        the window: "accumulation_steps", "window_batch_idx", "window_pending" and the gradient buffers ("window_grad",
+        and "window_table_grads" when the tables train).  Data parallel, every rank's partial gradient differs, so a
+        save inside a window raises there."""
+        if self.window.pending and self.world > 1:
+            raise RuntimeError(f"FusedTrainer.state_dict: {self.window.pending} micro-batches of an accumulation "
+                               "window are pending and every rank's partial gradient differs; save at a window "
+                               f"boundary (after a micro-step with (batch_idx + 1) % {self.accum} == 0)")
         m, v = self.exp_avg.clone(), self.exp_avg_sq.clone()
         if self.xchg is not None and self.world > 1:
             torch.distributed.all_reduce(m, group=self.pg)   # every rank holds zeros outside its own slice
             torch.distributed.all_reduce(v, group=self.pg)
         st = self.xchg.state if self.xchg is not None else self.adam_state
-        return {"model": {k: t.detach().cpu().clone() for k, t in self.model.state_dict().items()},
-                "exp_avg": m.cpu(), "exp_avg_sq": v.cpu(), "adam_state": st.detach().cpu().clone(),
-                "steps_done": self.steps_done, "lr": self.lr, "betas": tuple(self.betas), "eps": self.eps}
+        sd = {"model": {k: t.detach().cpu().clone() for k, t in self.model.state_dict().items()},
+              "exp_avg": m.cpu(), "exp_avg_sq": v.cpu(), "adam_state": st.detach().cpu().clone(),
+              "steps_done": self.steps_done, "lr": self.lr, "betas": tuple(self.betas), "eps": self.eps}
+        if self.window.pending:
+            sd.update(accumulation_steps=self.accum, window_batch_idx=self.window.batch_idx,
+                      window_pending=self.window.pending, window_grad=self.flat_g[: self.n_param].cpu().clone())
+            if self.table_grads is not None:
+                sd["window_table_grads"] = tuple(t.cpu().clone() for t in self.table_grads)
+        return sd
 
     def load_state_dict(self, sd: dict):
+        pending = int(sd.get("window_pending", 0))
+        if pending:
+            if int(sd["accumulation_steps"]) != self.accum:
+                raise ValueError(f"FusedTrainer.load_state_dict: the checkpoint was saved inside a window of "
+                                 f"accumulation_steps = {sd['accumulation_steps']}, this trainer has {self.accum}")
+            if self.world > 1:
+                raise ValueError("FusedTrainer.load_state_dict: a checkpoint inside an accumulation window holds one "
+                                 "rank's partial gradient; data-parallel training resumes at window boundaries only")
+            if ("window_table_grads" in sd) != (self.table_grads is not None):
+                raise ValueError("FusedTrainer.load_state_dict: the checkpoint's open window and this trainer disagree "
+                                 "on whether the token tables train")
         model_sd = sd["model"]
         if self.pooled is not None:
             # The pooled banks were computed from the frozen backbone and are keyed to its tensors' versions: copying the
@@ -632,6 +741,13 @@ class FusedTrainer:
         else:
             self.adam_state.copy_(sd["adam_state"])
         self.steps_done = int(sd.get("steps_done", 0))
+        # a checkpoint without an open window resumes at a window start
+        self.window.pending = pending
+        self.window.batch_idx = int(sd["window_batch_idx"]) if pending else 0
+        if pending:
+            self.flat_g[: self.n_param].copy_(sd["window_grad"])
+            for t, src in zip(self.table_grads or (), sd.get("window_table_grads", ())):
+                t.copy_(src)
         self._primed = None
         self._sync_initial_state()
 
@@ -666,6 +782,7 @@ class FusedTrainer:
         """One pass over the loader.  With >= 2 token slots the next batch is staged one step ahead so that its
         pooled gather overlaps the current step."""
         self.check_banks()
+        self.start_epoch()
         total = torch.zeros((), dtype=torch.float64, device=self.device)
         nb = 0
         n_slots = len(self.tok_slots)
@@ -693,7 +810,7 @@ class FusedTrainer:
             else:
                 slot = nslot if nslot is not None else slot
             cur = nxt
-        avg = float(total.item()) / nb
+        avg = self._epoch_average(total, nb)
         self.check()
         return avg
 
@@ -1020,6 +1137,7 @@ def run_training(
     table_dtype: torch.dtype = torch.float32,
     backbone: Optional[str] = None,
     hard_negatives: Union[None, int, dict] = None,
+    fused_accumulation: Optional[bool] = None,
 ) -> TwoTowersModel:
     """Main training function (training.py:383-529).  `fused` (additive) selects the FusedTrainer; by
     default it is used whenever the dataset is token-bank backed and no gradient accumulation / wandb
@@ -1033,7 +1151,20 @@ def run_training(
     `hard_negatives` (additive): mined negatives on the fused path with the device feeder (data.HardNegativeMiner).
     None reads TT_HARD_NEGATIVES (unset or 0 = off, the default; an integer d = on with depth d); an int d is the same;
     a dict holds the miner's arguments plus "warmup_epochs" (default 1).  After warmup_epochs epochs of in-batch
-    negatives the table is re-mined from the current towers at the start of every epoch."""
+    negatives the table is re-mined from the current towers at the start of every epoch.
+
+    `fused_accumulation` (additive): honour `accumulation_steps` on the fused path (FusedTrainer(accumulation_steps=a):
+    micro-batches add into the flat gradient, one optimiser step and, data parallel, one exchange per window).  None
+    reads TT_FUSED_ACCUMULATION (unset or 0 = off, the default).  Off, one GPU takes the fused path only at
+    accumulation_steps == 1 and data-parallel runs step every global batch."""
+    if isinstance(accumulation_steps, bool) or not isinstance(accumulation_steps, int) or accumulation_steps < 1:
+        raise ValueError(f"accumulation_steps must be an integer >= 1, got {accumulation_steps!r}")
+    if fused_accumulation is None:
+        env = os.environ.get("TT_FUSED_ACCUMULATION", "0").strip() or "0"
+        try:
+            fused_accumulation = int(env) != 0
+        except ValueError:
+            raise ValueError(f"TT_FUSED_ACCUMULATION must be 0 or 1, got {env!r}") from None
     hn = hard_negative_config(hard_negatives)
     if backbone is None:
         backbone = os.environ.get("TT_BACKBONE", "table")
@@ -1107,9 +1238,9 @@ def run_training(
     bank_backed = use_bank_tokenizer(train_ds, val_ds) is not None
     train_dl = TripletDataLoader(train_ds, batch_size=batch_size, num_workers=num_workers, device=device)
     if fused is None:
-        # one GPU: the reference-shaped loops serve gradient accumulation and wandb's gradient hooks; several GPUs:
-        # only the fused step exchanges gradients, so it is the path (accumulation folds into the larger global batch)
-        fused = bank_backed and (world > 1 or (accumulation_steps == 1 and not use_wandb))
+        # one GPU: the reference-shaped loops serve wandb's gradient hooks and, unless fused_accumulation, gradient
+        # accumulation; several GPUs: only the fused step exchanges gradients, so it is the path
+        fused = bank_backed and (world > 1 or ((accumulation_steps == 1 or fused_accumulation) and not use_wandb))
     if world > 1 and not fused:
         raise ValueError("data-parallel training needs the fused step (a token-bank dataset and fused != False)")
     host_feeder = os.environ.get("TT_HOST_FEEDER") == "1" or len(train_ds) < 2 * batch_size
@@ -1117,14 +1248,16 @@ def run_training(
         raise ValueError("hard negatives need the fused step with the device feeder (DeviceTripletFeeder); the "
                          "reference-shaped loops and TokenTripletLoader draw in-batch negatives only (unset "
                          "TT_HOST_FEEDER, use at least two batches of pairs)")
-    if world > 1 and accumulation_steps != 1:
-        say(f"  note: accumulation_steps={accumulation_steps} is ignored under data parallelism; the global batch "
-            f"of {batch_size} triplets is one optimiser step")
+    # micro-batches per optimiser step of the fused trainer
+    fused_accum = accumulation_steps if fused_accumulation else 1
+    if fused and accumulation_steps != 1 and not fused_accumulation:
+        say(f"  note: accumulation_steps={accumulation_steps} is ignored by the fused step (TT_FUSED_ACCUMULATION=1 "
+            f"honours it); the batch of {batch_size} triplets is one optimiser step")
 
     say("Training configuration:")
     say(f"  Physical batch size: {batch_size}")
     say(f"  Gradient accumulation steps: {accumulation_steps}")
-    say(f"  Effective batch size: {batch_size * (accumulation_steps if world == 1 else 1)}")
+    say(f"  Effective batch size: {batch_size * (fused_accum if fused else accumulation_steps)}")
     say(f"  Mixed precision: {use_mixed_precision}")
     say(f"  DataLoader workers: {num_workers}")
     say(f"  Fused B200 step: {fused}")
@@ -1145,7 +1278,7 @@ def run_training(
             say(f"Encoded {len(banks[0]) + len(banks[1])} training texts ({len(banks[0])} queries, "
                 f"{len(banks[1])} passages) with the frozen MiniLM backbone in {time.perf_counter() - t0:.1f}s")
             trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, Lq, Ld, token_slots=2,
-                                   world_size=world, rank=rank, pooled=banks)
+                                   world_size=world, rank=rank, pooled=banks, accumulation_steps=fused_accum)
         else:
             # the device feeder draws the in-batch negatives itself and hands their indices to the trainer, which then
             # pools every positive document once (TT_NEG_REUSE=0: gather the negatives' tokens like any document)
@@ -1155,7 +1288,7 @@ def run_training(
                 reuse = False
                 say("  Hard negatives: neg-index reuse is off (a mined negative is not a positive of the batch)")
             trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, token_slots=2, world_size=world,
-                                   rank=rank, in_batch_negatives=reuse)
+                                   rank=rank, in_batch_negatives=reuse, accumulation_steps=fused_accum)
             if hn is not None:  # the frozen table's pooled rows, for mining only (the step still pools tokens)
                 banks = (PooledBank.build(model.query_tower, train_ds.query_bank, trainer.Lq, world_size=world,
                                           rank=rank),
