@@ -102,8 +102,10 @@ extern "C" int tt_device_info(int* sms, int* cc_major, int* cc_minor) {
 // ------------------------------------------------------------------------------------------------
 // tower MLP
 // ------------------------------------------------------------------------------------------------
+// fp32: h (forward without h) or dz1 [M, P], then the backward's slice sums
 extern "C" size_t tt_mlp_ws_bytes(int M, int H, int P, int precision) {
-  if (precision == TT_PREC_FP32) return ws_round((size_t)M * P * 4) + 256;
+  if (precision == TT_PREC_FP32)
+    return ws_round((size_t)M * P * 4) + ws_round(mlp_bwd_fp32_scratch_floats(M, H, P) * 4) + 256;
   return mlp_sm100_ws_bytes(M, H, P) + 256;
 }
 
@@ -148,9 +150,12 @@ extern "C" int tt_encode_bwd(const float* dy, const float* x, const float* h, co
     return 0;
   }
   TT_REQUIRE(ws_bytes >= tt_mlp_ws_bytes(M, H, P, precision), "tt_encode_bwd: workspace too small");
-  if (precision == TT_PREC_FP32)
-    return mlp_bwd_fp32(dy, x, h, W1, W2, M, H, P, dW1, db1, dW2, db2, dx, accumulate, reinterpret_cast<float*>(ws),
+  if (precision == TT_PREC_FP32) {
+    char* p = reinterpret_cast<char*>(ws);
+    float* dz1 = ws_take<float>(p, (size_t)M * P);
+    return mlp_bwd_fp32(dy, x, h, W1, W2, M, H, P, dW1, db1, dW2, db2, dx, accumulate, dz1, reinterpret_cast<float*>(p),
                         st);
+  }
   return mlp_bwd_sm100(dy, x, h, W1, W2, M, H, P, dW1, db1, dW2, db2, dx, accumulate, precision, ws, ws_bytes, st);
 }
 
@@ -159,6 +164,7 @@ extern "C" int tt_encode_bwd(const float* dy, const float* x, const float* h, co
 // ------------------------------------------------------------------------------------------------
 struct ApiStepWs {
   float *xhat, *cnt, *nrm, *h, *y, *stats, *dy, *dz1, *dxhat, *g;
+  float* fp32_scratch;  // mlp_bwd_fp32's slice sums, shared by both towers (fp32 only)
   void* pool_ws;
   size_t pool_ws_bytes;
   void* mma_ws;
@@ -188,6 +194,8 @@ static size_t carve_step_ws(char* base, int B, int Lq, int Ld, int H, int P, int
   if (precision != TT_PREC_FP32) {
     w.mma_ws_bytes = step_sm100_ws_bytes(B, H, P, train_table);
     w.mma_ws = ws_take<char>(p, w.mma_ws_bytes);
+  } else {
+    w.fp32_scratch = ws_take<float>(p, mlp_bwd_fp32_scratch_floats(2 * B, H, P));
   }
   if (out) *out = w;
   return (size_t)(p - base) + 256;
@@ -295,13 +303,15 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
     if ((rc = triplet_loss_bwd(yq, yp, yn, w.stats, nullptr, a->grad_scale, B, P, a->inv_batch, w.dy,
                                w.dy + (size_t)B * P, w.dy + (size_t)2 * B * P, nullptr, st)))
       return rc;
-    // 5. tower backward (document tower: positives and negatives in one M = 2B pass)
-    if ((rc = mlp_bwd_fp32(w.dy, w.xhat, w.h, a->Wq1, a->Wq2, B, H, P, a->dWq1, a->dbq1, a->dWq2, a->dbq2, dxhat, acc,
-                           w.dz1, st)))
+    // 5. tower backward (document tower: positives and negatives in one M = 2B pass); grad_accumulate adds the old
+    // gradient after the sum, as the tensor-core chains do
+    const int facc = acc ? kAccumAfterSum : 0;
+    if ((rc = mlp_bwd_fp32(w.dy, w.xhat, w.h, a->Wq1, a->Wq2, B, H, P, a->dWq1, a->dbq1, a->dWq2, a->dbq2, dxhat, facc,
+                           w.dz1, w.fp32_scratch, st)))
       return rc;
     if ((rc = mlp_bwd_fp32(w.dy + (size_t)B * P, w.xhat + (size_t)B * H, w.h + (size_t)B * P, a->Wd1, a->Wd2, 2 * B, H,
-                           P, a->dWd1, a->dbd1, a->dWd2, a->dbd2, dxhat ? dxhat + (size_t)B * H : nullptr, acc,
-                           w.dz1 + (size_t)B * P, st)))
+                           P, a->dWd1, a->dbd1, a->dWd2, a->dbd2, dxhat ? dxhat + (size_t)B * H : nullptr, facc,
+                           w.dz1 + (size_t)B * P, w.fp32_scratch, st)))
       return rc;
   } else {
     StepSm100 s{};

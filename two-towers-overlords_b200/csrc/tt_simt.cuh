@@ -5,6 +5,7 @@ namespace tt {
 
 // C[m,n] = epi( sum_k A(m,k) * B(n,k) ), A(m,k) = A[m*a_sm + k*a_sk], B(n,k) = B[n*b_sn + k*b_sk].
 // epi: (+bias[n]) -> (relu) -> (* (gate[m*ldc+n] > 0)) -> (C += | C =)
+// kslice > 0 (set by sgemm_rows): CTA z sums k in [z*kslice, (z+1)*kslice) into C + z*M*ldc
 struct SgemmArgs {
   const float* A;
   long long a_sm, a_sk;
@@ -17,11 +18,9 @@ struct SgemmArgs {
   int relu;
   const float* gate;
   int accumulate;
+  int kslice;
 };
 int sgemm(const SgemmArgs& a, cudaStream_t st);
-
-// out[n] (+)= sum_m X[m*ld + n], fixed summation order
-int colsum(const float* X, int M, int N, long long ld, float* out, int accumulate, cudaStream_t st);
 
 // `accumulate` of colsum2 and of the split-K reduction (launch_gemm): 0 = out is overwritten; kAccumOldFirst = the
 // running sum starts from out (tt_encode_bwd); kAccumAfterSum = out = fl(out + sum) in fp32, the sum being exactly what
@@ -33,12 +32,21 @@ constexpr int kColsumSlices = 32;
 int colsum2(const float* X0, int M0, float* out0, const float* X1, int M1, float* out1, int N, long long ld,
             int accumulate, float* scratch, cudaStream_t st);
 
-// fp32 strict-mode projection (tt_mlp_simt.cu)
+// C [M, N] dense (+)= sum_k A(m,k) B(n,k) as row_slices(K) fixed, non-empty slices of K (at most kRowSlices), each an
+// sgemm into partial [slice][M*N], then added in ascending slice order in double; accumulate as for colsum2.  For the
+// weight gradients, whose K is the batch: short fp32 chains, and a grid of slices x tiles instead of tiles alone.
+constexpr int kRowSlices = 32;
+int row_slices(int K);
+int sgemm_rows(const SgemmArgs& a, float* partial, cudaStream_t st);
+
+// fp32 strict-mode projection (tt_mlp_simt.cu).  mlp_bwd_fp32: dz1 [M, P]; scratch of
+// mlp_bwd_fp32_scratch_floats(M, H, P) floats (weight-gradient slices, column-sum slices); accumulate as for colsum2
 int mlp_fwd_fp32(const float* x, int M, int H, int P, const float* W1, const float* b1, const float* W2,
                  const float* b2, float* h, float* y, cudaStream_t st);
 int mlp_bwd_fp32(const float* dy, const float* x, const float* h, const float* W1, const float* W2, int M, int H,
                  int P, float* dW1, float* db1, float* dW2, float* db2, float* dx, int accumulate, float* dz1,
-                 cudaStream_t st);
+                 float* scratch, cudaStream_t st);
+size_t mlp_bwd_fp32_scratch_floats(int M, int H, int P);
 
 // loss (tt_loss.cu)
 struct LossSplitOut {  // optional operands for the tensor-core backward: dY as bf16 hi/lo, row-major + transposed
