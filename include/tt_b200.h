@@ -422,8 +422,9 @@ int tt_encoder_fwd(const tt_encoder_weights* w, const void* ids, int ids_dtype, 
 int tt_split_bf16_terms(const float* x, int rows, int cols, void* hi, void* lo, tt_stream_t stream);
 
 /* Diagnostics / parity tests: device address of a named internal buffer of a tensor-core step workspace:
- * "trace" (task timeline of the persistent chain kernel after a TT_CHAIN_TRACE=1 step: [160][64] pairs of
- * {task << 2 | kind, globaltimer ns}), "x_hi" / "x_lo" / "x_lo2" (bf16 terms [3B,H] of the pooled rows; x_lo2 in
+ * "trace" (task timeline of the persistent chain kernel after a TT_CHAIN_TRACE=1 step: [160][128] pairs of
+ * {task << 4 | event, globaltimer ns}; the launch does not clear it, so the caller zeroes it before the launch it
+ * wants to trace, or slots of earlier launches remain), "x_hi" / "x_lo" / "x_lo2" (bf16 terms [3B,H] of the pooled rows; x_lo2 in
  * bf16x3 steps only), "h_hi" / "h_lo" / "dy_hi" / "dy_lo" (bf16 terms [3B,P]); rows q | p | n. */
 int tt_debug_step_buffer(void* ws, int B, int Lq, int Ld, int H, int P, int vocab, int precision, int train_table,
                          const char* name, void** ptr);

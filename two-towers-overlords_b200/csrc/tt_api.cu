@@ -210,7 +210,9 @@ extern "C" size_t tt_step_ws_bytes(int B, int Lq, int Ld, int H, int P, int voca
 }
 
 // Diagnostics and parity tests: device address of a named internal buffer of a tensor-core step workspace.
-//   "trace"  per-CTA task timeline of the last TT_CHAIN_TRACE=1 step: [160][64] x {task << 2 | kind, globaltimer ns}
+//   "trace"  per-CTA task timeline of the last TT_CHAIN_TRACE=1 step: [160][128] x {task << 4 | event, globaltimer ns};
+//            the launch does not clear it (a memset would sit between the pooled gather and the chain kernel, its
+//            programmatic dependent): the caller zeroes it first, or slots of earlier launches remain
 //   "x_hi" / "x_lo" / "x_lo2"            bf16 terms [3B, H] of the pooled rows xhat (rows q | p | n; x_lo2 is written by
 //                                        bf16x3 steps only)
 //   "h_hi" / "h_lo" / "dy_hi" / "dy_lo"  bf16 terms [3B, P] of the hidden activations / of dY (rows q | p | n)

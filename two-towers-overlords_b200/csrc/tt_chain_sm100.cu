@@ -114,8 +114,8 @@ __device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
-__device__ __forceinline__ void signal(unsigned* p) {
-  asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
+__device__ __forceinline__ void red_relaxed(unsigned* p) {
+  asm volatile("red.relaxed.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async;" ::: "memory"); }
 __device__ __forceinline__ unsigned ld_relaxed(const unsigned* p) {
@@ -359,12 +359,25 @@ struct EpiCtx {
   int tslot, tidx;
 };
 
-// timeline event of the current task: kind 0 = start, 1 = end, 2 = accumulators ready, 3 = sibling sums arrived
-__device__ __forceinline__ void trace_ev(EpiCtx& e, int kind) {
+// timeline events of the current task, seen by epilogue thread 0 (scripts/chain_timeline.py names them)
+enum {
+  EV_START = 0, EV_END, EV_ACC,  // task start / end; accumulators ready (G: the dW2 partial tiles have arrived)
+  EV_STATS_IN,    // F2L: the row's partial sums of every column tile have arrived
+  EV_Y_OUT,       // F2L: y tile written to the exchange buffer
+  EV_Y_IN,        // F2L: the sibling row groups' y tiles have arrived
+  EV_PART_OUT,    // F2L: this task's partial sums written
+  EV_STATS_LOADED,  // F2L: the row's sums loaded and added
+  EV_STORED,      // results written, before the hand-off to other CTAs
+  EV_ALL_IN,      // G: every contraction task has signalled
+};
+// dep: a value the event waits for (the timer read is predicated on it, so it cannot issue before dep's loads land)
+__device__ __forceinline__ void trace_ev(EpiCtx& e, int kind, float dep = 0.f) {
   if (e.trace && e.tid == 0 && e.tslot < kTraceSlots) {
     unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    e.trace[e.tslot * 2] = ((unsigned long long)e.tidx << 2) | (unsigned long long)kind;
+    asm volatile(
+        "{\n .reg .pred p;\n setp.eq.f32 p, %1, %1;\n @p mov.u64 %0, %%globaltimer;\n @!p mov.u64 %0, %%globaltimer;\n}"
+        : "=l"(t) : "f"(dep) : "memory");
+    e.trace[e.tslot * 2] = ((unsigned long long)e.tidx << 4) | (unsigned long long)kind;
     e.trace[e.tslot * 2 + 1] = t;
     ++e.tslot;
   }
@@ -380,11 +393,26 @@ __device__ __forceinline__ void acc_advance(EpiCtx& e, int n) {
     e.aph ^= 1u;
   }
 }
-// all writes of this CTA's epilogue visible device-wide (also to TMA reads of other CTAs), then one signal per counter
-__device__ __forceinline__ void publish(const EpiCtx& e) {
-  fence_proxy_async();
-  __threadfence();
+// Hands everything the 256 epilogue threads have written so far to other CTAs: one barrier, then ONE gpu-scope release
+// by thread 0 (one fence, one relaxed add per counter).  Why that is enough, in the terms of the PTX ISA's memory
+// consistency model:
+//  - bar.sync: the barrier orders each participating thread's earlier memory accesses before every participant's
+//    later ones (instruction "bar, barrier"; it contributes to "Base causality order" like any synchronizes-with).
+//  - fence.acq_rel.gpu followed by a strong write to the counter is a release pattern, wait_counter's relaxed poll
+//    followed by fence.acq_rel.gpu the matching acquire pattern ("Release and acquire patterns").  Base causality
+//    order is transitive, so a write of any epilogue thread precedes every read the consumer issues after its acquire.
+//    cooperative_groups' grid sync and CUTLASS's GenericBarrier arrive the same way.
+//  - Proxies: h, dY and dz1 terms and the weight terms are read by other CTAs' TMA copies (async proxy).  A generic-
+//    proxy write and an async-proxy read of the same address are ordered when a proxy fence lies on the base-causality
+//    path between them ("Proxy-preserved base causality order"); the consumer's producer thread executes
+//    fence.proxy.async after its acquire and before it issues the copies (chain_kernel), so the writers need none.
+__device__ __forceinline__ void publish(const EpiCtx& e, unsigned* ctr, unsigned* ctr2 = nullptr) {
   epi_bar();
+  if (e.tid == 0) {
+    asm volatile("fence.acq_rel.gpu;" ::: "memory");
+    red_relaxed(ctr);
+    if (ctr2) red_relaxed(ctr2);
+  }
 }
 
 // per-warp column sums of one chunk -> staging; reduce_cs() then adds the four lane quarters in a fixed order
@@ -455,13 +483,9 @@ __device__ void epi_split(const ChainParams& p, EpiCtx& e, int task_i) {
         }
       }
     }
-    if (part == 0) {  // layer 1 can start
-      publish(e);
-      if (e.tid == 0) signal(p.ctr + 0);
-    }
+    if (part == 0) publish(e, p.ctr + 0);  // layer 1 can start
   }
-  publish(e);
-  if (e.tid == 0) signal(p.ctr + 2);
+  publish(e, p.ctr + 2);
 }
 
 __device__ __forceinline__ int warp_valid_rows(const EpiCtx& e, int valid) { return max(0, min(32, valid - e.q * 32)); }
@@ -471,7 +495,7 @@ __device__ void epi_f1(const ChainParams& p, EpiCtx& e, int task_i) {
   const int n0 = (task_i % p.NC) * BN;
   mbar_wait(&e.acc_full[e.ab], e.aph);
   tc_fence_after();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   const int row = e.q * 32 + e.lane;
   const bool ok = row < rt.valid;
   const int vr = warp_valid_rows(e, rt.valid);
@@ -497,17 +521,21 @@ __device__ void epi_f1(const ChainParams& p, EpiCtx& e, int task_i) {
   tc_fence_before();
   mbar_arrive(&e.acc_empty[e.ab]);
   acc_advance(e, 1);
-  publish(e);
-  if (e.tid == 0) signal(h_ready(p) + rt.seg * p.RTB + rt.r);
+  publish(e, h_ready(p) + rt.seg * p.RTB + rt.r);
 }
 
-// Layer 2 and the loss.  Task ((r, c), seg) owns the 128 x 64 tile of y for ONE row group (q | p | n) of 128 triplets:
+// Layer 2 and the loss.  Task ((r, c), seg) owns the 128 x 64 tile of y for ONE row group (q | p | n) of 128 triplets;
+// the three tasks of (r, c) run on three CTAs at the same time.
 //   1. y = acc + b2 goes to an exchange buffer (layout [column][row]: every access of a warp is one 128 B line) and
-//      the accumulator is released; the three tasks of (r, c) run on three CTAs at the same time and wait for each other;
-//   2. every task reads all three tiles and forms the partial |q|^2, |p|^2, |n|^2, q.p, q.n of its columns; the seg 0
-//      task publishes them; all tasks of row tile r wait until the partials of every column tile have arrived;
-//   3. cosines, hinge, and the closed-form dY of the task's OWN row group -> (hi, lo) terms row-major and transposed,
-//      db2 partial sums.
+//      the accumulator is released.
+//   2. Partial sums of the tile's columns, one slot [5][128] per column tile: the p and n tasks form |p|^2 / |n|^2
+//      from their own y and hand off y and the partial in one release, without waiting for anyone; the q task waits
+//      for the p and n tiles, loads them and forms |q|^2, q.p and q.n.
+//   3. Every task waits once, until all 3 x NCF tasks of row tile r have handed off (the p and n tasks load the
+//      sibling tiles then, together with the partial sums), then forms the cosines, hinge and the closed-form dY of
+//      its OWN row group -> (hi, lo) terms, db2 partial sums.
+// Each partial is one fmaf chain over a thread's 32 columns, the two column halves are added (half 0 + half 1), then
+// the slots in column-tile order: the sums do not depend on which task forms which partial.
 __device__ void epi_f2l(const ChainParams& p, EpiCtx& e, int task_i) {
   const int seg = task_i % 3, rc = task_i / 3, r = rc / p.NCF, c = rc % p.NCF, n0 = c * 64;
   const int valid = min(BM, p.B - r * BM);
@@ -518,7 +546,7 @@ __device__ void epi_f2l(const ChainParams& p, EpiCtx& e, int task_i) {
   const size_t wrow0 = (size_t)seg * p.B + (size_t)r * BM + e.q * 32;  // this warp's first row in the [3B, P] arrays
   mbar_wait(&e.acc_full[e.ab], e.aph);
   tc_fence_after();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   const uint32_t accb = e.tmem_base + ((uint32_t)(e.q * 32) << 16) + (uint32_t)(e.ab * BN + e.hf * 32);
   const float* bias = p.b2[seg != 0];
   float* X = p.ybuf + (size_t)rc * 3 * 64 * 128;  // [seg][64 columns][128 rows]
@@ -539,74 +567,77 @@ __device__ void epi_f2l(const ChainParams& p, EpiCtx& e, int task_i) {
   tc_fence_before();
   mbar_arrive(&e.acc_empty[e.ab]);  // the accumulator is free: the next main loop may overwrite it
   acc_advance(e, 1);
-  __threadfence();
-  epi_bar();
-  if (e.tid == 0) {
-    signal(y_ready(p) + rc);
-    wait_counter(y_ready(p) + rc, 3u);
-  }
-  epi_bar();
-  // ---- the other two row groups' values of the same (triplet, column)s: all 64 loads in flight at once -----------------
+  trace_ev(e, EV_Y_OUT);
+  // the other two row groups' tiles of the same (triplet, column)s
   const int s1 = seg == 0 ? 1 : 0, s2 = seg == 2 ? 1 : 2;  // the two foreign groups, ascending
+  const float* x1 = X + (size_t)(s1 * 64 + e.hf * 32) * 128 + row;
+  const float* x2 = X + (size_t)(s2 * 64 + e.hf * 32) * 128 + row;
   float f1[32], f2[32];
-  {
-    const float* x1 = X + (size_t)(s1 * 64 + e.hf * 32) * 128 + row;
-    const float* x2 = X + (size_t)(s2 * 64 + e.hf * 32) * 128 + row;
+  const int nslots = p.NCF;
+  float* sp = p.stat_part + ((size_t)(r * nslots + c) * 5) * 128 + row;  // this column tile's slot
+  float* xs = e.cs_s;  // [5][128]: the column halves meet here (the column-sum staging is idle until the dY stores)
+  if (seg == 0) {
+    if (e.tid == 0) wait_counter(y_ready(p) + rc, 2u);
+    epi_bar();
+    trace_ev(e, EV_Y_IN);
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {  // all 64 loads in flight at once
+      f1[j] = __ldcg(x1 + (size_t)j * 128);
+      f2[j] = __ldcg(x2 + (size_t)j * 128);
+    }
+    float qq = 0.f, qp = 0.f, qn = 0.f;
 #pragma unroll
     for (int j = 0; j < 32; ++j) {
+      qq = fmaf(own[j], own[j], qq);
+      qp = fmaf(own[j], f1[j], qp);
+      qn = fmaf(own[j], f2[j], qn);
+    }
+    if (e.hf == 1) {
+      xs[row] = qq; xs[384 + row] = qp; xs[512 + row] = qn;
+    }
+    epi_bar();
+    if (e.hf == 0) {
+      sp[0] = qq + xs[row]; sp[384] = qp + xs[384 + row]; sp[512] = qn + xs[512 + row];
+    }
+    trace_ev(e, EV_PART_OUT);
+    publish(e, stat_ready(p) + r);  // (also hands the q tile to the p and n tasks)
+  } else {
+    float ss = 0.f;  // |p|^2 or |n|^2
+#pragma unroll
+    for (int j = 0; j < 32; ++j) ss = fmaf(own[j], own[j], ss);
+    if (e.hf == 1) xs[seg * 128 + row] = ss;
+    epi_bar();
+    if (e.hf == 0) sp[seg * 128] = ss + xs[seg * 128 + row];
+    trace_ev(e, EV_PART_OUT);
+    publish(e, y_ready(p) + rc, stat_ready(p) + r);
+  }
+  if (e.tid == 0) wait_counter(stat_ready(p) + r, 3u * (unsigned)nslots);
+  epi_bar();
+  trace_ev(e, EV_STATS_IN);
+  if (seg != 0) {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {  // in flight together with the partial sums below
       f1[j] = __ldcg(x1 + (size_t)j * 128);
       f2[j] = __ldcg(x2 + (size_t)j * 128);
     }
   }
-  // q, p, n views of (own, f1, f2): seg 0 -> (own, f1, f2), seg 1 -> (f1, own, f2), seg 2 -> (f1, f2, own)
-  float qq = 0.f, pp = 0.f, nn = 0.f, qp = 0.f, qn = 0.f;
-#pragma unroll
-  for (int j = 0; j < 32; ++j) {
-    const float a = seg == 0 ? own[j] : f1[j];
-    const float b = seg == 0 ? f1[j] : (seg == 1 ? own[j] : f2[j]);
-    const float d = seg == 2 ? own[j] : f2[j];
-    qq = fmaf(a, a, qq);
-    pp = fmaf(b, b, pp);
-    nn = fmaf(d, d, nn);
-    qp = fmaf(a, b, qp);
-    qn = fmaf(a, d, qn);
-  }
-  // one slot of partial sums per column tile: the two column halves of the tile meet in shared memory first
-  const int nslots = p.NCF;
-  float* xs = e.cs_s;  // [5][128] (the column-sum staging is idle until the stores below)
-  if (seg == 0 && e.hf == 1) {
-    xs[row] = qq; xs[128 + row] = pp; xs[256 + row] = nn; xs[384 + row] = qp; xs[512 + row] = qn;
-  }
-  epi_bar();
-  if (seg == 0 && e.hf == 0) {
-    float* sp = p.stat_part + ((size_t)(r * nslots + c) * 5) * 128 + row;
-    sp[0] = qq + xs[row]; sp[128] = pp + xs[128 + row]; sp[256] = nn + xs[256 + row]; sp[384] = qp + xs[384 + row];
-    sp[512] = qn + xs[512 + row];
-    __threadfence();
-  }
-  epi_bar();
-  if (e.tid == 0) {
-    if (seg == 0) signal(stat_ready(p) + r);
-    wait_counter(stat_ready(p) + r, (unsigned)p.NCF);
-  }
-  epi_bar();
-  trace_ev(e, 3);
   // ---- the whole row's sums, slot order fixed (identical in every task of this row tile) ------------------------
-  qq = pp = nn = qp = qn = 0.f;
-  for (int s0 = 0; s0 < nslots; s0 += 4) {  // four slots (20 loads) in flight; the additions keep slot order
-    float v[4][5];
+  float qq = 0.f, pp = 0.f, nn = 0.f, qp = 0.f, qn = 0.f;
+  for (int s0 = 0; s0 < nslots; s0 += 8) {  // eight slots (40 loads) in flight; the additions keep slot order
+    float v[8][5];
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const float* sp = p.stat_part + ((size_t)(r * nslots + min(s0 + u, nslots - 1)) * 5) * 128 + row;
+    for (int u = 0; u < 8; ++u) {
+      const float* spu = p.stat_part + ((size_t)(r * nslots + min(s0 + u, nslots - 1)) * 5) * 128 + row;
 #pragma unroll
-      for (int w = 0; w < 5; ++w) v[u][w] = __ldcg(sp + 128 * w);
+      for (int w = 0; w < 5; ++w) v[u][w] = __ldcg(spu + 128 * w);
     }
 #pragma unroll
-    for (int u = 0; u < 4; ++u)
+    for (int u = 0; u < 8; ++u)
       if (s0 + u < nslots) {
         qq += v[u][0]; pp += v[u][1]; nn += v[u][2]; qp += v[u][3]; qn += v[u][4];
       }
   }
+  trace_ev(e, EV_STATS_LOADED, qq + pp + nn + qp + qn);
   const float nq = sqrtf(qq), np_ = sqrtf(pp), nn_ = sqrtf(nn);
   const float cq = fmaxf(nq, kCosEps), cp = fmaxf(np_, kCosEps), cn = fmaxf(nn_, kCosEps);
   const float cos_p = qp / (cq * cp), cos_n = qn / (cq * cn);
@@ -654,11 +685,8 @@ __device__ void epi_f2l(const ChainParams& p, EpiCtx& e, int task_i) {
   epi_bar();
   if (e.tid < 64) p.cs2[(size_t)(seg * p.RTB + r) * p.P + n0 + e.tid] = reduce_cs(e, 0, e.tid, 32);  // db2 partials
   if (seg == 0 && c == 0 && e.tid == 0) p.hinge_part[r] = (e.hs_s[0] + e.hs_s[1]) + (e.hs_s[2] + e.hs_s[3]);
-  publish(e);
-  if (e.tid == 0) {
-    signal(dy_ready(p) + seg * p.RTB + r);
-    signal(p.ctr + 1);
-  }
+  trace_ev(e, EV_STORED);
+  publish(e, dy_ready(p) + seg * p.RTB + r, p.ctr + 1);
 }
 
 __device__ void epi_dz(const ChainParams& p, EpiCtx& e, int task_i) {
@@ -666,29 +694,35 @@ __device__ void epi_dz(const ChainParams& p, EpiCtx& e, int task_i) {
   const int n0 = (task_i % p.NC) * BN;
   mbar_wait(&e.acc_full[e.ab], e.aph);
   tc_fence_after();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   const int row = e.q * 32 + e.lane;
   const bool ok = row < rt.valid;
   const int vr = warp_valid_rows(e, rt.valid);
   const size_t wrow0 = (size_t)rt.grow + e.q * 32;
+  // ReLU gate from the hi term of h: bf16 rounding keeps the sign and never turns a normal positive value into 0.
+  // The gate loads of all four chunks are issued at once, ahead of the chunk loop, and kept as one bit per column.
+  uint64_t live = 0;  // bit 16 ch + j: h > 0 at column n0 + 64 hf + 16 ch + j
+  if (ok && n0 + e.hf * 64 < p.P) {  // (P is a multiple of 64: a warp's 64 columns are all inside or all outside)
+    const uint4* hp = reinterpret_cast<const uint4*>(p.h_hi + (wrow0 + e.lane) * p.P + n0 + e.hf * 64);
+    uint4 raw[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) raw[i] = __ldcg(hp + i);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const bf16* g = reinterpret_cast<const bf16*>(&raw[i]);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) live |= (uint64_t)(__bfloat162float(g[j]) > 0.f) << (8 * i + j);
+    }
+  }
   for (int ch = 0; ch < 4; ++ch) {
     const int n = n0 + e.hf * 64 + ch * 16;
     if (n >= p.P) break;
     float v[16];
     tmem_ld16(acc_addr(e, e.ab, ch), v);
-    const size_t o = (wrow0 + e.lane) * p.P + n;
-    if (ok) {
-      // ReLU gate from the hi term of h: bf16 rounding keeps the sign and never turns a normal positive value into 0
-      alignas(16) bf16 g[16];
-      reinterpret_cast<uint4*>(g)[0] = __ldcg(reinterpret_cast<const uint4*>(p.h_hi + o));
-      reinterpret_cast<uint4*>(g)[1] = __ldcg(reinterpret_cast<const uint4*>(p.h_hi + o) + 1);
+    const uint32_t m = (uint32_t)(live >> (16 * ch));
 #pragma unroll
-      for (int j = 0; j < 16; ++j) v[j] = __bfloat162float(g[j]) > 0.f ? v[j] : 0.f;
-      if (p.dz1) store16(p.dz1 + o, v);
-    } else {
-#pragma unroll
-      for (int j = 0; j < 16; ++j) v[j] = 0.f;
-    }
+    for (int j = 0; j < 16; ++j) v[j] = (m >> j) & 1u ? v[j] : 0.f;  // (0 for rows past the batch)
+    if (ok && p.dz1) store16(p.dz1 + (wrow0 + e.lane) * p.P + n, v);
     alignas(16) bf16 hi[16], lo[16];
     split16(v, hi, lo);
     stage16(e.rs, e.lane, hi);  // (rows past the batch are zero: the weight-gradient contraction reads whole k-blocks)
@@ -705,11 +739,8 @@ __device__ void epi_dz(const ChainParams& p, EpiCtx& e, int task_i) {
   epi_bar();
   if (e.tid < BN && n0 + e.tid < p.P)
     p.cs1[(size_t)(rt.seg * p.RTB + rt.r) * p.P + n0 + e.tid] = reduce_cs(e, 0, e.tid);
-  publish(e);
-  if (e.tid == 0) {
-    signal(dz_ready(p) + rt.seg * p.RTB + rt.r);
-    signal(p.ctr + 1);
-  }
+  trace_ev(e, EV_STORED);
+  publish(e, dz_ready(p) + rt.seg * p.RTB + rt.r, p.ctr + 1);
 }
 
 // fp32 tile of this warp (32 rows x 64 columns) -> g, through the staging block, 16 columns at a time
@@ -732,7 +763,7 @@ __device__ void epi_dx(const ChainParams& p, EpiCtx& e, int task_i) {
   const int n0 = (task_i % p.NCH) * BN;
   mbar_wait(&e.acc_full[e.ab], e.aph);
   tc_fence_after();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   epi_store_f32(p, e, p.dxhat, (size_t)rt.grow + e.q * 32, n0, p.H, p.H, warp_valid_rows(e, rt.valid));
   tc_fence_before();
   mbar_arrive(&e.acc_empty[e.ab]);
@@ -748,17 +779,13 @@ __device__ void epi_dw(const ChainParams& p, EpiCtx& e, Task tk) {
   float* part = (two ? p.part2 : p.part1) + (size_t)ci * p.P * N;
   mbar_wait(&e.acc_full[e.ab], e.aph);
   tc_fence_after();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   epi_store_f32(p, e, part, (size_t)m0 + e.q * 32, n0, N, N, warp_valid_rows(e, p.P - m0));
   tc_fence_before();
   mbar_arrive(&e.acc_empty[e.ab]);
   acc_advance(e, 1);
-  __threadfence();
-  epi_bar();
-  if (e.tid == 0) {
-    if (two) signal(p.ctr + 5);  // the second-layer gradient's partial tiles: the tail sums them without waiting for dW1
-    signal(p.ctr + 1);
-  }
+  // counter 5 counts the second-layer gradient's partial tiles: the tail sums them without waiting for dW1
+  publish(e, p.ctr + 1, two ? p.ctr + 5 : nullptr);
 }
 
 __device__ __forceinline__ float4 add4(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
@@ -810,7 +837,7 @@ __device__ void epi_grad(const ChainParams& p, EpiCtx& e, int task_i) {
   // on dW1 (W2's fp32 values were last read by S, so its Adam update is safe already)
   if (e.tid == 0) wait_counter(p.ctr + 5, p.dw2_signals);
   epi_bar();
-  trace_ev(e, 2);
+  trace_ev(e, EV_ACC);
   AdamCoef k{0.f, 1.f};
   if (p.adam_p) {
     const volatile double* st = p.adam_state;
@@ -820,7 +847,7 @@ __device__ void epi_grad(const ChainParams& p, EpiCtx& e, int task_i) {
   const int nG = p.off[T_COUNT] - p.off[T_G];
   // A weight gradient pair (both towers) is a list of float4 items cut into chunks of 512 that the CTAs CLAIM (one
   // atomic per chunk): a CTA that arrives early takes more of them, the CTA that finishes the last contraction task
-  // finds little left.  A thread keeps two items and, per item, four chunk loads in flight; the additions keep the
+  // finds little left.  A thread keeps two items and, per item, eight chunk loads in flight; the additions keep the
   // order of the batch-row chunks, so the sums do not depend on who computes them.
   volatile int* claim_s = reinterpret_cast<volatile int*>(e.cs_s);  // (the column-sum staging is idle in this phase)
   int round = 0;
@@ -850,61 +877,60 @@ __device__ void epi_grad(const ChainParams& p, EpiCtx& e, int task_i) {
       locate(two ? it + kEpiThreads : it, src[1], dst[1], nch[1]);
       float4 acc[2] = {make_float4(0.f, 0.f, 0.f, 0.f), make_float4(0.f, 0.f, 0.f, 0.f)};
       const int nmax = max(nch[0], nch[1]);
-      for (int j = 0; j < nmax; j += 4) {
-        float4 t[2][4];
+      for (int j = 0; j < nmax; j += 8) {
+        float4 t[2][8];
 #pragma unroll
         for (int u = 0; u < 2; ++u)
 #pragma unroll
-          for (int c4 = 0; c4 < 4; ++c4)
-            t[u][c4] = (j + c4 < nch[u]) ? __ldcg(src[u] + (size_t)(j + c4) * n4) : make_float4(0.f, 0.f, 0.f, 0.f);
+          for (int c8 = 0; c8 < 8; ++c8)
+            t[u][c8] = (j + c8 < nch[u]) ? __ldcg(src[u] + (size_t)(j + c8) * n4) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
         for (int u = 0; u < 2; ++u)
 #pragma unroll
-          for (int c4 = 0; c4 < 4; ++c4)
-            if (j + c4 < nch[u]) acc[u] = add4(acc[u], t[u][c4]);
+          for (int c8 = 0; c8 < 8; ++c8)
+            if (j + c8 < nch[u]) acc[u] = add4(acc[u], t[u][c8]);
       }
       emit4(p, k, dst[0], acc[0]);
       if (two) emit4(p, k, dst[1], acc[1]);
     }
   };
-  sum_pairs(p.ctr + 6, p.part2, p.dW2, (size_t)p.P * p.P / 4);
-  // phase B: everything else has signalled
-  if (e.tid == 0) wait_counter(p.ctr + 1, p.total_signals);
-  epi_bar();
-  sum_pairs(p.ctr + 7, p.part1, p.dW1, (size_t)p.P * p.H / 4);
   // bias gradients: one output per warp at a time, the lanes take the row-tile partials (lane-strided, then a fixed
-  // xor tree), so every CTA shares this tail instead of the first few
-  {
-    const int nout = 4 * p.P;  // db2[0] | db2[1] | db1[0] | db1[1]
-    const int gw = task_i * 8 + e.we, nw = nG * 8;
-    for (int o = gw; o < nout; o += nw) {
-      const int which = o / p.P, n = o - which * p.P, t = which & 1;
-      const float* src;
-      int cnt;
-      if (which < 2) {
-        src = p.cs2 + (size_t)(t ? p.RTB : 0) * p.P + n;
-        cnt = t ? 2 * p.RTB : p.RTB;
-      } else {
-        src = p.cs1 + (size_t)(t ? p.RTB : 0) * p.P + n;
-        cnt = t ? 2 * p.RTB : p.RTB;
-      }
+  // xor tree), so every CTA shares them instead of the first few
+  const int gw = task_i * 8 + e.we, nw = nG * 8;
+  auto bias_grads = [&](const float* cs, float* const (&db)[2]) {
+    for (int o = gw; o < 2 * p.P; o += nw) {
+      const int t = o / p.P, n = o - t * p.P;
+      const float* src = cs + (size_t)(t ? p.RTB : 0) * p.P + n;
+      const int cnt = t ? 2 * p.RTB : p.RTB;
       float s = 0.f;
       for (int r = e.lane; r < cnt; r += 32) s += __ldcg(src + (size_t)r * p.P);
       s = warp_sum(s);
-      if (e.lane == 0) emit1(p, k, (which < 2 ? p.db2[t] : p.db1[t]) + n, s);
+      if (e.lane == 0) emit1(p, k, db[t] + n, s);
     }
-  }
+  };
+  sum_pairs(p.ctr + 6, p.part2, p.dW2, (size_t)p.P * p.P / 4);
+  // db2 and the loss only need the layer-2 / loss tasks, which every dW2 partial tile waited for (b2 was last read
+  // there, so its Adam update is safe here too)
+  bias_grads(p.cs2, p.db2);
   if (task_i == 0 && e.tid == 0) {
     float s = 0.f;
     for (int r = 0; r < p.RTB; ++r) s += __ldcg(p.hinge_part + r);
     *p.loss = s * p.inv_batch;
   }
+  // phase B: everything else has signalled
+  if (e.tid == 0) wait_counter(p.ctr + 1, p.total_signals);
+  epi_bar();
+  trace_ev(e, EV_ALL_IN);
+  sum_pairs(p.ctr + 7, p.part1, p.dW1, (size_t)p.P * p.H / 4);
+  bias_grads(p.cs1, p.db1);
+  trace_ev(e, EV_STORED);
   // The last tail task to finish clears the dependency counters for the next launch (every other task of this
   // launch has completed by then: the tail waited for all of them), so a graph replay needs no memset node.
   epi_bar();
   if (e.tid == 0) {
-    __threadfence();
-    if (atomicAdd(p.ctr + 4, 1u) == (unsigned)nG - 1u) {
+    unsigned prev;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(prev) : "l"(p.ctr + 4) : "memory");
+    if (prev == (unsigned)nG - 1u) {
       for (int i = 0; i < p.n_counters; ++i) p.ctr[i] = 0u;
     }
   }
@@ -1056,7 +1082,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
     for (int idx = blockIdx.x; idx < n_tasks; idx += gridDim.x) {
       const Task tk = decode(p, idx);
       e.tidx = idx;
-      trace_ev(e, 0);
+      trace_ev(e, EV_START);
       switch (tk.type) {
         case T_S:
           epi_split(p, e, tk.i);
@@ -1070,7 +1096,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const __grid_constan
         case T_DW1: epi_dw(p, e, tk); break;
         default: epi_grad(p, e, tk.i); break;
       }
-      trace_ev(e, 1);
+      trace_ev(e, EV_END);
     }
   }
   tc_fence_before();
@@ -1224,8 +1250,9 @@ int chain_sm100(const StepSm100& s, bool after_gather, cudaStream_t st) {
   }
   {
     const char* e = getenv("TT_CHAIN_TRACE");
+    // the caller zeroes the trace buffer before the launch it wants (a memset here would sit between the pooled
+    // gather and its programmatic dependent, and take the overlap out of the step being traced)
     p.trace = (e && atoi(e) != 0 && grid <= kTraceCtas) ? w.trace : nullptr;
-    if (p.trace) TT_CUDA(cudaMemsetAsync(w.trace, 0, (size_t)kTraceCtas * kTraceSlots * 16, st));
   }
   // (no memset of the counters: the workspace is zero-filled once by its owner and every launch leaves them at zero)
   p.use_pdl = after_gather ? 1 : 0;

@@ -23,9 +23,9 @@ struct StepWs {
   float *stat_part, *cs1, *cs2, *hinge_part, *ybuf;
   unsigned* counters;
   int n_counters;
-  unsigned long long* trace;  // TT_CHAIN_TRACE=1: [CTA][kTraceSlots] x {task index << 1 | end, globaltimer ns}
+  unsigned long long* trace;  // TT_CHAIN_TRACE=1: [CTA][kTraceSlots] x {task index << 4 | event, globaltimer ns}
 };
-constexpr int kTraceSlots = 64, kTraceCtas = 160;
+constexpr int kTraceSlots = 128, kTraceCtas = 160;
 
 static inline size_t carve_step(char* base, int B, int H, int P, int train_table, StepWs* out) {
   char* p = base;

@@ -289,9 +289,9 @@ class FusedTrainer:
         # TWO step workspaces: the pooled gather of step i+1 (tokens + frozen tables only, never the projection
         # weights) runs beside everything else of step i, so consecutive steps alternate between them
         # How the projection chain is launched (tt_step_args.chain).  Default: the persistent chain kernel — everything
-        # after the pooled gather in ONE launch (123 us alone at configs[1] against 157 us for one kernel per
+        # after the pooled gather in ONE launch (115 us alone at configs[1] against 157-162 us for one kernel per
         # contraction).  It wants every SM, so nothing runs beside it: on one GPU a step is gather -> chain in one stream
-        # (2 launches, the second a programmatic dependent of the first; 0.239 ms), under data parallelism the NEXT
+        # (2 launches, the second a programmatic dependent of the first; 0.230-0.233 ms), under data parallelism the NEXT
         # step's gather runs beside the exchange kernel, which mostly waits (N = 2: 0.272 ms).  The per-kernel chain
         # (TT_CHAIN=0) lets the look-ahead gather's CTAs slip between its small kernels instead; since the chain kernel
         # lost its transposed copies that schedule is the slower one (0.242-0.248 ms; N = 2: 0.275 ms).  A trainable table
