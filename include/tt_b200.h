@@ -208,6 +208,18 @@ typedef struct tt_step_args {
    * window that carries nothing uses 0; set grad_scale = 1/a for the reference's scaling).  Appended, like the
    * pooled_* fields, while TT_B200_VERSION stayed at 100: rebuild callers against this header.                    */
   int grad_accumulate;
+  /* optional optimiser of the token tables (NULL = the table gradients are only computed, as above): when
+   * table_param_q / table_param_d are set and the call has TT_STEP_BACK, the table gradient of this call (plus the old
+   * dtable_* when grad_accumulate = 1) is consumed by one dense torch.optim.Adam step on EVERY row of both tables, run
+   * in the scatter-add's epilogue; dtable_q / dtable_d are then not written (still give them: they select the trainable
+   * table and hold a window's partial sum).  An untouched row has gradient 0: its moments decay, and it still moves once
+   * its exp_avg is non-zero.  The tables share the projections' step count and hyper-parameters (adam_state is
+   * advanced by this call before the table update reads it, adam_lr / adam_beta1 / adam_beta2 / adam_eps), so these
+   * fields need adam_param.  table_param_q / table_param_d must be table_q / table_d (distinct fp32 tables);
+   * table_exp_avg* are fp32 [vocab, H].  Appended, like grad_accumulate, while TT_B200_VERSION stayed at 100: rebuild
+   * callers against this header.                                                                                   */
+  float *table_param_q, *table_param_d;
+  float *table_exp_avg_q, *table_exp_avg_sq_q, *table_exp_avg_d, *table_exp_avg_sq_d;
 } tt_step_args;
 #define TT_STEP_FRONT 1
 #define TT_STEP_BACK 2

@@ -75,6 +75,9 @@ class StepArgs(ctypes.Structure):
         ("pooled_d", c_void_p), ("pooled_d_rows", c_int64),
         ("pooled_index", c_void_p),
         ("grad_accumulate", c_int),
+        ("table_param_q", c_void_p), ("table_param_d", c_void_p),
+        ("table_exp_avg_q", c_void_p), ("table_exp_avg_sq_q", c_void_p),
+        ("table_exp_avg_d", c_void_p), ("table_exp_avg_sq_d", c_void_p),
     ]
 
 

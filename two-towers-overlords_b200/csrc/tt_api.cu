@@ -67,15 +67,13 @@ __global__ void adam_dev_kernel(float* __restrict__ p, const float* __restrict__
                                 const double* __restrict__ state, float grad_scale) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const float step_size = (float)((double)lr / (1.0 - state[1]));
-  const float bc2_sqrt = (float)sqrt(1.0 - state[2]);
-  const float gi = g[i] * grad_scale;
-  const float mi = m[i] + (gi - m[i]) * (1.f - beta1);
-  const float vi = v[i] * beta2 + (1.f - beta2) * gi * gi;
+  const float step_size = adam_step_size(state, lr);
+  const float bc2_sqrt = adam_bc2_sqrt(state);
+  float pi = p[i], mi = m[i], vi = v[i];
+  adam_element(pi, mi, vi, g[i] * grad_scale, beta1, beta2, eps, step_size, bc2_sqrt);
   m[i] = mi;
   v[i] = vi;
-  const float denom = sqrtf(vi) / bc2_sqrt + eps;
-  p[i] = p[i] - step_size * (mi / denom);
+  p[i] = pi;
 }
 
 }  // namespace
@@ -248,6 +246,19 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
   TT_REQUIRE(a->grad_accumulate == 0 || a->grad_accumulate == 1, "tt_triplet_step: grad_accumulate must be 0 or 1, got %d",
              a->grad_accumulate);
   const int acc = a->grad_accumulate;
+  const bool table_adam = a->table_param_q != nullptr || a->table_param_d != nullptr;
+  if (table_adam) {
+    TT_REQUIRE(a->table_param_q && a->table_param_d, "tt_triplet_step: give both table_param_q and table_param_d or "
+               "neither");
+    TT_REQUIRE(train_table, "tt_triplet_step: the table optimiser needs the table gradients (dtable_q / dtable_d)");
+    TT_REQUIRE(a->table_dtype == TT_F32, "tt_triplet_step: the table optimiser needs fp32 tables");
+    TT_REQUIRE(a->table_param_q == a->table_q && a->table_param_d == a->table_d && a->table_q != a->table_d,
+               "tt_triplet_step: table_param_q / table_param_d must be the two distinct tables the step gathers from");
+    TT_REQUIRE(a->adam_param != nullptr, "tt_triplet_step: the table optimiser shares the projections' step count: it "
+               "needs adam_param");
+    TT_REQUIRE(a->adam_state && a->table_exp_avg_q && a->table_exp_avg_sq_q && a->table_exp_avg_d &&
+               a->table_exp_avg_sq_d, "tt_triplet_step: the table optimiser needs adam_state and all four table moments");
+  }
   const size_t need = tt_step_ws_bytes(B, a->Lq, a->Ld, H, P, a->vocab, a->precision, train_table);
   TT_REQUIRE(a->ws && a->ws_bytes >= need, "tt_triplet_step: workspace too small (%zu < %zu)", a->ws_bytes, need);
   cudaStream_t st = as_stream(stream);
@@ -349,16 +360,21 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
                                a->adam_beta1, a->adam_beta2, a->adam_eps, a->adam_state, 1.f, stream)))
       return rc;
   }
-  // 6. table gradients (D2 extension)
+  // 6. table gradients (D2 extension), or with table_param_* the tables' Adam step in the scatter-add's epilogue.  Every
+  // path above has advanced adam_state for this step in stream order, so the tables use the projections' step count
   if (train_table) {
     if ((rc = pool_bwd_prep(w.dxhat, w.xhat, w.cnt, w.nrm, 3 * B, H, w.g, st))) return rc;
+    const TableAdam tq{a->table_param_q, a->table_exp_avg_q, a->table_exp_avg_sq_q, a->adam_lr, a->adam_beta1,
+                       a->adam_beta2, a->adam_eps, a->adam_state};
+    const TableAdam td{a->table_param_d, a->table_exp_avg_d, a->table_exp_avg_sq_d, a->adam_lr, a->adam_beta1,
+                       a->adam_beta2, a->adam_eps, a->adam_state};
     PoolBwdSeg sq{a->q_ids, a->q_mask, B, a->Lq, 0};
     if ((rc = pool_bwd_scatter(&sq, 1, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_q, acc, w.pool_ws,
-                               w.pool_ws_bytes, st)))
+                               w.pool_ws_bytes, st, table_adam ? &tq : nullptr)))
       return rc;
     PoolBwdSeg sd[2] = {{a->p_ids, a->p_mask, B, a->Ld, B}, {a->n_ids, a->n_mask, B, a->Ld, 2 * B}};
     if ((rc = pool_bwd_scatter(sd, 2, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_d, acc, w.pool_ws,
-                               w.pool_ws_bytes, st)))
+                               w.pool_ws_bytes, st, table_adam ? &td : nullptr)))
       return rc;
   }
   return 0;

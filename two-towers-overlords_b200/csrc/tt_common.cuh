@@ -70,6 +70,25 @@ __device__ __forceinline__ long long load_index(const void* p, int dtype, size_t
   }
 }
 
+// torch.optim.Adam (single/multi-tensor, non-fused, no weight decay / amsgrad) on one element: lerp, mul + addcmul,
+// sqrt / bc2_sqrt + eps, addcdiv.  Every rounding is spelled out with _rn intrinsics, so no kernel's surroundings can
+// change which products the compiler contracts into FMAs: the kernels that call this helper agree bit for bit.  The
+// FMAs are the ones the compiler chose for the plain expressions m + (g - m)(1 - beta1), v beta2 + (1 - beta2) g g and
+// p - step_size (m / denom) in adam_dev_kernel before this helper existed, which the persistent chain kernel's Adam tail
+// and tt_dp_reduce_adam match.
+__device__ __forceinline__ void adam_element(float& p, float& m, float& v, float g, float beta1, float beta2, float eps,
+                                             float step_size, float bc2_sqrt) {
+  m = __fmaf_rn(__fsub_rn(g, m), __fsub_rn(1.f, beta1), m);
+  v = __fmaf_rn(v, beta2, __fmul_rn(__fmul_rn(__fsub_rn(1.f, beta2), g), g));
+  const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), bc2_sqrt), eps);
+  p = __fmaf_rn(-step_size, __fdiv_rn(m, denom), p);
+}
+// bias corrections of a device step count state {t, beta1^t, beta2^t, -} that was already advanced to this step
+__device__ __forceinline__ float adam_step_size(const double* state, float lr) {
+  return (float)((double)lr / (1.0 - state[1]));
+}
+__device__ __forceinline__ float adam_bc2_sqrt(const double* state) { return (float)sqrt(1.0 - state[2]); }
+
 // fp32 -> (hi, lo) bf16 pair with hi + lo == x to ~2^-17 relative
 __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {
   hi = __float2bfloat16_rn(x);

@@ -46,12 +46,21 @@ struct PoolBwdSeg {
   const void* mask;
   int B, L, row0;
 };
+// Adam on the table in the scatter-add's epilogue: p / m / v [vocab,H] fp32; state {t, beta1^t, beta2^t, -} already
+// advanced to this step (the projections' optimiser step)
+struct TableAdam {
+  float *p, *m, *v;
+  float lr, beta1, beta2, eps;
+  const double* state;
+};
 size_t pool_bwd_ws_bytes(long long n_tokens, int vocab);
 // g [rows,H]: per-sequence gradient of the masked SUM's mean, i.e. d(loss)/d(pooled mean)/cnt;
 // dtable[id] (+)= sum over tokens with that id of mask_t * g[seq(t)], reduced in position order.
+// adam != nullptr: that sum (plus the old dtable row when accumulate) is the gradient of one dense Adam step on every
+// row of the table instead, and dtable is not written.
 int pool_bwd_scatter(const PoolBwdSeg* segs, int nseg, int ids_dtype, int mask_dtype, const float* g,
                      int vocab, int H, float* dtable, int accumulate, void* ws, size_t ws_bytes,
-                     cudaStream_t st);
+                     cudaStream_t st, const TableAdam* adam = nullptr);
 // dxhat -> g: through F.normalize and the mean (rows [0,rows))
 int pool_bwd_prep(const float* dxhat, const float* xhat, const float* cnt, const float* nrm, int rows,
                   int H, float* g, cudaStream_t st);

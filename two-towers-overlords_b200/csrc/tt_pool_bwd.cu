@@ -9,6 +9,9 @@
 //   3. reduce:  one warp per table row sums mask_t * g[seq(t)] over its run in sorted order and writes
 //               the row once (zero rows for untouched ids).  Runs longer than kHeavy entries go to a
 //               second kernel that splits them over the 8 warps of a CTA in a fixed order.
+//               Adam variant (trainable tables with their optimiser in the step): the warp that formed a row's
+//               gradient takes the row's dense Adam step itself (read + write p, m, v: 24 B per element instead of
+//               the 4 B gradient write + 28 B of a separate dense Adam pass), and dtable is not written.
 // No float atomics anywhere; two runs give bit-identical tables.
 #include "tt_pool.cuh"
 
@@ -237,13 +240,37 @@ __device__ __forceinline__ void run_sum(const BwdSegs& S, const unsigned* __rest
 
 constexpr int kChunk = 2048;  // entries of a heavy row summed by one CTA
 
+// The finished gradient o of four consecutive elements of row `id`: written to dtable, or (ADAM) one Adam step on the
+// table's p / m / v with it.  o already holds the old dtable row when accumulating.
+template <bool ADAM>
+__device__ __forceinline__ void finish_row4(float4 o, int id, int H, int col4, float* __restrict__ dtable,
+                                            const TableAdam& ta, float step_size, float bc2_sqrt) {
+  const size_t off = (size_t)id * H + (size_t)col4 * 4;
+  if (!ADAM) {
+    *reinterpret_cast<float4*>(dtable + off) = o;
+    return;
+  }
+  float4 p = *reinterpret_cast<const float4*>(ta.p + off);
+  float4 m = *reinterpret_cast<const float4*>(ta.m + off);
+  float4 v = *reinterpret_cast<const float4*>(ta.v + off);
+  adam_element(p.x, m.x, v.x, o.x, ta.beta1, ta.beta2, ta.eps, step_size, bc2_sqrt);
+  adam_element(p.y, m.y, v.y, o.y, ta.beta1, ta.beta2, ta.eps, step_size, bc2_sqrt);
+  adam_element(p.z, m.z, v.z, o.z, ta.beta1, ta.beta2, ta.eps, step_size, bc2_sqrt);
+  adam_element(p.w, m.w, v.w, o.w, ta.beta1, ta.beta2, ta.eps, step_size, bc2_sqrt);
+  *reinterpret_cast<float4*>(ta.p + off) = p;
+  *reinterpret_cast<float4*>(ta.m + off) = m;
+  *reinterpret_cast<float4*>(ta.v + off) = v;
+}
+
 // heavy bookkeeping (ints): [0] number of heavy ids, [1] number of chunks, then per heavy id {id, first chunk, chunks},
 // then per chunk {id, index of the chunk inside its row}
-template <int NV>
+// ADAM: every light row, touched or not (g = 0 exactly), takes its Adam step here; heavy rows take theirs in
+// heavy_final_kernel, so each row of [0, vocab) is updated exactly once
+template <int NV, bool ADAM>
 __global__ void __launch_bounds__(256)
     seg_reduce_kernel(const BwdSegs S, const unsigned* __restrict__ vals, const int* __restrict__ id_off, int vocab,
                       const float* __restrict__ g, float* __restrict__ dtable, int accumulate, int* __restrict__ hv,
-                      int max_heavy) {
+                      int max_heavy, const TableAdam ta) {
   constexpr int H = NV * 128;
   const int id = blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
@@ -269,6 +296,8 @@ __global__ void __launch_bounds__(256)
   float acc[NV * 4];
 #pragma unroll
   for (int i = 0; i < NV * 4; ++i) acc[i] = 0.f;
+  const float step_size = ADAM ? adam_step_size(ta.state, ta.lr) : 0.f;
+  const float bc2_sqrt = ADAM ? adam_bc2_sqrt(ta.state) : 0.f;
   run_sum<NV>(S, vals, beg, end, g, lane, acc);
   float* out = dtable + (size_t)id * H;
 #pragma unroll
@@ -279,7 +308,7 @@ __global__ void __launch_bounds__(256)
       const float4 old = *dst;
       o.x += old.x; o.y += old.y; o.z += old.z; o.w += old.w;
     }
-    *dst = o;
+    finish_row4<ADAM>(o, id, H, k * 32 + lane, dtable, ta, step_size, bc2_sqrt);
   }
 }
 
@@ -319,14 +348,16 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-// stage 2: one warp per heavy row adds its chunk sums in chunk order
-template <int NV>
+// stage 2: one warp per heavy row adds its chunk sums in chunk order (ADAM: then takes the row's Adam step)
+template <int NV, bool ADAM>
 __global__ void __launch_bounds__(256)
     heavy_final_kernel(const int* __restrict__ hv, const float* __restrict__ partial, float* __restrict__ dtable,
-                       int accumulate) {
+                       int accumulate, const TableAdam ta) {
   constexpr int H = NV * 128;
   const int lane = threadIdx.x & 31;
   const int n_heavy = hv[0];
+  const float step_size = ADAM ? adam_step_size(ta.state, ta.lr) : 0.f;
+  const float bc2_sqrt = ADAM ? adam_bc2_sqrt(ta.state) : 0.f;
   for (int h = blockIdx.x * 8 + (threadIdx.x >> 5); h < n_heavy; h += gridDim.x * 8) {
     const int id = hv[2 + 3 * h], base = hv[2 + 3 * h + 1], nch = hv[2 + 3 * h + 2];
 #pragma unroll
@@ -336,12 +367,11 @@ __global__ void __launch_bounds__(256)
         const float4 t = *(reinterpret_cast<const float4*>(partial + (size_t)(base + c) * H) + k * 32 + lane);
         acc.x += t.x; acc.y += t.y; acc.z += t.z; acc.w += t.w;
       }
-      float4* dst = reinterpret_cast<float4*>(dtable + (size_t)id * H) + k * 32 + lane;
       if (accumulate) {
-        const float4 old = *dst;
+        const float4 old = *(reinterpret_cast<const float4*>(dtable + (size_t)id * H) + k * 32 + lane);
         acc.x += old.x; acc.y += old.y; acc.z += old.z; acc.w += old.w;
       }
-      *dst = acc;
+      finish_row4<ADAM>(acc, id, H, k * 32 + lane, dtable, ta, step_size, bc2_sqrt);
     }
   }
 }
@@ -378,7 +408,8 @@ int pool_bwd_prep(const float* dxhat, const float* xhat, const float* cnt, const
 }
 
 int pool_bwd_scatter(const PoolBwdSeg* segs, int nseg, int ids_dtype, int mask_dtype, const float* g, int vocab,
-                     int H, float* dtable, int accumulate, void* ws, size_t ws_bytes, cudaStream_t st) {
+                     int H, float* dtable, int accumulate, void* ws, size_t ws_bytes, cudaStream_t st,
+                     const TableAdam* adam) {
   TT_REQUIRE(nseg >= 1 && nseg <= 4, "tt_pool_bwd: nseg must be in [1,4]");
   TT_REQUIRE(H == 128 || H == 256 || H == 384 || H == 768, "tt_pool_bwd: hidden size %d not supported", H);
   BwdSegs S{};
@@ -431,19 +462,28 @@ int pool_bwd_scatter(const PoolBwdSeg* segs, int nseg, int ids_dtype, int mask_d
   TT_LAUNCH_CHECK();
   const int rblocks = (vocab + 7) / 8;
   const int hblocks = 4 * sm_count();
-#define TT_SEG_CASE(NV)                                                                                         \
-  seg_reduce_kernel<NV><<<rblocks, 256, 0, st>>>(S, valA, id_off, vocab, g, dtable, accumulate, hv, max_heavy);   \
-  TT_LAUNCH_CHECK();                                                                                            \
-  heavy_chunk_kernel<NV><<<hblocks, 256, 0, st>>>(S, valA, id_off, g, hv, max_heavy, partial);                    \
-  TT_LAUNCH_CHECK();                                                                                            \
-  heavy_final_kernel<NV><<<sm_count(), 256, 0, st>>>(hv, partial, dtable, accumulate);                            \
+  const TableAdam ta = adam ? *adam : TableAdam{};
+#define TT_SEG_CASE(NV, ADAM)                                                                                         \
+  seg_reduce_kernel<NV, ADAM><<<rblocks, 256, 0, st>>>(S, valA, id_off, vocab, g, dtable, accumulate, hv, max_heavy,  \
+                                                       ta);                                                          \
+  TT_LAUNCH_CHECK();                                                                                                  \
+  heavy_chunk_kernel<NV><<<hblocks, 256, 0, st>>>(S, valA, id_off, g, hv, max_heavy, partial);                          \
+  TT_LAUNCH_CHECK();                                                                                                  \
+  heavy_final_kernel<NV, ADAM><<<sm_count(), 256, 0, st>>>(hv, partial, dtable, accumulate, ta);                        \
   TT_LAUNCH_CHECK();
-  switch (H / 128) {
-    case 1: { TT_SEG_CASE(1) } break;
-    case 2: { TT_SEG_CASE(2) } break;
-    case 3: { TT_SEG_CASE(3) } break;
-    default: { TT_SEG_CASE(6) } break;
+#define TT_SEG_H(ADAM)                       \
+  switch (H / 128) {                         \
+    case 1: { TT_SEG_CASE(1, ADAM) } break;  \
+    case 2: { TT_SEG_CASE(2, ADAM) } break;  \
+    case 3: { TT_SEG_CASE(3, ADAM) } break;  \
+    default: { TT_SEG_CASE(6, ADAM) } break; \
   }
+  if (adam) {
+    TT_SEG_H(true)
+  } else {
+    TT_SEG_H(false)
+  }
+#undef TT_SEG_H
 #undef TT_SEG_CASE
   return 0;
 }

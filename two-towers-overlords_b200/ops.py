@@ -211,6 +211,7 @@ class TripletStep:
         self.slots = []
         self._keep = []
         self._adam = None
+        self._table_adam = None
         self.chain = 0
 
     def bind(self, tokens, tables, params, grads, margin, inv_batch, grad_scale=1.0, table_grads=None):
@@ -370,9 +371,22 @@ class TripletStep:
                       float(lr), float(betas[0]), float(betas[1]), float(eps))
         self._keep.append((state, param, grad, exp_avg, exp_avg_sq))
 
+    def bind_table_adam(self, params, exp_avgs, exp_avg_sqs):
+        """Optional optimiser of the trainable token tables (tt_step_args.table_*): params = (table_q, table_d) as bound
+        with bind() (fp32), exp_avgs / exp_avg_sqs = their fp32 moment pairs.  run(..., optimise=True) then takes one
+        dense Adam step on both tables in the table gradient's epilogue, with the projections' step count and
+        hyper-parameters (bind_adam)."""
+        assert self.train_table, "bind_table_adam needs a step built with train_table=True"
+        for t in tuple(params) + tuple(exp_avgs) + tuple(exp_avg_sqs):
+            assert t.dtype == torch.float32 and t.shape == params[0].shape
+        self._table_adam = (N.ptr(params[0]), N.ptr(params[1]), N.ptr(exp_avgs[0]), N.ptr(exp_avg_sqs[0]),
+                            N.ptr(exp_avgs[1]), N.ptr(exp_avg_sqs[1]))
+        self._keep.append((params, exp_avgs, exp_avg_sqs))
+
     def run(self, slot: int = 0, phases: int = 0, optimise: bool = False, accumulate: bool = False):
         """phases: 0 = whole step, 1 = pooled gather only (TT_STEP_FRONT), 2 = the rest (TT_STEP_BACK).
-        optimise: also apply the optimiser bound with bind_adam() (gradients only otherwise).
+        optimise: also apply the optimiser bound with bind_adam() (gradients only otherwise), and the tables' one bound
+        with bind_table_adam().
         accumulate: add this micro-batch's gradients to the gradient buffers (tt_step_args.grad_accumulate)."""
         a = self.slots[slot]
         a.phases = int(phases)
@@ -381,12 +395,18 @@ class TripletStep:
             assert self._adam is not None, "run(optimise=True) needs bind_adam() first"
             (a.adam_state, a.adam_param, a.adam_grad, a.adam_exp_avg, a.adam_exp_avg_sq, a.adam_n, a.adam_lr,
              a.adam_beta1, a.adam_beta2, a.adam_eps) = self._adam
+            if self._table_adam is not None:
+                (a.table_param_q, a.table_param_d, a.table_exp_avg_q, a.table_exp_avg_sq_q, a.table_exp_avg_d,
+                 a.table_exp_avg_sq_d) = self._table_adam
         else:
             a.adam_param = None
-        N.check(self.lib.tt_triplet_step(ctypes.byref(a), N.stream()), "tt_triplet_step")
-        a.phases = 0
-        a.adam_param = None
-        a.grad_accumulate = 0
+        try:
+            N.check(self.lib.tt_triplet_step(ctypes.byref(a), N.stream()), "tt_triplet_step")
+        finally:
+            a.phases = 0
+            a.adam_param = None
+            a.table_param_q = a.table_param_d = None
+            a.grad_accumulate = 0
         return self.loss
 
 

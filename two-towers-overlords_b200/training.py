@@ -168,13 +168,21 @@ class FusedTrainer:
     parallel, the one exchange) runs after micro-batch `batch_idx` of the epoch whenever (batch_idx + 1) % a == 0.
     `batch_idx` restarts at 0 with every epoch (train_epoch / train_epoch_device / start_epoch()); a trailing partial
     window is not stepped and its gradient carries into the next epoch's first window, as in the reference.  a = 1 is
-    the plain trainer."""
+    the plain trainer.
+
+    `optimize_tables=True` trains the token tables too (the model's tables must be trainable fp32,
+    TwoTowersModel(train_table=True)): torch.optim.Adam's dense step on every row of both tables with the projections'
+    step count, as `torch.optim.Adam(model.parameters())` applies it.  On one GPU it runs in the epilogue of the table
+    gradient's scatter-add inside the step call; data parallel (exchange="peer") the tables live in a second peer
+    segment and their flat gradient goes through the same fused reduce-scatter / Adam / all-gather kernel right after
+    the projections'.  Off (the default), a trainable-table model only gets its table gradients (`table_grads`)."""
 
     def __init__(self, model: TwoTowersModel, margin: float, lr: float, batch_size: int, Lq: int = 32, Ld: int = 256,
                  precision: Optional[str] = None, world_size: int = 1, rank: int = 0, use_graph: bool = True,
                  betas=(0.9, 0.999), eps: float = 1e-8, process_group=None, ids_dtype=torch.int32,
                  mask_dtype=torch.uint8, token_slots: int = 1, exchange: Optional[str] = None,
-                 exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None, accumulation_steps: int = 1):
+                 exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None, accumulation_steps: int = 1,
+                 optimize_tables: bool = False):
         qt, dt = model.query_tower, model.document_tower
         self.window = AccumulationWindow(accumulation_steps)
         self.accum = self.window.a
@@ -213,6 +221,17 @@ class FusedTrainer:
             self.train_table = False
         else:
             self.train_table = bool(qt.pretrained_model.table.requires_grad)
+        self.optimize_tables = bool(optimize_tables)
+        if self.optimize_tables:
+            if not self.train_table:
+                raise ValueError("FusedTrainer(optimize_tables=True) needs trainable token tables: build the model with "
+                                 "TwoTowersModel(train_table=True)")
+            if any(t.pretrained_model.table.dtype != torch.float32 for t in (qt, dt)):
+                raise ValueError("FusedTrainer(optimize_tables=True) needs fp32 token tables (bf16 tables do not train)")
+            if exchange == "nccl" or (world_size > 1 and not exchange
+                                      and os.environ.get("TT_DP_EXCHANGE", "peer") == "nccl"):
+                raise ValueError("FusedTrainer(optimize_tables=True) exchanges the tables with the peer exchange only; "
+                                 "exchange='nccl' is the projections-only baseline")
         params = model.projection_parameters()
         sizes = [p.numel() for p in params]
         self.n_param = sum(sizes)
@@ -237,6 +256,29 @@ class FusedTrainer:
         self.exp_avg = torch.zeros(self.n_param, dtype=torch.float32, device=dev)
         self.exp_avg_sq = torch.zeros(self.n_param, dtype=torch.float32, device=dev)
         self.adam_state = torch.zeros(4, dtype=torch.float64, device=dev)
+        # the tables' optimiser state: flat [2VH] moments (query table | document table); data parallel, a second
+        # exchange whose peer segment holds both tables and a flat [2VH + 1] gradient in the same layout
+        self.txchg = None
+        self.table_grads = None
+        self.table_exp_avg = self.table_exp_avg_sq = None
+        if self.optimize_tables:
+            tables = (qt.pretrained_model.table, dt.pretrained_model.table)
+            nt = tables[0].numel()
+            self.n_table = 2 * nt
+            if self.exchange == "peer":
+                self.txchg = comm.DpExchange(self.n_table, world_size, rank, dev, group=process_group)
+                self.table_flat_g = torch.zeros(self.n_table + 1, dtype=torch.float32, device=dev)
+                with torch.no_grad():
+                    for i, t in enumerate(tables):
+                        view = self.txchg.flat_p[i * nt: (i + 1) * nt].view_as(t)
+                        view.copy_(t.data)
+                        t.data = view  # the table Parameter now aliases the peer segment
+                self.table_grads = tuple(self.table_flat_g[i * nt: (i + 1) * nt].view_as(t)
+                                         for i, t in enumerate(tables))
+            self._table_m = torch.zeros(self.n_table, dtype=torch.float32, device=dev)
+            self._table_v = torch.zeros(self.n_table, dtype=torch.float32, device=dev)
+            self.table_exp_avg = tuple(self._table_m[i * nt: (i + 1) * nt].view_as(t) for i, t in enumerate(tables))
+            self.table_exp_avg_sq = tuple(self._table_v[i * nt: (i + 1) * nt].view_as(t) for i, t in enumerate(tables))
         self.p_views, self.g_views = [], []
         off = 0
         with torch.no_grad():
@@ -282,8 +324,7 @@ class FusedTrainer:
             self.row_bufs = [torch.zeros(3 * batch_size, dtype=torch.int32, device=dev) for _ in range(n_slots)]
             self._rows_loaded = [False] * n_slots  # step() refuses a slot whose rows were never given
         self.tok = self.tok_slots[0]
-        self.table_grads = None
-        if self.train_table:
+        if self.train_table and self.table_grads is None:
             self.table_grads = (torch.zeros_like(qt.pretrained_model.table, dtype=torch.float32),
                                 torch.zeros_like(dt.pretrained_model.table, dtype=torch.float32))
         # TWO step workspaces: the pooled gather of step i+1 (tokens + frozen tables only, never the projection
@@ -322,6 +363,8 @@ class FusedTrainer:
                 # with the tensor-core precisions; a launch after the step otherwise)
                 so.bind_adam(self.adam_state, self.flat_p, self.flat_g, self.exp_avg, self.exp_avg_sq, self.lr,
                              self.betas, self.eps)
+                if self.optimize_tables:  # the tables' Adam step rides in the table gradient's epilogue
+                    so.bind_table_adam(tables, self.table_exp_avg, self.table_exp_avg_sq)
             self.step_objs.append(so)
         self.step_obj = self.step_objs[0]
         # In-batch negatives (the reference's batcher, backend/data.py:113-137): negative i IS positive neg_index[i], so
@@ -380,6 +423,14 @@ class FusedTrainer:
             self.flat_p.copy_(tmp)
         st = self.xchg.state if self.xchg is not None else self.adam_state
         dist.broadcast(st, src=0, group=self.pg)
+        if self.txchg is not None:  # trained tables: only their gradients are exchanged afterwards, as above
+            tmp = self.txchg.flat_p.clone()
+            dist.broadcast(tmp, src=0, group=self.pg)
+            if not torch.equal(tmp, self.txchg.flat_p):
+                if self.rank != 0:
+                    print(f"[rank {self.rank}] FusedTrainer: initial token tables differed from rank 0's; taking rank 0's")
+                self.txchg.flat_p.copy_(tmp)
+            dist.broadcast(self.txchg.state, src=0, group=self.pg)
         torch.cuda.synchronize()
 
     def sync_ranks(self):
@@ -396,6 +447,8 @@ class FusedTrainer:
         loss is read on the host and at the end of every epoch."""
         if self.xchg is not None:
             self.xchg.check()
+        if self.txchg is not None:
+            self.txchg.check()
 
     # -- pieces ------------------------------------------------------------------------------------
     def load_tokens(self, q: TokenBatch, p: TokenBatch, n: TokenBatch, slot: int = 0):
@@ -435,9 +488,13 @@ class FusedTrainer:
         self.step_objs[parity].run(slot, phases, optimise=optimise, accumulate=accumulate)
 
     def _exchange(self):
-        """The fused reduce-scatter / Adam / all-gather kernel (tt_dp_reduce_adam) on the current stream."""
+        """The fused reduce-scatter / Adam / all-gather kernel (tt_dp_reduce_adam) on the current stream; with trained
+        tables a second call on their flat gradient follows (its loss slot stays 0)."""
         self.xchg.reduce_adam(self.flat_g, self.exp_avg, self.exp_avg_sq, self.lr, self.betas, self.eps,
                               self.exchange_ctas)
+        if self.txchg is not None:
+            self.txchg.reduce_adam(self.table_flat_g, self._table_m, self._table_v, self.lr, self.betas, self.eps,
+                                   self.exchange_ctas)
 
     def _pipelined(self, slot: int, next_slot: Optional[int], parity: int, mode=(False, True)):
         """One training step on the current stream, in the schedule __init__ chose: whole step (gather -> persistent
@@ -510,7 +567,7 @@ class FusedTrainer:
         N.check(N.load().tt_adam_step_dev(N.ptr(self.flat_p), N.ptr(self.flat_g), N.ptr(self.exp_avg),
                                           N.ptr(self.exp_avg_sq), self.n_param, self.lr, b1, b2, self.eps,
                                           N.ptr(self.adam_state), 1.0, N.stream()), "tt_adam_step_dev")
-        # (table training uses a plain SGD-free path: the caller owns the table optimiser)
+        # projections only: optimize_tables is refused with this NCCL baseline
 
     def _warm_up(self):
         # one eager forward/backward on a side stream (first-use kernel attributes), gradients only: harmless, except
@@ -669,10 +726,12 @@ class FusedTrainer:
         return avg
 
     # -- checkpoint / resume (main.py:142-152 saves `model.state_dict()`; this adds the optimiser so a run can resume) --
-    def _slice_bounds(self):
-        per = (self.n_param + 1 + self.world - 1) // self.world
+    def _slice_bounds(self, n: Optional[int] = None):
+        """This rank's slice [lo, hi) of an exchanged flat buffer of n parameters (tt_dp_segment_bytes' layout)."""
+        n = self.n_param if n is None else n
+        per = (n + 1 + self.world - 1) // self.world
         S = (per + 63) // 64 * 64
-        return min(self.rank * S, self.n_param), min((self.rank + 1) * S, self.n_param)
+        return min(self.rank * S, n), min((self.rank + 1) * S, n)
 
     def state_dict(self) -> dict:
         """Model weights (reference key names) + Adam moments and step count.  Collective in peer mode with
@@ -697,6 +756,17 @@ class FusedTrainer:
                       window_pending=self.window.pending, window_grad=self.flat_g[: self.n_param].cpu().clone())
             if self.table_grads is not None:
                 sd["window_table_grads"] = tuple(t.cpu().clone() for t in self.table_grads)
+        if self.optimize_tables:
+            tm, tv = self._table_m.clone(), self._table_v.clone()
+            if self.txchg is not None and self.world > 1:
+                torch.distributed.all_reduce(tm, group=self.pg)   # sharded like exp_avg
+                torch.distributed.all_reduce(tv, group=self.pg)
+            nt = self.n_table // 2
+            shape = self.table_exp_avg[0].shape
+            sd["table_exp_avg"] = (tm[:nt].view(shape).cpu(), tm[nt:].view(shape).cpu())
+            sd["table_exp_avg_sq"] = (tv[:nt].view(shape).cpu(), tv[nt:].view(shape).cpu())
+            if self.txchg is not None:
+                sd["table_adam_state"] = self.txchg.state.detach().cpu().clone()
         return sd
 
     def load_state_dict(self, sd: dict):
@@ -711,6 +781,9 @@ class FusedTrainer:
             if ("window_table_grads" in sd) != (self.table_grads is not None):
                 raise ValueError("FusedTrainer.load_state_dict: the checkpoint's open window and this trainer disagree "
                                  "on whether the token tables train")
+        if self.optimize_tables and "table_exp_avg" not in sd:
+            raise ValueError("FusedTrainer.load_state_dict: this trainer optimises the token tables, the checkpoint holds "
+                             "no table moments (it was saved without optimize_tables)")
         model_sd = sd["model"]
         if self.pooled is not None:
             # The pooled banks were computed from the frozen backbone and are keyed to its tensors' versions: copying the
@@ -740,6 +813,16 @@ class FusedTrainer:
             self.xchg.state.copy_(sd["adam_state"])
         else:
             self.adam_state.copy_(sd["adam_state"])
+        if self.optimize_tables:
+            for dst, src in ((self.table_exp_avg, sd["table_exp_avg"]), (self.table_exp_avg_sq, sd["table_exp_avg_sq"])):
+                for t, x in zip(dst, src):
+                    t.copy_(x)
+            if self.txchg is not None:
+                lo, hi = self._slice_bounds(self.n_table)
+                for t in (self._table_m, self._table_v):
+                    t[:lo].zero_()
+                    t[hi:].zero_()
+                self.txchg.state.copy_(sd.get("table_adam_state", sd["adam_state"]))
         self.steps_done = int(sd.get("steps_done", 0))
         # a checkpoint without an open window resumes at a window start
         self.window.pending = pending
@@ -776,6 +859,16 @@ class FusedTrainer:
             self.loss_view = self.loss_view.clone()
             self.xchg.close()
             self.xchg = None
+            if self.txchg is not None:  # and the trained tables out of theirs
+                self.txchg.check()
+                with torch.no_grad():
+                    keep = self.txchg.flat_p.clone()
+                    nt = self.n_table // 2
+                    for i, t in enumerate((self.model.query_tower.pretrained_model.table,
+                                           self.model.document_tower.pretrained_model.table)):
+                        t.data = keep[i * nt: (i + 1) * nt].view_as(t)
+                self.txchg.close()
+                self.txchg = None
             self.exchange = "closed"
 
     def train_epoch(self, loader: TokenTripletLoader, log_every: int = 0) -> float:
@@ -1119,6 +1212,16 @@ def hard_negative_config(hard_negatives: Union[None, int, dict]) -> Optional[dic
     return {"miner": kw, "warmup_epochs": warmup}
 
 
+def train_table_config(train_table: Optional[bool]) -> bool:
+    """run_training(train_table=...) -> bool.  None reads TT_TRAIN_TABLE (unset / 0 = off, 1 = on)."""
+    if train_table is None:
+        env = os.environ.get("TT_TRAIN_TABLE", "0").strip() or "0"
+        if env not in ("0", "1"):
+            raise ValueError(f"TT_TRAIN_TABLE must be 0 or 1, got {env!r}")
+        return env == "1"
+    return bool(train_table)
+
+
 def run_training(
     num_epochs: int = 3,
     batch_size: int = 1024,
@@ -1138,6 +1241,7 @@ def run_training(
     backbone: Optional[str] = None,
     hard_negatives: Union[None, int, dict] = None,
     fused_accumulation: Optional[bool] = None,
+    train_table: Optional[bool] = None,
 ) -> TwoTowersModel:
     """Main training function (training.py:383-529).  `fused` (additive) selects the FusedTrainer; by
     default it is used whenever the dataset is token-bank backed and no gradient accumulation / wandb
@@ -1156,7 +1260,12 @@ def run_training(
     `fused_accumulation` (additive): honour `accumulation_steps` on the fused path (FusedTrainer(accumulation_steps=a):
     micro-batches add into the flat gradient, one optimiser step and, data parallel, one exchange per window).  None
     reads TT_FUSED_ACCUMULATION (unset or 0 = off, the default).  Off, one GPU takes the fused path only at
-    accumulation_steps == 1 and data-parallel runs step every global batch."""
+    accumulation_steps == 1 and data-parallel runs step every global batch.
+
+    `train_table` (additive): train both token tables with the projections (TwoTowersModel(train_table=True), every
+    parameter under one torch.optim.Adam step count).  None reads TT_TRAIN_TABLE (unset or 0 = off, the default; 1 =
+    on).  The fused path runs FusedTrainer(optimize_tables=True), the reference-shaped loops
+    torch.optim.Adam(model.parameters()).  Needs the token-table backbone with fp32 tables and no hard negatives."""
     if isinstance(accumulation_steps, bool) or not isinstance(accumulation_steps, int) or accumulation_steps < 1:
         raise ValueError(f"accumulation_steps must be an integer >= 1, got {accumulation_steps!r}")
     if fused_accumulation is None:
@@ -1170,6 +1279,17 @@ def run_training(
         backbone = os.environ.get("TT_BACKBONE", "table")
     if backbone not in ("table", "minilm"):
         raise ValueError(f"backbone must be 'table' or 'minilm', got {backbone!r}")
+    train_table = train_table_config(train_table)
+    if train_table:
+        if backbone == "minilm":
+            raise ValueError("train_table needs the token-table backbone: the MiniLM backbone is frozen (model.py:28-30) "
+                             "and has no token table")
+        if hn is not None:
+            raise ValueError("train_table and hard negatives are exclusive: the miner's pooled banks come from the frozen "
+                             "table and would go stale at the first step")
+        if table_dtype != torch.float32:
+            raise ValueError(f"train_table needs fp32 token tables, got table_dtype={table_dtype} (bf16 tables do not "
+                             "train)")
     # one process per GPU under torchrun / torch.distributed.run (SURVEY.md §8e): `batch_size` is the GLOBAL batch,
     # every rank trains on its contiguous slice and evaluates its shard of the documents
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -1213,12 +1333,15 @@ def run_training(
     if backbone == "minilm":
         model = TwoTowersModel(projection_dim=projection_dim, backbone="minilm").to(device)
     else:
-        model = TwoTowersModel(projection_dim=projection_dim, table_dtype=table_dtype).to(device)
+        model = TwoTowersModel(projection_dim=projection_dim, table_dtype=table_dtype, train_table=train_table).to(device)
     if world > 1:  # random-init tables and projections are drawn per process: rank 0's become everybody's
         for t in list(model.parameters()) + list(model.buffers()):
             dist.broadcast(t.data, src=0)
     criterion = TripletLoss(margin=margin)
     optimizer = torch.optim.Adam(model.parameters(), lr=learning_rate)
+    if train_table:
+        say(f"Trainable parameters: {sum(p.numel() for p in model.parameters() if p.requires_grad):,} "
+            "(token tables included)")
     if use_wandb:
         if world == 1:
             wandb.watch(model, log="all", log_freq=100)
@@ -1288,7 +1411,8 @@ def run_training(
                 reuse = False
                 say("  Hard negatives: neg-index reuse is off (a mined negative is not a positive of the batch)")
             trainer = FusedTrainer(model, margin, learning_rate, batch_size // world, token_slots=2, world_size=world,
-                                   rank=rank, in_batch_negatives=reuse, accumulation_steps=fused_accum)
+                                   rank=rank, in_batch_negatives=reuse, accumulation_steps=fused_accum,
+                                   optimize_tables=train_table)
             if hn is not None:  # the frozen table's pooled rows, for mining only (the step still pools tokens)
                 banks = (PooledBank.build(model.query_tower, train_ds.query_bank, trainer.Lq, world_size=world,
                                           rank=rank),
