@@ -182,8 +182,12 @@ typedef struct tt_step_args {
    * (backend/data.py:113-137), so negative row i is the same token sequence as positive row neg_index[i]
    * (0 <= neg_index[i] < B, int32 on the device).  Given the indices, the pooled gather visits every positive
    * once and writes its pooled row to the negative rows that name it — the same bits as gathering the same tokens
-   * again, for half the document rows read; n_ids / n_mask are not read then.  Frozen tables only.  An index out
-   * of range raises err_flag.                                                                                  */
+   * again, for half the document rows read; n_ids / n_mask are not read anywhere in the call then.  With table
+   * gradients (dtable_q / dtable_d) each negative's gradient row g_n[i] (d loss / d masked token sum) is folded
+   * into the positive it copies: g'_p[j] = ((g_p[j] + g_n[i1]) + g_n[i2]) + ... over the negatives i1 < i2 < ...
+   * naming j, in fp32 and ascending i, and the document table's gradient (or its Adam step) sums over the
+   * positives' tokens only.  That is the same gradient as walking the negatives' tokens, up to the fp32 summation
+   * order.  An index out of range raises err_flag and adds nothing to any positive.                          */
   const int32_t* neg_index;
   /* optional frozen front end (NULL = pool tokens as before): rows of F.normalize(masked_mean(backbone(text)))
    * computed once per text.  Output row i     = pooled_q[pooled_index[i]],

@@ -279,7 +279,6 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
   pp.nrm = w.nrm;
   pp.err = a->err_flag;
   if (a->neg_index) {  // in-batch negatives: the n rows are copies of the p rows they name
-    TT_REQUIRE(!train_table, "tt_triplet_step: neg_index needs frozen tables (the table gradient walks the negatives' tokens)");
     pp.nseg = 2;
     pp.alias = a->neg_index;
     pp.alias_n = B;
@@ -373,7 +372,12 @@ extern "C" int tt_triplet_step(const tt_step_args* a, tt_stream_t stream) {
                                w.pool_ws_bytes, st, table_adam ? &tq : nullptr)))
       return rc;
     PoolBwdSeg sd[2] = {{a->p_ids, a->p_mask, B, a->Ld, B}, {a->n_ids, a->n_mask, B, a->Ld, 2 * B}};
-    if ((rc = pool_bwd_scatter(sd, 2, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_d, acc, w.pool_ws,
+    int nsd = 2;
+    if (a->neg_index) {  // negative i pooled positive neg_index[i]'s tokens: fold its g row into that positive's
+      if ((rc = pool_bwd_fold_neg(a->neg_index, B, H, w.g + (size_t)2 * B * H, w.g + (size_t)B * H, st))) return rc;
+      nsd = 1;
+    }
+    if ((rc = pool_bwd_scatter(sd, nsd, a->ids_dtype, a->mask_dtype, w.g, a->vocab, H, a->dtable_d, acc, w.pool_ws,
                                w.pool_ws_bytes, st, table_adam ? &td : nullptr)))
       return rc;
   }

@@ -64,5 +64,8 @@ int pool_bwd_scatter(const PoolBwdSeg* segs, int nseg, int ids_dtype, int mask_d
 // dxhat -> g: through F.normalize and the mean (rows [0,rows))
 int pool_bwd_prep(const float* dxhat, const float* xhat, const float* cnt, const float* nrm, int rows,
                   int H, float* g, cudaStream_t st);
+// in-batch negatives (neg_index int32 [B]): g_p[j] = ((g_p[j] + g_n[i1]) + g_n[i2]) + ... over the negatives
+// i1 < i2 < ... with neg_index[i] == j, in place (g_p, g_n [B,H]); an index outside [0,B) adds nothing
+int pool_bwd_fold_neg(const int* neg_index, int B, int H, const float* g_n, float* g_p, cudaStream_t st);
 
 }  // namespace tt

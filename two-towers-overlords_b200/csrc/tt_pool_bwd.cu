@@ -3,7 +3,9 @@
 // so this is the D2 extension of SURVEY.md — its oracle is autograd through nn.Embedding.)
 //
 //   1. prep:    g[seq] = d(loss)/d(masked sum) = normalize-backward(dxhat) / max(cnt,1e-9)
-//   2. sort:    stable LSD radix sort (8-bit digits) of (token id, position) pairs; masked tokens get
+//      fold:    (in-batch negatives named by index) g_p[j] += g_n[i] for every negative i naming positive j, in
+//               ascending i; the document table then sums over the positives' tokens only
+//   2. sort:   stable LSD radix sort (8-bit digits) of (token id, position) pairs; masked tokens get
 //               the sentinel key `vocab`.  Warp-private contiguous chunks + __match_any_sync ranking keep
 //               the sort stable, hence the reduction order (ascending position) is fixed.
 //   3. reduce:  one warp per table row sums mask_t * g[seq(t)] over its run in sorted order and writes
@@ -68,6 +70,52 @@ __global__ void pool_bwd_prep_kernel(const float* __restrict__ dxhat, const floa
     o.z = (d[j].z - x[j].z * k) * inv;
     o.w = (d[j].w - x[j].w * k) * inv;
     *reinterpret_cast<float4*>(g + (size_t)row * H + (j * 32 + lane) * 4) = o;
+  }
+}
+
+// ---- 1b. fold of the in-batch negatives --------------------------------------------------------
+// Negative row i is the token sequence of positive row neg_index[i], so its share of the table gradient is that
+// positive's with g_n[i] in place of g_p[j]: add it into g_p[j] and the scatter walks the positives' tokens only.
+// One warp per positive j; the CTA stages neg_index in shared tiles and every warp ballots over them in ascending i,
+// so g'_p[j] = ((g_p[j] + g_n[i1]) + g_n[i2]) + ... for i1 < i2 < ...  Indices outside [0, B) match no positive.
+constexpr int kFoldWarps = 8;
+constexpr int kFoldTile = 1024;
+
+template <int NV>
+__global__ void __launch_bounds__(kFoldWarps * 32)
+    pool_bwd_fold_kernel(const int* __restrict__ neg_index, int B, const float* __restrict__ g_n,
+                         float* __restrict__ g_p) {
+  constexpr int H = NV * 128;
+  __shared__ int s_idx[kFoldTile];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int j = blockIdx.x * kFoldWarps + warp;  // j >= B: a spare warp of the last CTA, which writes nothing
+  const float* src = g_p + (size_t)min(j, B - 1) * H;
+  float4 acc[NV];
+#pragma unroll
+  for (int k = 0; k < NV; ++k) acc[k] = *(reinterpret_cast<const float4*>(src) + k * 32 + lane);
+  bool any = false;
+  for (int t0 = 0; t0 < B; t0 += kFoldTile) {
+    const int n = min(kFoldTile, B - t0);
+    __syncthreads();
+    for (int t = threadIdx.x; t < n; t += kFoldWarps * 32) s_idx[t] = __ldg(neg_index + t0 + t);
+    __syncthreads();
+    for (int c = 0; c < n; c += 32) {
+      unsigned hit = __ballot_sync(0xffffffffu, c + lane < n && s_idx[c + lane] == j);
+      any |= hit != 0u;
+      while (hit) {
+        const int i = t0 + c + __ffs(hit) - 1;
+        hit &= hit - 1u;
+#pragma unroll
+        for (int k = 0; k < NV; ++k) {
+          const float4 v = __ldg(reinterpret_cast<const float4*>(g_n + (size_t)i * H) + k * 32 + lane);
+          acc[k].x += v.x; acc[k].y += v.y; acc[k].z += v.z; acc[k].w += v.w;
+        }
+      }
+    }
+  }
+  if (j < B && any) {
+#pragma unroll
+    for (int k = 0; k < NV; ++k) *(reinterpret_cast<float4*>(g_p + (size_t)j * H) + k * 32 + lane) = acc[k];
   }
 }
 
@@ -402,6 +450,19 @@ int pool_bwd_prep(const float* dxhat, const float* xhat, const float* cnt, const
     case 2: pool_bwd_prep_kernel<2><<<blocks, 128, 0, st>>>(dxhat, xhat, cnt, nrm, rows, g); break;
     case 3: pool_bwd_prep_kernel<3><<<blocks, 128, 0, st>>>(dxhat, xhat, cnt, nrm, rows, g); break;
     default: pool_bwd_prep_kernel<6><<<blocks, 128, 0, st>>>(dxhat, xhat, cnt, nrm, rows, g); break;
+  }
+  TT_LAUNCH_CHECK();
+  return 0;
+}
+
+int pool_bwd_fold_neg(const int* neg_index, int B, int H, const float* g_n, float* g_p, cudaStream_t st) {
+  if (B == 0) return 0;
+  const int blocks = (B + kFoldWarps - 1) / kFoldWarps;
+  switch (H / 128) {
+    case 1: pool_bwd_fold_kernel<1><<<blocks, kFoldWarps * 32, 0, st>>>(neg_index, B, g_n, g_p); break;
+    case 2: pool_bwd_fold_kernel<2><<<blocks, kFoldWarps * 32, 0, st>>>(neg_index, B, g_n, g_p); break;
+    case 3: pool_bwd_fold_kernel<3><<<blocks, kFoldWarps * 32, 0, st>>>(neg_index, B, g_n, g_p); break;
+    default: pool_bwd_fold_kernel<6><<<blocks, kFoldWarps * 32, 0, st>>>(neg_index, B, g_n, g_p); break;
   }
   TT_LAUNCH_CHECK();
   return 0;

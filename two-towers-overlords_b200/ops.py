@@ -302,13 +302,13 @@ class TripletStep:
 
     def set_neg_index(self, slot: int, neg_index: Optional[torch.Tensor]):
         """In-batch negatives for `slot` (tt_step_args.neg_index): int32 [B] on the device, negative row i is the same
-        document as positive row neg_index[i]; its pooled row is then a copy instead of a second gather.  None: the
-        negatives are gathered from their own token tensors."""
+        document as positive row neg_index[i]; its pooled row is then a copy instead of a second gather, and with table
+        gradients its gradient row is folded into that positive's.  None: the negatives are gathered from their own
+        token tensors."""
         a = self.slots[slot]
         if neg_index is None:
             a.neg_index = None
             return
-        assert not self.train_table, "neg_index needs frozen tables"
         assert neg_index.dtype == torch.int32 and neg_index.is_cuda and tuple(neg_index.shape) == (self.shape[0],)
         a.neg_index = N.ptr(neg_index)
         self._keep.append(neg_index)

@@ -184,6 +184,8 @@ class FusedTrainer:
                  exchange_ctas: int = 0, in_batch_negatives: bool = False, pooled=None, accumulation_steps: int = 1,
                  optimize_tables: bool = False):
         qt, dt = model.query_tower, model.document_tower
+        if in_batch_negatives and world_size > 1:  # refused before any buffer or peer segment is allocated
+            raise ValueError("in_batch_negatives: the negatives of a data-parallel slice name documents of other ranks")
         self.window = AccumulationWindow(accumulation_steps)
         self.accum = self.window.a
         self.model = model
@@ -370,13 +372,10 @@ class FusedTrainer:
         # In-batch negatives (the reference's batcher, backend/data.py:113-137): negative i IS positive neg_index[i], so
         # its pooled row is copied instead of gathered a second time (tt_step_args.neg_index).  One int32 [B] buffer per
         # token slot (static addresses: the step graphs read them); fill them with load_neg_index() / the device feeder.
+        # With trainable tables each negative's table-gradient row is folded into the positive it copies.
         self.in_batch_negatives = bool(in_batch_negatives)
         self.neg_bufs = None
         if self.in_batch_negatives:
-            if self.train_table:
-                raise ValueError("in_batch_negatives needs frozen tables")
-            if world_size > 1:
-                raise ValueError("in_batch_negatives: the negatives of a data-parallel slice name documents of other ranks")
             self.neg_bufs = [torch.zeros(batch_size, dtype=torch.int32, device=dev) for _ in self.tok_slots]
             self._neg_loaded = [False] * len(self.tok_slots)  # step() refuses a slot whose indices were never given
             for so in self.step_objs:
@@ -1404,9 +1403,9 @@ def run_training(
                                    world_size=world, rank=rank, pooled=banks, accumulation_steps=fused_accum)
         else:
             # the device feeder draws the in-batch negatives itself and hands their indices to the trainer, which then
-            # pools every positive document once (TT_NEG_REUSE=0: gather the negatives' tokens like any document)
-            reuse = (not host_feeder and world == 1 and os.environ.get("TT_NEG_REUSE", "1") != "0"
-                     and not model.query_tower.pretrained_model.table.requires_grad)
+            # pools every positive document once, and with trainable tables scatter-adds its tokens once (TT_NEG_REUSE=0:
+            # gather the negatives' tokens like any document)
+            reuse = not host_feeder and world == 1 and os.environ.get("TT_NEG_REUSE", "1") != "0"
             if hn is not None:
                 reuse = False
                 say("  Hard negatives: neg-index reuse is off (a mined negative is not a positive of the batch)")
